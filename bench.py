@@ -32,6 +32,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is written into it, bytecode caches included
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in ("iclr2025_3d-mom_b200", os.path.join("iclr2025_3d-mom_b200", "dropin"), "tests", ""):
     sys.path.insert(0, os.path.join(ROOT, p))
@@ -61,6 +62,8 @@ def parse():
     ap.add_argument("--no-shared-spatial", action="store_true",
                     help="render every frame with the full six-plane HexPlane pass instead of sharing the spatial product over a sequence")
     ap.add_argument("--cpu-points", type=int, default=0, help="override the cpu_baseline sample size")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed to DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -780,15 +783,49 @@ class no_gc:
 
 
 def run_steps(trainer, cams, gts, n_global, steps, barrier, max_over_ranks):
+    """K timed steps; returns (device ms, max over ranks; the loss tensor the last step returned, None if K = 0)."""
+    loss = None
     with no_gc():
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            trainer.step(cams, gts, global_batch=n_global)
+            loss = trainer.step(cams, gts, global_batch=n_global)
         e1.record()
         barrier()
-    return max_over_ranks(e0.elapsed_time(e1))
+    return max_over_ranks(e0.elapsed_time(e1)), loss
+
+
+DUMP_ROWS = 65536           # Gaussians sampled (fixed seed) from each per-Gaussian tensor by dump_outputs
+DUMP_LIMIT = 64 << 20       # bytes
+
+
+def dump_outputs(out_dir, model, trainer, loss):
+    """What one training step hands its caller, after the last timed step: the loss of the global batch (the sum over ranks of
+    what each rank's step returned), every trainable parameter
+    as the optimiser left it (grid planes in logical NCHW order) and the densification statistics the step accumulated
+    (viewspace_grad, max_radii).  Per-Gaussian tensors are sampled to DUMP_ROWS rows chosen with a fixed seed, the rest are
+    written whole; float32, except the loss (float64).  Same arguments, same inputs: two builds compare file by file."""
+    import numpy as np
+    if loss is None:
+        raise SystemExit("--dump-outputs needs at least one timed step (--steps >= 1)")
+    os.makedirs(out_dir, exist_ok=True)
+    P = model._xyz.shape[0]
+    rows = torch.from_numpy(np.sort(np.random.default_rng(0).choice(P, min(P, DUMP_ROWS), replace=False)))
+    trainable = {id(p) for p in trainer.trainable}
+    tensors = [(n, p) for n, p in model.named_parameters() if id(p) in trainable]
+    tensors += [("viewspace_grad", trainer.viewspace_grad), ("max_radii", trainer.max_radii)]
+    arrays = {"loss": np.array([float(loss)], dtype=np.float64)}
+    for n, t in tensors:
+        t = t.detach()
+        if t.dim() > 0 and t.shape[0] == P:
+            t = t[rows.to(t.device)]
+        arrays[n] = t.float().contiguous().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    for n, a in arrays.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a)
 
 
 def run_steps_e2e(trainer, cams, host_images, n_global, steps, device, barrier, max_over_ranks, impl, warm=2):
@@ -945,7 +982,14 @@ def _main():
     timeline = None
     with ClockSampler(local, enabled=(rank == 0)) as clk:
         # headline: EXACTLY K un-instrumented steps between barriers, device time, max over ranks
-        ms = run_steps(trainer, cams, gts_dev, n_global, args.steps, barrier, max_over_ranks)
+        ms, last_loss = run_steps(trainer, cams, gts_dev, n_global, args.steps, barrier, max_over_ranks)
+        if args.dump_outputs:
+            if world > 1 and last_loss is not None:      # each rank's step returns its LOCAL share of the batch loss
+                import torch.distributed as dist
+                last_loss = last_loss.detach().clone()
+                dist.all_reduce(last_loss)
+            if rank == 0:
+                dump_outputs(args.dump_outputs, model, trainer, last_loss)
         # the same K steps again with every entry point / rasterizer phase bracketed by CUDA events: the per-kernel durations
         # of the `kernels` table and the roofline (the ~150 extra event records per step make this pass a few per cent slower)
         calls, phases = {}, {}
@@ -956,7 +1000,7 @@ def _main():
             piped, trainer.pipeline_views = trainer.pipeline_views, False
             with _b200lib.CallTimer() as timer:
                 _b200lib.lib().b200gs_profile_enable(1)
-                ms_instr = run_steps(trainer, cams, gts_dev, n_global, args.steps, barrier, max_over_ranks)
+                ms_instr, _ = run_steps(trainer, cams, gts_dev, n_global, args.steps, barrier, max_over_ranks)
                 calls = timer.summary()
                 phases = read_phases()
                 _b200lib.lib().b200gs_profile_enable(0)
@@ -996,7 +1040,7 @@ def _main():
         dev_w = [h.to(device) for h in host_w]
         for _ in range(2):
             trainer.step(cams_w, dev_w, global_batch=nw)
-        ms_w = run_steps(trainer, cams_w, dev_w, nw, args.steps, barrier, max_over_ranks)
+        ms_w, _ = run_steps(trainer, cams_w, dev_w, nw, args.steps, barrier, max_over_ranks)
         ms_we, _, _, _ = run_steps_e2e(trainer, cams_w, host_w, nw, args.steps, device, barrier, max_over_ranks, impl)
         weak = {"scaling": "weak", "views_per_gpu": args.views_per_gpu, "global_batch": nw, "value": nw * args.steps / (ms_w / 1e3),
                 "unit": "view-iters/s", "ms_per_step": ms_w / args.steps, "e2e_value": nw * args.steps / (ms_we / 1e3)}

@@ -1,5 +1,6 @@
 """GPU parity: our rasterizer (through the C ABI / drop-in Python API) against the
-reference's own CUDA code (oracle/_ref/libref_rast.so) on identical seeded inputs.
+reference's own CUDA code on identical seeded inputs (its outputs are stored in
+tests/golden/parity_test_raster_parity.npz, see tests/ref_golden.py).
 
 Bars (BASELINE.json north_star): bit-exact radii, tile keys, sorted order, tile ranges;
 colour and depth within 1e-4 max-abs; gradients within 1e-3 relative (of the tensor's
@@ -8,8 +9,8 @@ import numpy as np
 import pytest
 import torch
 
-import ref_harness as rh
 from b200gs import synthetic as syn
+from ref_golden import Golden
 
 pytestmark = pytest.mark.gpu
 
@@ -59,76 +60,62 @@ _FULL = [(1000000, 1280, 720, 0.010), (1000000, 1920, 1080, 0.004), (5000000, 38
 
 @pytest.mark.parametrize("P,W,H,mu", [(2000, 64, 48, 0.02), (20000, 200, 120, 0.01), (200000, 512, 512, 0.004),
                                       (200000, 512, 512, 0.010)] + _FULL)
-def test_forward_bit_exact_and_image(P, W, H, mu):
-    assert rh.have_ref(), "oracle/_ref/libref_rast.so missing (run oracle/build_ref.sh)"
+def test_forward_bit_exact_and_image(P, W, H, mu, request):
     from b200gs.rasterizer import _C
+    ref = Golden(request)
     act, cam = _scene(P, W, H, mu)
     bg = torch.tensor([0.1, 0.2, 0.3], device="cuda")
-    R_ref, c_ref, d_ref, radii_ref = rh.ref_forward(cam, bg, act["means3D"], act["opacities"], shs=act["shs"],
-                                                    scales=act["scales"], rotations=act["rotations"])
     out = _C.rasterize_gaussians(bg, act["means3D"], torch.Tensor([]), act["opacities"], act["scales"],
                                  act["rotations"], 1.0, torch.Tensor([]), cam.viewmatrix, cam.projmatrix,
                                  cam.tanfovx, cam.tanfovy, H, W, act["shs"], 3, cam.campos, False, False)
     R, color, depth, radii, geom, binb, img = out
     torch.cuda.synchronize()
-    assert R == R_ref
-    assert torch.equal(radii, radii_ref)
+    assert R == ref.value("R")
+    assert ref.equal("radii", radii)
     get = _export(P, R, cam, (geom, binb, img))
-    vis = radii_ref.cpu().numpy() > 0
-    assert np.array_equal(get("tiles_touched", np.uint32), rh.ref_get("tiles_touched"))
-    assert np.array_equal(get("keys", np.uint64), rh.ref_get("keys"))
-    assert np.array_equal(get("point_list", np.uint32), rh.ref_get("point_list"))
+    vis = radii.cpu().numpy() > 0
+    assert ref.equal("tiles_touched", get("tiles_touched", np.uint32))
+    assert ref.equal("keys", get("keys", np.uint64))
+    assert ref.equal("point_list", get("point_list", np.uint32))
     tiles = ((W + 15) // 16) * ((H + 15) // 16)
-    assert np.array_equal(get("ranges", np.uint32), rh.ref_get("ranges")[: 2 * tiles])
+    assert ref.equal("ranges", get("ranges", np.uint32)[: 2 * tiles])
     # per-Gaussian projected state (visible ones; the reference leaves culled slots stale)
-    np.testing.assert_array_equal(get("depths", np.float32)[vis], rh.ref_get("depths")[vis])
-    np.testing.assert_array_equal(get("means2D", np.float32).reshape(-1, 2)[vis], rh.ref_get("means2D").reshape(-1, 2)[vis])
-    np.testing.assert_array_equal(get("cov3D", np.float32).reshape(-1, 6)[vis], rh.ref_get("cov3D").reshape(-1, 6)[vis])
-    np.testing.assert_array_equal(get("conic_opacity", np.float32).reshape(-1, 4)[vis],
-                                  rh.ref_get("conic_opacity").reshape(-1, 4)[vis])
-    np.testing.assert_allclose(get("rgb", np.float32).reshape(-1, 3)[vis], rh.ref_get("rgb").reshape(-1, 3)[vis],
-                               rtol=0, atol=2e-6)
-    assert np.array_equal(get("n_contrib", np.uint32), rh.ref_get("n_contrib"))
-    np.testing.assert_allclose(get("accum_alpha", np.float32), rh.ref_get("accum_alpha"), rtol=0, atol=1e-6)
-    assert (color - c_ref).abs().max().item() <= COLOR_TOL
-    assert (depth - d_ref).abs().max().item() <= COLOR_TOL
-
-
-def _rel(a, b):
-    return (a - b).abs().max().item() / max(b.abs().max().item(), 1e-20)
+    assert ref.equal("depths", get("depths", np.float32)[vis])
+    assert ref.equal("means2D", get("means2D", np.float32).reshape(-1, 2)[vis])
+    assert ref.equal("cov3D", get("cov3D", np.float32).reshape(-1, 6)[vis])
+    assert ref.equal("conic_opacity", get("conic_opacity", np.float32).reshape(-1, 4)[vis])
+    assert ref.maxdiff("rgb", get("rgb", np.float32).reshape(-1, 3)[vis]) <= 2e-6
+    assert ref.equal("n_contrib", get("n_contrib", np.uint32))
+    assert ref.maxdiff("accum_alpha", get("accum_alpha", np.float32)) <= 1e-6
+    assert ref.maxdiff("color", color) <= COLOR_TOL
+    assert ref.maxdiff("depth", depth) <= COLOR_TOL
 
 
 @pytest.mark.parametrize("P,W,H,mu,depth_grad", [(20000, 200, 120, 0.01, True), (200000, 512, 512, 0.004, False),
                                                  (200000, 512, 512, 0.010, True)] + [c + (True,) for c in _FULL])
-def test_backward_gradients(P, W, H, mu, depth_grad):
+def test_backward_gradients(P, W, H, mu, depth_grad, request):
+    ref = Golden(request)
     act, cam = _scene(P, W, H, mu)
     bg = torch.tensor([0.0, 0.0, 0.0], device="cuda")
     g = torch.Generator(device="cpu").manual_seed(7)
     gt = torch.rand(3, H, W, generator=g).cuda()
-    R_ref, c_ref, d_ref, radii_ref = rh.ref_forward(cam, bg, act["means3D"], act["opacities"], shs=act["shs"],
-                                                    scales=act["scales"], rotations=act["rotations"])
     color, radii, depth, inp, means2D = _ours_forward(cam, bg, act, requires_grad=True)
     loss = (color - gt).abs().mean()
     wd = torch.randn(1, H, W, generator=g).cuda() / (H * W) if depth_grad else None
     if depth_grad:
         loss = loss + (depth * wd).sum()
     loss.backward()
-    dL_dcolor = torch.sign(c_ref - gt) / (3 * H * W)
-    # use OUR colour's sign pattern so both sides see the same upstream gradient
-    dL_dcolor = torch.sign(color.detach() - gt) / (3 * H * W)
-    dL_ddepth = wd if depth_grad else torch.zeros(1, H, W, device="cuda")
-    gr = rh.ref_backward(cam, bg, R_ref, radii_ref, dL_dcolor, dL_ddepth, act["means3D"], shs=act["shs"],
-                         scales=act["scales"], rotations=act["rotations"])
-    pairs = [("means3D", inp["means3D"].grad, gr["means3D"]), ("means2D", means2D.grad, gr["means2D"]),
-             ("sh", inp["shs"].grad, gr["sh"]), ("opacity", inp["opacities"].grad, gr["opacity"]),
-             ("scales", inp["scales"].grad, gr["scales"]), ("rotations", inp["rotations"].grad, gr["rotations"])]
-    for name, ours, ref in pairs:
+    # the reference's backward was given OUR colour's sign pattern, so both sides saw the same upstream gradient
+    pairs = [("means3D", inp["means3D"].grad), ("means2D", means2D.grad), ("sh", inp["shs"].grad),
+             ("opacity", inp["opacities"].grad), ("scales", inp["scales"].grad), ("rotations", inp["rotations"].grad)]
+    for name, ours in pairs:
         assert ours is not None, name
-        r = _rel(ours, ref)
+        r = ref.rel(name, ours)
         assert r <= GRAD_RTOL, f"{name}: rel err {r:.3e}"
 
 
-def test_precomputed_colors_and_cov():
+def test_precomputed_colors_and_cov(request):
+    ref = Golden(request)
     P, W, H = 20000, 160, 96
     act, cam = _scene(P, W, H, 0.01)
     bg = torch.tensor([0.3, 0.1, 0.0], device="cuda")
@@ -143,21 +130,17 @@ def test_precomputed_colors_and_cov():
     L = Rm * s[:, None, :]
     Sig = L @ L.transpose(1, 2)
     cov = torch.stack([Sig[:, 0, 0], Sig[:, 0, 1], Sig[:, 0, 2], Sig[:, 1, 1], Sig[:, 1, 2], Sig[:, 2, 2]], -1).contiguous()
-    R_ref, c_ref, d_ref, radii_ref = rh.ref_forward(cam, bg, act["means3D"], act["opacities"], colors_precomp=colors,
-                                                    cov3D_precomp=cov)
     color, radii, depth, inp, means2D = _ours_forward(cam, bg, act, colors_precomp=colors, cov3D_precomp=cov,
                                                       requires_grad=True)
-    assert torch.equal(radii, radii_ref)
-    assert (color - c_ref).abs().max().item() <= COLOR_TOL
+    assert ref.equal("radii", radii)
+    assert ref.maxdiff("color", color) <= COLOR_TOL
     gt = torch.rand(3, H, W, generator=g).cuda()
     (color - gt).pow(2).mean().backward()
-    dL = 2 * (color.detach() - gt) / (3 * H * W)
-    gr = rh.ref_backward(cam, bg, R_ref, radii_ref, dL, torch.zeros(1, H, W, device="cuda"), act["means3D"],
-                         colors_precomp=colors, cov3D_precomp=cov)
-    assert _rel(inp["colors_precomp"].grad, gr["colors"]) <= GRAD_RTOL
-    assert _rel(inp["cov3D_precomp"].grad, gr["cov3D"]) <= GRAD_RTOL
-    assert _rel(inp["means3D"].grad, gr["means3D"]) <= GRAD_RTOL
-    assert _rel(inp["opacities"].grad, gr["opacity"]) <= GRAD_RTOL
+    # the reference's backward was given dL = 2 (OUR colour - gt) / (3 H W)
+    assert ref.rel("colors", inp["colors_precomp"].grad) <= GRAD_RTOL
+    assert ref.rel("cov3D", inp["cov3D_precomp"].grad) <= GRAD_RTOL
+    assert ref.rel("means3D", inp["means3D"].grad) <= GRAD_RTOL
+    assert ref.rel("opacity", inp["opacities"].grad) <= GRAD_RTOL
 
 
 def test_edge_cases_empty_and_behind_camera():
