@@ -1,7 +1,6 @@
 // extern "C" surface of libb200gs.so (declared in include/b200gs.h).
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -12,20 +11,9 @@ namespace b200gs {
 
 static thread_local char g_err[512] = "";
 
-// Kernel variants (b200gs_set_option): the defaults are the fastest variants that have passed tools/native/mlp_variant_check
-// on a B200 (bit-identical outputs; gradients equal up to float-atomic order); 0 selects the first-generation kernels. The
-// environment (B200GS_MLP_BWD_V2 / B200GS_MLP_FWD_ELECT = integer) overrides the initial value.
-static int env_int(const char* name, int dflt) { const char* e = getenv(name); return (e && e[0] >= '0' && e[0] <= '9') ? atoi(e) : dflt; }
-int g_opt_mlp_bwd_v2 = env_int("B200GS_MLP_BWD_V2", 87);
-int g_opt_mlp_fwd_elect = env_int("B200GS_MLP_FWD_ELECT", 2);
-int g_opt_hexplane_time_bwd = env_int("B200GS_HEXPLANE_TIME_BWD", 2);    // 0.417 -> 0.354 ms (profiles/r2a_hexplane_time_check.txt)
-int g_opt_mlp_bwd_sms = env_int("B200GS_MLP_BWD_SMS", 0);
-int g_opt_mlp_fwd_sms = env_int("B200GS_MLP_FWD_SMS", 0);
-int g_opt_sort_ballot_rank = env_int("B200GS_SORT_BALLOT_RANK", 1);    // 103 -> 87 us per 1M-pair 32-bit sort, 96 -> 79 us per 2.4M-pair 12-bit sort (profiles/r3h_sort_check.txt)
-int g_opt_lookback_parallel = env_int("B200GS_LOOKBACK_PARALLEL", 1);    // 111 -> 103 us per 1M-pair sort (profiles/r2a_sort_check.txt)
-int g_opt_hexplane_time_fwd = env_int("B200GS_HEXPLANE_TIME_FWD", 2);    // 0.134 -> 0.112 ms, bit-identical
-int g_opt_composite_pairs = env_int("B200GS_COMPOSITE_PAIRS", 1);      // two pixels per lane + packed FP32 pairs in the compositing backward
-int g_opt_mlp_bwd_ablate = 0;                                             // timing experiments only (wrong results); never from the environment
+// CTA caps of the persistent MLP kernels (b200gs_set_option); 0 = every SM
+int g_opt_mlp_fwd_sms = 0;
+int g_opt_mlp_bwd_sms = 0;
 
 // ---- opt-in phase timing ---------------------------------------------------------------------------------------------
 int g_prof_enabled = 0;
@@ -133,40 +121,15 @@ int b200gs_version(void) { return 100; }
 
 int b200gs_set_option(const char* name, int value)
 {
-    if (name && !strcmp(name, "mlp_bwd_v2")) {
-        if (value != 0 && value != 1 && value != 3 && value != 5 && value != 7 && value != 55 && value != 87) { set_error("b200gs_set_option: mlp_bwd_v2 = %d is not built (0, 1, 3, 5, 7, 55, 87)", value); return -1; }
-        b200gs::g_opt_mlp_bwd_v2 = value;
-        return 0;
-    }
-    if (name && !strcmp(name, "mlp_fwd_elect")) { b200gs::g_opt_mlp_fwd_elect = value; return 0; }
-    if (name && !strcmp(name, "hexplane_time_bwd")) { b200gs::g_opt_hexplane_time_bwd = value; return 0; }
-    if (name && !strcmp(name, "mlp_bwd_ablate")) {          // wrong results by design: only for a process that says it is profiling
-        const char* e = getenv("B200GS_PROFILING");
-        if (value != 0 && !(e && e[0] == '1')) { set_error("b200gs_set_option: mlp_bwd_ablate needs B200GS_PROFILING=1 in the environment"); return -1; }
-        b200gs::g_opt_mlp_bwd_ablate = value;
-        return 0;
-    }
-    if (name && !strcmp(name, "lookback_parallel")) { b200gs::g_opt_lookback_parallel = value; return 0; }
-    if (name && !strcmp(name, "sort_ballot_rank")) { b200gs::g_opt_sort_ballot_rank = value; return 0; }
-    if (name && !strcmp(name, "mlp_bwd_sms")) { b200gs::g_opt_mlp_bwd_sms = value; return 0; }
     if (name && !strcmp(name, "mlp_fwd_sms")) { b200gs::g_opt_mlp_fwd_sms = value; return 0; }
-    if (name && !strcmp(name, "hexplane_time_fwd")) { b200gs::g_opt_hexplane_time_fwd = value; return 0; }
-    if (name && !strcmp(name, "composite_pairs")) { b200gs::g_opt_composite_pairs = value; return 0; }
+    if (name && !strcmp(name, "mlp_bwd_sms")) { b200gs::g_opt_mlp_bwd_sms = value; return 0; }
     set_error("b200gs_set_option: unknown option '%s'", name ? name : "(null)");
     return -1;
 }
 int b200gs_get_option(const char* name)
 {
-    if (name && !strcmp(name, "mlp_bwd_v2")) return b200gs::g_opt_mlp_bwd_v2;
-    if (name && !strcmp(name, "mlp_fwd_elect")) return b200gs::g_opt_mlp_fwd_elect;
-    if (name && !strcmp(name, "hexplane_time_bwd")) return b200gs::g_opt_hexplane_time_bwd;
-    if (name && !strcmp(name, "mlp_bwd_ablate")) return b200gs::g_opt_mlp_bwd_ablate;
-    if (name && !strcmp(name, "lookback_parallel")) return b200gs::g_opt_lookback_parallel;
-    if (name && !strcmp(name, "sort_ballot_rank")) return b200gs::g_opt_sort_ballot_rank;
-    if (name && !strcmp(name, "mlp_bwd_sms")) return b200gs::g_opt_mlp_bwd_sms;
     if (name && !strcmp(name, "mlp_fwd_sms")) return b200gs::g_opt_mlp_fwd_sms;
-    if (name && !strcmp(name, "hexplane_time_fwd")) return b200gs::g_opt_hexplane_time_fwd;
-    if (name && !strcmp(name, "composite_pairs")) return b200gs::g_opt_composite_pairs;
+    if (name && !strcmp(name, "mlp_bwd_sms")) return b200gs::g_opt_mlp_bwd_sms;
     return -1;
 }
 

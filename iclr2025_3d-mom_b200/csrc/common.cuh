@@ -21,9 +21,8 @@ typedef uint64_t u64;
 // Per-thread last error text (the library keeps no other global state).
 void set_error(const char* fmt, ...);
 int check_launch(const char* what);   // returns 0 or sets error and returns -1
-// opt-in kernel variants, see b200gs_set_option (api.cu)
-extern int g_opt_sort_ballot_rank, g_opt_mlp_bwd_sms, g_opt_mlp_fwd_sms;
-extern int g_opt_mlp_bwd_v2, g_opt_mlp_fwd_elect, g_opt_hexplane_time_bwd, g_opt_mlp_bwd_ablate, g_opt_lookback_parallel, g_opt_hexplane_time_fwd, g_opt_composite_pairs;
+// CTA caps of the persistent MLP kernels, see b200gs_set_option (api.cu)
+extern int g_opt_mlp_fwd_sms, g_opt_mlp_bwd_sms;
 
 // Opt-in phase timing (b200gs_profile_enable / b200gs_profile_read, api.cu): CUDA events recorded on the launching stream around
 // the kernels of one phase of a multi-kernel entry point, so that bench.py can report each kernel family's live duration

@@ -13,16 +13,15 @@
 //     and every shared-memory store below is a full line / conflict free.
 //   * dX chain on the tensor cores, SS mode, full three-term split (dY_lo W_hi + dY_hi W_lo + dY_hi W_hi, FP32-level
 //     accuracy: its error would otherwise reach the per-point xyz gradients un-averaged):  D_RH[p][in] += dz[p][out]
-//     W2_h[out][in], D_FE = dh W1.  A = DYK, un-swizzled K-major core matrices (chunk stride padded to 2064 B so the
-//     column-chunk-per-lane stores do not collide), hi and lo planes; B = the transposed TF32 hi / lo weight images the
-//     forward left behind the stash, W1 resident, the current head's W2 pair streamed in with cp.async.
+//     W2_h[out][in], D_FE = dh W1.  A = the hi and lo dY planes of DYM read as a K-major operand (see below); B = the
+//     transposed TF32 hi / lo weight images the forward left behind the stash, streamed in with cp.async.
 //   * weight gradients on the tensor cores: D_W[out][in] += tf32(dY)^T tf32(X), contraction over the 128
 //     points of the tile, with M = 128 rows = [dY_hi ; dY_lo] (the two halves are added at the flush, so
 //     dY is exact and only X is rounded).  Both operands are MN-major; for TF32 the only MN-major shared-memory layout
 //     tcgen05 accepts is SWIZZLE_128B_BASE32B (descriptor layout type 1): atoms of 4 k-rows x 128 B
 //     (32 MN elements), the 32-byte granule index XORed with the row index (probed on hardware,
 //     tools/probe/umma_probe.cu).  The accumulators D_W2[3], D_W1 stay in TMEM for the whole life of
-//     the CTA and are flushed with one atomic per element per CTA at the end.
+//     the CTA and are flushed once per CTA at the end.
 // Shared memory (~225 KB): W2 slot 32 K (hi|lo) | W1 32 K (hi|lo) | DYM 64 K | XH 32 K | DYK 2 x 33 K.
 // TMEM columns: D_RH [0,64)  D_FE [64,128)  D_W2[h] [128 + 64 h, +64)  D_W1 [320,384).
 #include "tc5_common.cuh"
@@ -33,7 +32,7 @@ namespace tc5 {
 
 constexpr int BT = 256;                     // threads per CTA
 constexpr u32 KCH = 2064;                   // DYK: bytes between 4-column chunks (2048 + 16 pad)
-constexpr u32 KPLANE = 16 * KCH;            // one hi / lo plane of DYK
+constexpr u32 KPLANE = 16 * KCH;            // one half of DYK (one TMA staging slot)
 constexpr u64 DESC_SW128_32B = 1ull << 61;  // smem descriptor layout type SWIZZLE_128B_BASE32B
 
 struct BwdArgs {
@@ -43,7 +42,8 @@ struct BwdArgs {
     const float* feat; const float* saved;
     const float* d_pts; const float* d_scales; const float* d_rot;
     float* d_feat;
-    u32 dy_sbo;                 // SINGLE_DY: byte stride between 8-point groups of the K-major view of the dY image
+    u32 dy_sbo;                 // 512: byte stride between 8-point groups of the K-major view of the dY image (an argument,
+                                // not a constant: folded into the code it makes ptxas spill in the TMA kernel)
 };
 
 __device__ __forceinline__ float4 tf32x4(float4 v)
@@ -66,41 +66,35 @@ __device__ __forceinline__ float4 lds128(u32 addr)
     return v;
 }
 
-// V2 (same arithmetic, same operands, same TMEM map as the first generation):
+// Pipeline (same arithmetic, same operands and same TMEM map as the first generation, which measured 0.744 ms per 1M points):
 //   * the two 32 KB weight slots alternate between consecutive MMA groups and the image of the NEXT group is streamed in
 //     (cp.async) while the current phase computes, so no phase waits for its weights (W1 is re-streamed per tile from L2);
 //   * MMAs are issued from a warp-uniform branch by the elected lane of warp 0 with the shared-memory descriptors formed by
 //     adding constants to two hoisted bases: ~2 SASS instructions per tcgen05.mma instead of ~15 (the single issuing
 //     thread sits on the critical path of every phase);
 //   * the TMEM-resident weight gradients leave through a padded shared-memory transpose as hi + lo sums, one coalesced
-//     128-bit RED per 4 elements (8x fewer atomics than one scalar atomic per hi / lo element, whole lines per warp).
-// VER: 0 = first generation; otherwise bit 0 = V2, bits 1-2 = how the upstream gradients d_out reach a phase (0: loaded at its
-// start, 1: loaded into registers one phase ahead, 2 / 3: prefetched into L1 / L2 one phase ahead); bit 4 = SINGLE_DY: the dX
-// chain reads its A operand dY from the MN-major SWIZZLE_128B_BASE32B image of the weight-gradient MMAs, re-described as a
-// K-major operand (rows = points, 128-byte rows of 32 out-features, 8-row group stride BwdArgs::dy_sbo = 512 B -- the one
-// combination that reproduces the product exactly on hardware, tools/probe/umma_probe2.cu), so dY is stored to shared
-// memory twice (hi, lo) instead of four times: 0.744 -> 0.686 ms per 1M points (profiles/r2a_mlp_variant_check.txt);
-// bit 5 = TMA: the 66 KB of shared memory that frees become two 32 KB staging slots, and the stash / feature rows of a phase
-// (one contiguous 32 KB tile each, tc5_common.cuh) arrive by ONE bulk copy (cp.async.bulk -> UBLKCP, the TMA engine) requested two
-// phases ahead by the MMA-issuing thread and counted on the slot's mbarrier, instead of 8 LDG.128 per thread held in registers
-// across a phase: 0.686 -> 0.597 ms (profiles/r2i_mlp_variant_check.txt; d_out in registers on top of it lost: 0.648).
-// ABL (timing experiments only, WRONG RESULTS, option "mlp_bwd_ablate"): what the kernel costs without one of its parts --
-// 1: d_out read from constants instead of global memory, 2: no operand stores to shared memory, 4: no MMAs (and no waits for
-// them), 8: no gradient math (dz / dW3 / bias sums), 16: no d_feature stores, 32: stash / feature rows from constants.
-template <int VER, int ABL = 0>
+//     128-bit RED per 4 elements (8x fewer atomics than one scalar atomic per hi / lo element, whole lines per warp);
+//   * the upstream gradients d_out of the next phase are prefetched into L2 one phase ahead (loading them into registers
+//     one phase ahead, or prefetching into L1, measured slower);
+//   * ONE dY image: the dX chain reads its A operand dY from the MN-major SWIZZLE_128B_BASE32B image of the weight-gradient
+//     MMAs, re-described as a K-major operand (rows = points, 128-byte rows of 32 out-features, 8-row group stride
+//     BwdArgs::dy_sbo = 512 B -- the one combination that reproduces the product exactly on hardware, tools/probe/umma_probe2.cu,
+//     profiles/r2a_umma_probe2.txt), so dY is stored to shared memory twice (hi, lo) instead of four times: 0.744 -> 0.686 ms
+//     per 1M points (profiles/r2a_mlp_variant_check.txt).
+// TMA (tiled feature layout only): the 66 KB of shared memory that frees become two 32 KB staging slots, and the stash / feature
+// rows of a phase (one contiguous 32 KB tile each, tc5_common.cuh) arrive by ONE bulk copy (cp.async.bulk -> UBLKCP, the TMA
+// engine) requested two phases ahead by the MMA-issuing thread and counted on the slot's mbarrier, instead of 8 LDG.128 per
+// thread held in registers across a phase: 0.686 -> 0.597 ms (profiles/r2i_mlp_variant_check.txt; d_out in registers on top
+// of it lost: 0.648).  Row-major features are read with the LDG.128 path (TMA = false).
+template <bool TMA>
 __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_constant__ BwdArgs a)
 {
-    constexpr bool A_NODIN = (ABL & 1) != 0, A_NOSTS = (ABL & 2) != 0, A_NOMMA = (ABL & 4) != 0, A_NOMATH = (ABL & 8) != 0,
-                   A_NODFEAT = (ABL & 16) != 0, A_NOLOAD = (ABL & 32) != 0;
-    constexpr bool V2 = (VER & 1) != 0, DIN_AHEAD = ((VER >> 1) & 3) == 1, DIN_PREFETCH = ((VER >> 1) & 3) >= 2, SINGLE_DY = ((VER >> 4) & 1) != 0, TMA = ((VER >> 5) & 1) != 0;
-    static_assert(!SINGLE_DY || V2, "the single dY image is built on the V2 kernel");
-    static_assert(!TMA || (SINGLE_DY && ABL == 0), "the TMA-staged rows live in the shared memory the single dY image frees");
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     float* W2B = reinterpret_cast<float*>(smem_raw);                 // current head: hi [16 k-chunks][64 n][4] | lo  (32 KB)
     float* W1B = W2B + 2 * MW * MW;                                  // hi | lo                                      (32 KB)
     unsigned char* DYM = smem_raw + 4 * MW * MW * 4;        // 64 KB, MN-major swizzled  [out: 64 hi rows | 64 lo rows][p 128]
     unsigned char* XH = DYM + 65536;                                 // 32 KB, MN-major swizzled  [in 64][p 128]
-    unsigned char* DYK = XH + 32768;              // 2 planes x 16 chunks x 2064 B, K-major  [p 128][out 64]
+    unsigned char* DYK = XH + 32768;              // 2 x 16 chunks x 2064 B: TMA staging slots / the D_RH bounce [p 128][in 64]
     u64* bar = reinterpret_cast<u64*>(DYK + 2 * KPLANE);
     u32* tmem_slot = reinterpret_cast<u32*>(bar + 3);          // bar[0]: MMA groups; bar[1], bar[2]: the two TMA staging slots
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -121,10 +115,6 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
         for (int i = 0; i < 8; ++i) cp_async16(reinterpret_cast<float4*>(dst) + tid + BT * i, src + tid + BT * i);
         cp_async_commit();
     };
-    if constexpr (!V2) {
-        copy_image_pair(W1B, 3);
-        cp_async_wait<0>();
-    }
     for (int i = tid; i < 98304 / 16; i += BT) reinterpret_cast<float4*>(DYM)[i] = make_float4(0.f, 0.f, 0.f, 0.f);   // DYM + XH
     if (tid == 0) {
         if (smem_u32(DYM) & 1023u) __trap();                          // the swizzle below assumes 1 KB aligned tiles
@@ -151,23 +141,23 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
     const u32 k_off = (u32)(8 * c + q) * KCH;
     const int p0 = 32 * pg + sub;                                     // point of iteration i: p0 + 4 i
     bool first_tile = true;
-    // V2: one MMA group (dX chain into d_col, weight gradient into w_col) issued by the elected lane of warp 0.  Called by
+    // One MMA group (dX chain into d_col, weight gradient into w_col) issued by the elected lane of warp 0.  Called by
     // every thread right after the block barrier, so warp 0 is converged; elect.sync picks the same lane every time, which
     // tcgen05.commit needs (it tracks the MMAs of the executing thread).  Descriptor start addresses are 14-bit fields of
     // (address >> 4) and shared memory ends below 256 KB, so adding (offset >> 4) to a hoisted base cannot carry out.
     auto issue_group = [&](u32 sW, u32 d_col, bool d_accumulate, u32 w_col, bool tma_go = false, const float* tma_src = nullptr, u32 tma_slot = 0) {
-        if (!A_NOMMA && warp == 0) {
+        if (warp == 0) {
             if (elect_one()) {
                 tc_fence_after();
                 const u64 dB = smem_desc(sW, MW * 16, 128);
-                const u64 dA = SINGLE_DY ? (smem_desc(sDYM, 16384, a.dy_sbo) | DESC_SW128_32B) : smem_desc(sDYK, KCH, 128);
+                const u64 dA = smem_desc(sDYM, 16384, a.dy_sbo) | DESC_SW128_32B;
                 const u64 dM = smem_desc(sDYM, 16384, 512) | DESC_SW128_32B, dX = smem_desc(sXH, 16384, 512) | DESC_SW128_32B;
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {          // K = 64 out features, 8 per instruction; lo*hi + hi*lo + hi*hi
                     const u64 bh = dB + (u64)((j * 2 * (MW * 16)) >> 4), bl = bh + (u64)((MW * MW * 4) >> 4);
-                    // SINGLE_DY: 8 out-features = one 32-byte step inside the 128-byte row, 32 out-features per 16 KB half; lo plane +32 KB
-                    const u64 ah = dA + (SINGLE_DY ? (u64)(((j >> 2) * 16384 + (j & 3) * 32) >> 4) : (u64)((j * 2 * KCH) >> 4));
-                    const u64 al = ah + (u64)((SINGLE_DY ? 32768u : KPLANE) >> 4);
+                    // 8 out-features = one 32-byte step inside the 128-byte row, 32 out-features per 16 KB half; lo plane +32 KB
+                    const u64 ah = dA + (u64)(((j >> 2) * 16384 + (j & 3) * 32) >> 4);
+                    const u64 al = ah + (u64)(32768u >> 4);
                     mma_ss(tbase + d_col, al, bh, id_kk, (d_accumulate || j > 0) ? 1u : 0u);
                     mma_ss(tbase + d_col, ah, bl, id_kk, 1u);
                     mma_ss(tbase + d_col, ah, bh, id_kk, 1u);
@@ -192,7 +182,7 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
     };
 
     u32 phase = 0;
-    u32 ngroup = 0;                  // V2: MMA groups committed so far; group n reads the weight slot n & 1 (0 = W2B, 1 = W1B)
+    u32 ngroup = 0;                  // MMA groups committed so far; group n reads the weight slot n & 1 (0 = W2B, 1 = W1B)
     bool pending = false;            // an MMA group has been committed and not yet waited for
     long long prev_row = -1;         // row (TMEM mapping) whose d_feature is still in D_FE
     float gW3[3][4][4], gB2[3][4], gB3[3][4], gB1[4];
@@ -207,7 +197,7 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
 #pragma unroll
     for (int e = 0; e < 4; ++e) gB1[e] = 0.f;
 
-    auto drain = [&](bool = true) {   // wait for the committed MMA group; then D_FE of the previous tile can be stored
+    auto drain = [&]() {   // wait for the committed MMA group; then D_FE of the previous tile can be stored
         if (pending) {
             mbar_wait(bar, phase); phase ^= 1; pending = false;
             tc_fence_after();
@@ -216,7 +206,7 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
             u32 v[32];
             tmem_ld32(lane_addr + C_FE + 32 * cT, v);
             tmem_wait_ld();
-            if (!A_NODFEAT && prev_row < a.P) {
+            if (prev_row < a.P) {
 #pragma unroll
                 for (int j = 0; j < 8; ++j)
                     *reinterpret_cast<float4*>(a.d_feat + (a.w.feat_tiled ? stash_off(prev_row, 32 * cT) + 16 * j : (size_t)prev_row * MW + 32 * cT + 4 * j)) =
@@ -259,16 +249,14 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
         const size_t step = a.w.feat_tiled ? 256 : 4 * MW;                       // rows r0 + 4 i
 #pragma unroll
         for (int i = 0; i < 8; ++i)
-            x[i] = A_NOLOAD ? make_float4(0.5f, 0.25f, 0.f, 1.f) :
-                   r0 + 4 * i < a.P ? __ldg(reinterpret_cast<const float4*>(base + step * i)) : make_float4(0.f, 0.f, 0.f, 0.f);
+            x[i] = r0 + 4 * i < a.P ? __ldg(reinterpret_cast<const float4*>(base + step * i)) : make_float4(0.f, 0.f, 0.f, 0.f);
     };
     auto load_stash = [&](float4* x, int plane, long long r0) {                  // tiled stash plane, see stash_off
         // r0 = tile * 128 + 32 pg + sub: the 8 rows r0 + 4 i are the same slot of 8 consecutive 4-point groups
         const float* src = a.saved + (size_t)plane * stash_plane_floats(a.P) + stash_off(r0, col0);
 #pragma unroll
         for (int i = 0; i < 8; ++i)
-            x[i] = A_NOLOAD ? make_float4(0.5f, 0.25f, 0.f, 1.f) :
-                   r0 + 4 * i < a.P ? __ldg(reinterpret_cast<const float4*>(src + 256 * i)) : make_float4(0.f, 0.f, 0.f, 0.f);
+            x[i] = r0 + 4 * i < a.P ? __ldg(reinterpret_cast<const float4*>(src + 256 * i)) : make_float4(0.f, 0.f, 0.f, 0.f);
     };
     auto load_phase_rows = [&](int ph, float4* x, long long r0) {
         if (ph >= 3) load_rows(x, a.feat, r0); else load_stash(x, 1 + ph, r0);
@@ -281,7 +269,7 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
         for (int i = 0; i < 8; ++i) {
             const long long r = r0 + 4 * i;
 #pragma unroll
-            for (int k = 0; k < 4; ++k) d[i][k] = A_NODIN ? 0.25f * (float)(k + 1) : (r < a.P && dsrc && k < kd) ? __ldg(dsrc + (size_t)r * kd + k) : 0.f;
+            for (int k = 0; k < 4; ++k) d[i][k] = (r < a.P && dsrc && k < kd) ? __ldg(dsrc + (size_t)r * kd + k) : 0.f;
         }
     };
 
@@ -293,8 +281,7 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
         if (!dsrc || tid > 4 * kd) return;                                   // 128 * kd * 4 bytes = 4 kd lines (+1: unaligned base)
         const char* p = reinterpret_cast<const char*>(dsrc + (size_t)tile * ROWS * kd) + 128 * tid;
         if (p >= reinterpret_cast<const char*>(dsrc + (size_t)a.P * kd)) return;
-        if constexpr (((VER >> 1) & 3) == 2) asm volatile("prefetch.global.L1 [%0];" :: "l"(p));
-        else asm volatile("prefetch.global.L2 [%0];" :: "l"(p));
+        asm volatile("prefetch.global.L2 [%0];" :: "l"(p));
     };
     const long long nblocks = (a.P + ROWS - 1) / ROWS;
     float4 hrow[8], xin[8];
@@ -313,9 +300,7 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
             iss_advance();
         }
     }
-    if constexpr (V2) copy_image_pair(W2B, next_phase(-1));            // group 0's weights -> slot 0 (waited for before its MMAs)
-    float din_next[8][4];
-    if constexpr (DIN_AHEAD) load_phase_dout(next_phase(-1), din_next, (long long)blockIdx.x * ROWS + p0);
+    copy_image_pair(W2B, next_phase(-1));            // group 0's weights -> slot 0 (waited for before its MMAs)
     for (long long blk = blockIdx.x; blk < nblocks; blk += gridDim.x) {
         const long long row0 = blk * ROWS + p0;
         // ---- relu(hidden): sign mask for dh + B operand of dW2 ----
@@ -334,19 +319,13 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
 #pragma unroll
             for (int k = 0; k < 4; ++k) w3[k] = k < kd ? __ldg(reinterpret_cast<const float4*>(a.w.w3[h] + k * MW + col0)) : make_float4(0.f, 0.f, 0.f, 0.f);
             float din[8][4];
-            if constexpr (DIN_AHEAD) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i)
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) din[i][k] = din_next[i][k];
-            } else load_phase_dout(h, din, row0);
+            load_phase_dout(h, din, row0);
             float dz[8][4];
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 const float zz[4] = {xin[i].x, xin[i].y, xin[i].z, xin[i].w};
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
-                    if constexpr (A_NOMATH) { dz[i][e] = zz[e] + din[i][e]; continue; }
                     const float wk[4] = {e == 0 ? w3[0].x : e == 1 ? w3[0].y : e == 2 ? w3[0].z : w3[0].w,
                                          e == 0 ? w3[1].x : e == 1 ? w3[1].y : e == 2 ? w3[1].z : w3[1].w,
                                          e == 0 ? w3[2].x : e == 1 ? w3[2].y : e == 2 ? w3[2].z : w3[2].w,
@@ -361,20 +340,18 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
                     for (int k = 0; k < 4; ++k)
                         if (k < kd) gW3[h][k][e] = fmaf(din[i][k], zz[e], gW3[h][k][e]);
                 }
-                if (!A_NOMATH && q == 0 && c == 0) {
+                if (q == 0 && c == 0) {
 #pragma unroll
                     for (int k = 0; k < 4; ++k) gB3[h][k] += din[i][k];
                 }
             }
             if constexpr (!TMA) load_phase_rows(next_phase(h), xin, row0);          // next head's rows, or the feature rows
-            if constexpr (DIN_AHEAD) load_phase_dout(next_phase(h), din_next, row0);        // (nothing for the feature phase)
-            if constexpr (DIN_PREFETCH) prefetch_phase_dout(next_phase(h), blk);
-            drain(false);            // the previous MMA group still reads DYK / DYM / XH and the W2 slot
-            if constexpr (!V2) copy_image_pair(W2B, h);
-            else copy_image_pair((ngroup & 1u) ? W2B : W1B, next_phase(h));   // the NEXT group's image -> the slot the drained group used
+            prefetch_phase_dout(next_phase(h), blk);                                   // (nothing for the feature phase)
+            drain();                 // the previous MMA group still reads DYK / DYM / XH and the W2 slot
+            copy_image_pair((ngroup & 1u) ? W2B : W1B, next_phase(h));   // the NEXT group's image -> the slot the drained group used
             if (!h_staged) {
 #pragma unroll
-                for (int i = 0; i < 8; ++i) if (!A_NOSTS || i == 0) sts128(sXH + mn_off + (u32)(p0 + 4 * i) * 128u, tf32x4(hrow[i]));
+                for (int i = 0; i < 8; ++i) sts128(sXH + mn_off + (u32)(p0 + 4 * i) * 128u, tf32x4(hrow[i]));
                 h_staged = true;
             }
 #pragma unroll
@@ -382,39 +359,18 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
                 const u32 pp = (u32)(p0 + 4 * i);
                 float4 hi, lo;
                 split4(dz[i], hi, lo);
-                if constexpr (A_NOSTS) { if (i > 0 || hi.x + lo.y != 12345.678f) continue; }     // keeps dz alive, stores (almost) never
-                if constexpr (!SINGLE_DY) {
-                    sts128(sDYK + k_off + pp * 16u, hi);
-                    sts128(sDYK + KPLANE + k_off + pp * 16u, lo);
-                }
                 sts128(sDYM + mn_off + pp * 128u, hi);
                 sts128(sDYM + 32768u + mn_off + pp * 128u, lo);
             }
-            if constexpr (V2) cp_async_wait<1>(); else cp_async_wait<0>();      // V2: all but the next group's image
+            cp_async_wait<1>();      // all but the next group's image
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             tc_fence_before();
             __syncthreads();
-            if constexpr (V2) {
-                const bool go = TMA && iss_tile < nblocks;
-                issue_group((ngroup & 1u) ? sW1 : sW2, C_RH, rh_started, C_W2 + 64 * h, go, go ? tma_src_of(iss_tile, iss_ph) : nullptr, n_iss & 1u);
-                if constexpr (TMA) iss_advance();
-                ++ngroup;
-            } else if (tid == 0) {
-                tc_fence_after();
-                for (int j = 0; j < 8; ++j) {          // K = 64 out features, 8 per instruction; lo*hi + hi*lo + hi*hi
-                    const u64 bh = smem_desc(sW2 + j * 2 * (MW * 16), MW * 16, 128);
-                    const u64 bl = smem_desc(sW2 + MW * MW * 4 + j * 2 * (MW * 16), MW * 16, 128);
-                    const u64 ah = smem_desc(sDYK + j * 2 * KCH, KCH, 128), al = smem_desc(sDYK + KPLANE + j * 2 * KCH, KCH, 128);
-                    mma_ss(tbase + C_RH, al, bh, id_kk, (rh_started || j > 0) ? 1u : 0u);
-                    mma_ss(tbase + C_RH, ah, bl, id_kk, 1u);
-                    mma_ss(tbase + C_RH, ah, bh, id_kk, 1u);
-                }
-                for (int j = 0; j < 16; ++j)           // K = 128 points, 8 per instruction (two 4-row atoms)
-                    mma_ss(tbase + C_W2 + 64 * h, smem_desc(sDYM + j * 1024, 16384, 512) | DESC_SW128_32B,
-                           smem_desc(sXH + j * 1024, 16384, 512) | DESC_SW128_32B, id_mn, (first_tile && j == 0) ? 0u : 1u);
-                tc_commit(bar);
-            }
-            pending = !A_NOMMA;
+            const bool go = TMA && iss_tile < nblocks;
+            issue_group((ngroup & 1u) ? sW1 : sW2, C_RH, rh_started, C_W2 + 64 * h, go, go ? tma_src_of(iss_tile, iss_ph) : nullptr, n_iss & 1u);
+            if constexpr (TMA) iss_advance();
+            ++ngroup;
+            pending = true;
             rh_started = true;
         }
         // ---- dh = d relu(hidden) masked ; d feature = dh W1 ; dW1 += dh^T feature ----
@@ -426,14 +382,12 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
         if (blk + gridDim.x < nblocks) {                              // next tile: relu(hidden) rows and the first phase's inputs
             load_stash(hrow, 0, (blk + gridDim.x) * ROWS + p0);
             if constexpr (!TMA) load_phase_rows(next_phase(-1), xin, (blk + gridDim.x) * ROWS + p0);
-            if constexpr (DIN_AHEAD) load_phase_dout(next_phase(-1), din_next, (blk + gridDim.x) * ROWS + p0);
-            if constexpr (DIN_PREFETCH) prefetch_phase_dout(next_phase(-1), blk + gridDim.x);
+            prefetch_phase_dout(next_phase(-1), blk + gridDim.x);
         }
         drain();
-        if constexpr (V2) {          // the next tile's first image -> the slot the drained group used (an empty group keeps the count)
-            if (blk + gridDim.x < nblocks) copy_image_pair((ngroup & 1u) ? W2B : W1B, next_phase(-1));
-            else cp_async_commit();
-        }
+        // the next tile's first image -> the slot the drained group used (an empty group keeps the count)
+        if (blk + gridDim.x < nblocks) copy_image_pair((ngroup & 1u) ? W2B : W1B, next_phase(-1));
+        else cp_async_commit();
         // TMA: the bounce goes through the staging slot the feature rows were just read from (every thread has them in registers
         // once the barrier below has been passed); the next request for that slot is issued after this phase's last barrier
         const u32 sBounce = TMA ? sDYK + ((n_cons - 1u) & 1u) * KPLANE : sDYK;
@@ -466,40 +420,19 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
             }
             float4 hi, lo;
             split4(x, hi, lo);
-            if constexpr (A_NOSTS) { if (i > 0 || hi.x + lo.y + frow[i].x != 12345.678f) continue; }
-            if constexpr (!SINGLE_DY) {
-                sts128(sDYK + k_off + pp * 16u, hi);
-                sts128(sDYK + KPLANE + k_off + pp * 16u, lo);
-            }
             sts128(sDYM + mn_off + pp * 128u, hi);
             sts128(sDYM + 32768u + mn_off + pp * 128u, lo);
             sts128(sXH + mn_off + pp * 128u, tf32x4(frow[i]));
         }
-        if constexpr (V2) cp_async_wait<1>();
+        cp_async_wait<1>();
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         tc_fence_before();
         __syncthreads();
-        if constexpr (V2) {
-            const bool go = TMA && iss_tile < nblocks;
-            issue_group((ngroup & 1u) ? sW1 : sW2, C_FE, false, C_W1, go, go ? tma_src_of(iss_tile, iss_ph) : nullptr, n_iss & 1u);
-            if constexpr (TMA) iss_advance();
-            ++ngroup;
-        } else if (tid == 0) {
-            tc_fence_after();
-            for (int j = 0; j < 8; ++j) {
-                const u64 bh = smem_desc(sW1 + j * 2 * (MW * 16), MW * 16, 128);
-                const u64 bl = smem_desc(sW1 + MW * MW * 4 + j * 2 * (MW * 16), MW * 16, 128);
-                const u64 ah = smem_desc(sDYK + j * 2 * KCH, KCH, 128), al = smem_desc(sDYK + KPLANE + j * 2 * KCH, KCH, 128);
-                mma_ss(tbase + C_FE, al, bh, id_kk, j > 0 ? 1u : 0u);
-                mma_ss(tbase + C_FE, ah, bl, id_kk, 1u);
-                mma_ss(tbase + C_FE, ah, bh, id_kk, 1u);
-            }
-            for (int j = 0; j < 16; ++j)
-                mma_ss(tbase + C_W1, smem_desc(sDYM + j * 1024, 16384, 512) | DESC_SW128_32B,
-                       smem_desc(sXH + j * 1024, 16384, 512) | DESC_SW128_32B, id_mn, (first_tile && j == 0) ? 0u : 1u);
-            tc_commit(bar);
-        }
-        pending = !A_NOMMA;
+        const bool go = TMA && iss_tile < nblocks;
+        issue_group((ngroup & 1u) ? sW1 : sW2, C_FE, false, C_W1, go, go ? tma_src_of(iss_tile, iss_ph) : nullptr, n_iss & 1u);
+        if constexpr (TMA) iss_advance();
+        ++ngroup;
+        pending = true;
         prev_row = blk * ROWS + pT;
         first_tile = false;
     }
@@ -508,42 +441,30 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
     // ---- flush ----
     if (!first_tile) {
         // TMEM-resident weight gradients: lanes 0..63 = out feature from dY_hi, lanes 64..127 the same from dY_lo
-        if constexpr (V2) {
-            // through shared memory (DYM is free: every MMA has completed), rows padded to 68 floats so that both the
-            // lane-per-row 128-bit stores and the row-contiguous 128-bit loads are conflict free; then hi + lo row pairs
-            // leave as one 128-bit RED per 4 elements, 512 contiguous bytes per warp.  CTAs start at different matrices /
-            // row blocks so that the 148 of them do not all hit the same lines at once.
-            constexpr u32 SP = 68 * 4;
-            for (int mi = 0; mi < 4; ++mi) {
-                const int m = (mi + (int)blockIdx.x) & 3;
-                if (m < 3 && !a.w.w2[m]) continue;
-                float* dst = m < 3 ? a.gw.w2[m] : a.gw.w1;
-                u32 v[32];
-                tmem_ld32(lane_addr + (m < 3 ? C_W2 + 64 * m : C_W1) + 32 * cT, v);
-                tmem_wait_ld();
-                __syncthreads();                                  // the previous matrix has been read out of the staging rows
+        // through shared memory (DYM is free: every MMA has completed), rows padded to 68 floats so that both the
+        // lane-per-row 128-bit stores and the row-contiguous 128-bit loads are conflict free; then hi + lo row pairs
+        // leave as one 128-bit RED per 4 elements, 512 contiguous bytes per warp.  CTAs start at different matrices /
+        // row blocks so that the 148 of them do not all hit the same lines at once.
+        constexpr u32 SP = 68 * 4;
+        for (int mi = 0; mi < 4; ++mi) {
+            const int m = (mi + (int)blockIdx.x) & 3;
+            if (m < 3 && !a.w.w2[m]) continue;
+            float* dst = m < 3 ? a.gw.w2[m] : a.gw.w1;
+            u32 v[32];
+            tmem_ld32(lane_addr + (m < 3 ? C_W2 + 64 * m : C_W1) + 32 * cT, v);
+            tmem_wait_ld();
+            __syncthreads();                                  // the previous matrix has been read out of the staging rows
 #pragma unroll
-                for (int j = 0; j < 8; ++j)
-                    sts128(sDYM + (u32)pT * SP + (u32)(32 * cT + 4 * j) * 4u,
-                           make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]), __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3])));
-                __syncthreads();
+            for (int j = 0; j < 8; ++j)
+                sts128(sDYM + (u32)pT * SP + (u32)(32 * cT + 4 * j) * 4u,
+                       make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]), __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3])));
+            __syncthreads();
 #pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const int idx = tid + BT * ((k + (int)(blockIdx.x >> 2)) & 3);      // 1024 float4 = 64 rows x 16
-                    const int r = idx >> 4, c4 = idx & 15;
-                    const float4 x = lds128(sDYM + (u32)r * SP + (u32)c4 * 16u), y = lds128(sDYM + (u32)(r + 64) * SP + (u32)c4 * 16u);
-                    red_add_v4(dst + r * MW + 4 * c4, x.x + y.x, x.y + y.y, x.z + y.z, x.w + y.w);
-                }
-            }
-        } else {
-            for (int m = 0; m < 4; ++m) {
-                if (m < 3 && !a.w.w2[m]) continue;
-                float* dst = m < 3 ? a.gw.w2[m] : a.gw.w1;
-                u32 v[32];
-                tmem_ld32(lane_addr + (m < 3 ? C_W2 + 64 * m : C_W1) + 32 * cT, v);
-                tmem_wait_ld();
-#pragma unroll
-                for (int e = 0; e < 32; ++e) atomicAdd(dst + (pT & 63) * MW + 32 * cT + e, __uint_as_float(v[e]));
+            for (int k = 0; k < 4; ++k) {
+                const int idx = tid + BT * ((k + (int)(blockIdx.x >> 2)) & 3);      // 1024 float4 = 64 rows x 16
+                const int r = idx >> 4, c4 = idx & 15;
+                const float4 x = lds128(sDYM + (u32)r * SP + (u32)c4 * 16u), y = lds128(sDYM + (u32)(r + 64) * SP + (u32)c4 * 16u);
+                red_add_v4(dst + r * MW + 4 * c4, x.x + y.x, x.y + y.y, x.z + y.z, x.w + y.w);
             }
         }
         // register-resident partial sums: fold the 4 `sub` lanes, then one atomic per column per warp
@@ -591,6 +512,10 @@ int deform_mlp_backward_tc5(const b200gs_mlp_weights* w, const b200gs_mlp_grads*
                             const float* saved, const float* d_pts, const float* d_scales, const float* d_rot,
                             float* d_feat, cudaStream_t stream)
 {
+    // the weight gradients leave as 128-bit REDs (see the flush above): W1 / W2 gradient rows must be 16-byte aligned
+    bool aligned = ((uintptr_t)gw->w1 & 15) == 0;
+    for (int h = 0; h < 3; ++h) aligned = aligned && (!w->w2[h] || ((uintptr_t)gw->w2[h] & 15) == 0);
+    if (!aligned) { set_error("deform_mlp_backward: gw->w1 / gw->w2 must be 16-byte aligned"); return -1; }
     tc5::BwdArgs a;
     a.w = *w; a.gw = *gw; a.P = P; a.feat = feat; a.saved = saved; a.d_pts = d_pts; a.d_scales = d_scales; a.d_rot = d_rot;
     a.d_feat = d_feat; a.dy_sbo = 512u;
@@ -598,48 +523,10 @@ int deform_mlp_backward_tc5(const b200gs_mlp_weights* w, const b200gs_mlp_grads*
     const int sms = g_opt_mlp_bwd_sms > 0 && g_opt_mlp_bwd_sms < NUM_SMS ? g_opt_mlp_bwd_sms : NUM_SMS;          // option: leave a few SMs to a concurrent stream
     const int grid = (int)(nblocks < sms ? nblocks : sms);
     const size_t smem = tc5::bwd_smem();
-    // experimental variant (see the kernel's header comment): opt-in until it has been measured on the GPU; needs 16-byte
-    // aligned W1 / W2 gradient rows for its 128-bit REDs
-    bool v2 = g_opt_mlp_bwd_v2 != 0 && ((uintptr_t)gw->w1 & 15) == 0;
-    for (int h = 0; h < 3; ++h) v2 = v2 && (!w->w2[h] || ((uintptr_t)gw->w2[h] & 15) == 0);
-    if (v2 && g_opt_mlp_bwd_ablate != 0) {           // timing experiments, wrong results (see the kernel's ABL comment)
-        void (*kern)(tc5::BwdArgs) = nullptr;
-        switch (g_opt_mlp_bwd_ablate) {
-            case 1: kern = tc5::deform_mlp_bwd_tc5_kernel<7, 1>; break;
-            case 2: kern = tc5::deform_mlp_bwd_tc5_kernel<7, 2>; break;
-            case 4: kern = tc5::deform_mlp_bwd_tc5_kernel<7, 4>; break;
-            case 8: kern = tc5::deform_mlp_bwd_tc5_kernel<7, 8>; break;
-            case 16: kern = tc5::deform_mlp_bwd_tc5_kernel<7, 16>; break;
-            case 32: kern = tc5::deform_mlp_bwd_tc5_kernel<7, 32>; break;
-            case 10: kern = tc5::deform_mlp_bwd_tc5_kernel<7, 10>; break;
-            default: set_error("deform_mlp_backward: mlp_bwd_ablate = %d is not built", g_opt_mlp_bwd_ablate); return -1;
-        }
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        kern<<<grid, tc5::BT, smem, stream>>>(a);
-        return check_launch("deform_mlp_backward(tcgen05 v2, ablation)");
-    }
-    if (v2) {
-        void (*kern)(tc5::BwdArgs) = tc5::deform_mlp_bwd_tc5_kernel<1>;
-        switch (g_opt_mlp_bwd_v2) {          // see the kernel's VER comment
-            case 3: kern = tc5::deform_mlp_bwd_tc5_kernel<3>; break;
-            case 5: kern = tc5::deform_mlp_bwd_tc5_kernel<5>; break;
-            case 7: kern = tc5::deform_mlp_bwd_tc5_kernel<7>; break;
-            // 55 (default): ONE dY image -- the dX chain reads the MN-major SWIZZLE_128B_BASE32B image of the weight-gradient
-            // MMAs re-described as a K-major operand with a 512-byte 8-row group stride (exact on hardware: tools/probe/umma_probe2.cu,
-            // profiles/r2a_umma_probe2.txt; the 1024-byte stride is NOT and was removed)
-            case 55: kern = tc5::deform_mlp_bwd_tc5_kernel<23>; break;
-            // 87 = 55 + the stash / feature rows of a phase staged by ONE 32 KB bulk copy (TMA engine) two phases ahead instead
-            // of 8 LDG.128 per thread one phase ahead; needs the tiled feature layout (falls back to 55 otherwise)
-            case 87: kern = w->feat_tiled ? tc5::deform_mlp_bwd_tc5_kernel<55> : tc5::deform_mlp_bwd_tc5_kernel<23>; break;
-            default: set_error("deform_mlp_backward: mlp_bwd_v2 = %d is not built (0, 1, 3, 5, 7, 55, 87)", g_opt_mlp_bwd_v2); return -1;
-            case 1: break;
-        }
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        kern<<<grid, tc5::BT, smem, stream>>>(a);
-        return check_launch("deform_mlp_backward(tcgen05 v2)");
-    }
-    cudaFuncSetAttribute(tc5::deform_mlp_bwd_tc5_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    tc5::deform_mlp_bwd_tc5_kernel<0><<<grid, tc5::BT, smem, stream>>>(a);
+    // the TMA staging needs the tiled feature layout (one contiguous 32 KB tile per phase)
+    void (*kern)(tc5::BwdArgs) = w->feat_tiled ? tc5::deform_mlp_bwd_tc5_kernel<true> : tc5::deform_mlp_bwd_tc5_kernel<false>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    kern<<<grid, tc5::BT, smem, stream>>>(a);
     return check_launch("deform_mlp_backward(tcgen05)");
 }
 

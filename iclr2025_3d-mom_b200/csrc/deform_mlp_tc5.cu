@@ -277,15 +277,14 @@ __device__ __forceinline__ void stage_kmajor2(float* __restrict__ hi, float* __r
     }
 }
 
-// ELECT (experimental, off by default: b200gs_set_option("mlp_fwd_elect", 1) or B200GS_MLP_FWD_ELECT=1): the MMAs are issued from a warp-uniform branch by the elected lane
-// of warp 0 (tc5_common.cuh elect_one) instead of `if (tid == 0)`, which makes the compiler wrap every tcgen05.mma in an
-// ELECT / BRA.U.ANY loop; same instructions, same order, same issuing thread.
-// MODE 0: default; 1: ELECT; 2: ELECT + the activation-stash stores of a layer are issued AFTER the next layer's MMAs have been
-// started (they are not on the MMA -> epilogue -> MMA chain, the values just stay in registers a little longer).
-template <int F, int MODE>
+// The MMAs are issued from a warp-uniform branch by the elected lane of warp 0 (tc5_common.cuh elect_one): `if (tid == 0)`
+// makes the compiler wrap every tcgen05.mma in an ELECT / BRA.U.ANY loop.  The activation-stash stores of a layer are issued
+// AFTER the next layer's MMAs have been started: they are not on the MMA -> epilogue -> MMA chain, the values just stay in
+// registers a little longer.  Neither changes a computed value (same MMAs in the same order, the same stores later); for
+// F = 128 they took the forward from 498 to 405 us per 1M points (B200, 1000 W power limit, tools/time_mlp.py MULTIRES=1,2,4,8).
+template <int F>
 __global__ void __launch_bounds__(NT2, 1) deform_mlp_fwd_tc5v2_kernel(const __grid_constant__ FwdArgs a)
 {
-    constexpr bool ELECT = MODE >= 1, DEFER_STASH = MODE >= 2;
     extern __shared__ __align__(1024) float smem[];
     float* W1h = smem;                         // [F/4][64][4]
     float* W1l = W1h + MW * F;
@@ -336,29 +335,19 @@ __global__ void __launch_bounds__(NT2, 1) deform_mlp_fwd_tc5v2_kernel(const __gr
 
     auto sync_then = [&]() { tmem_wait_st(); tc_fence_before(); __syncthreads(); };
     // the thread that issues the MMAs; every call site follows a block barrier, so warp 0 is converged for elect.sync
-    auto issuer = [&]() -> bool {
-        if constexpr (ELECT) return warp == 0 && elect_one();
-        else return tid == 0;
-    };
-    // epilogue of one 64-wide layer for this thread's 32 columns: bias, ReLU, stash, split; returns hi / lo in v / lo
-    auto layer_epilogue = [&](u32 d_col, const float* b, float* stash_plane, long long row, bool valid, u32* v, u32* lo) {
+    auto issuer = [&]() -> bool { return warp == 0 && elect_one(); };
+    // epilogue of one 64-wide layer for this thread's 32 columns: bias, ReLU, split; returns hi / lo in v / lo
+    auto layer_epilogue = [&](u32 d_col, const float* b, u32* v, u32* lo) {
         tmem_ld32(lane_addr + d_col + 32 * cT, v);
         tmem_wait_ld();
 #pragma unroll
         for (int e = 0; e < 32; ++e) v[e] = __float_as_uint(fmaxf(__uint_as_float(v[e]) + b[32 * cT + e], 0.f));
-        if (valid && !DEFER_STASH && stash_on) {
-            float* dst = stash_plane + stash_off(row, 32 * cT);          // this thread's 8 chunks are 16 floats apart
-#pragma unroll
-            for (int j = 0; j < 8; ++j)
-                *reinterpret_cast<float4*>(dst + 16 * j) =
-                    make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]), __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-        }
 #pragma unroll
         for (int e = 0; e < 32; ++e) lo[e] = __float_as_uint(tf32_lo(__uint_as_float(v[e])));      // hi = the raw value (hardware truncates)
     };
     auto deferred_stash = [&](float* stash_plane, long long row, bool valid, const u32* v) {
-        if (DEFER_STASH && valid && stash_on) {
-            float* dst = stash_plane + stash_off(row, 32 * cT);
+        if (valid && stash_on) {
+            float* dst = stash_plane + stash_off(row, 32 * cT);          // this thread's 8 chunks are 16 floats apart
 #pragma unroll
             for (int j = 0; j < 8; ++j)
                 *reinterpret_cast<float4*>(dst + 16 * j) =
@@ -417,7 +406,7 @@ __global__ void __launch_bounds__(NT2, 1) deform_mlp_fwd_tc5v2_kernel(const __gr
         // ---- hidden ----
         mbar_wait(bars + 0, parity);
         tc_fence_after();
-        layer_epilogue(C_D2, bias, a.saved, r, valid, v, lo);
+        layer_epilogue(C_D2, bias, v, lo);
         tmem_st32(lane_addr + C_H_HI + 32 * cT, v);
         tmem_st32(lane_addr + C_H_LO + 32 * cT, lo);
         sync_then();
@@ -434,7 +423,7 @@ __global__ void __launch_bounds__(NT2, 1) deform_mlp_fwd_tc5v2_kernel(const __gr
         for (int h = 0; h < 3; ++h) {
             mbar_wait(bars + 1 + h, parity);
             tc_fence_after();
-            layer_epilogue(C_D2 + 64 * h, bias + MW + h * MW, a.saved + (size_t)(1 + h) * stash_plane_floats(a.P), r, valid, v, lo);
+            layer_epilogue(C_D2 + 64 * h, bias + MW + h * MW, v, lo);
             if (h > 0) {                         // the previous head's last layer still reads Z
                 mbar_wait(bars + 4 + (h - 1), parity);
                 tc_fence_after();
@@ -520,19 +509,12 @@ int deform_mlp_forward_tc5(const b200gs_mlp_weights* w, long long P, const float
         return -1;
     }
     if (w->w2[0] && w->w2[1] && w->w2[2]) {          // all heads on (the reference's configuration): pipelined kernel
-        // experimental issue idiom (see the kernel's comment): opt-in until it has been measured on the GPU
-        if (g_opt_mlp_fwd_elect != 0 && w->feat_dim == 64) {
-            void (*kern)(tc5::FwdArgs) = g_opt_mlp_fwd_elect >= 2 ? tc5::deform_mlp_fwd_tc5v2_kernel<64, 2> : tc5::deform_mlp_fwd_tc5v2_kernel<64, 1>;
-            cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            kern<<<grid, tc5::NT2, smem, stream>>>(a);
-            return check_launch("deform_mlp_forward(tcgen05 v2, elected issuer)");
-        }
         if (w->feat_dim == 64) {
-            cudaFuncSetAttribute(tc5::deform_mlp_fwd_tc5v2_kernel<64, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            tc5::deform_mlp_fwd_tc5v2_kernel<64, 0><<<grid, tc5::NT2, smem, stream>>>(a);
+            cudaFuncSetAttribute(tc5::deform_mlp_fwd_tc5v2_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            tc5::deform_mlp_fwd_tc5v2_kernel<64><<<grid, tc5::NT2, smem, stream>>>(a);
         } else {
-            cudaFuncSetAttribute(tc5::deform_mlp_fwd_tc5v2_kernel<128, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            tc5::deform_mlp_fwd_tc5v2_kernel<128, 0><<<grid, tc5::NT2, smem, stream>>>(a);
+            cudaFuncSetAttribute(tc5::deform_mlp_fwd_tc5v2_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            tc5::deform_mlp_fwd_tc5v2_kernel<128><<<grid, tc5::NT2, smem, stream>>>(a);
         }
         return check_launch("deform_mlp_forward(tcgen05 v2)");
     }

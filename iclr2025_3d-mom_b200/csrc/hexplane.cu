@@ -430,11 +430,11 @@ hexplane_time_fwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, const _
     }
 }
 
-// Opt-in variant ("hexplane_time_fwd" = 1 / 2, unmeasured): compile-time 2 levels, both levels' factor rows requested before the
-// first is used, both feature rows stored at the end; same arithmetic per element as the kernel above.  MINB = resident CTAs per
-// SM the register budget is set for (3: 42 registers like the kernel above, 2: no cap).
-template <int MINB>
-__global__ void __launch_bounds__(512, MINB)
+// 2 levels (the reference's configuration): compile-time level count, both levels' factor rows requested before the first is
+// used, both feature rows stored at the end; same arithmetic per element as the kernel above, bit-identical features.  The
+// register budget is set for 2 resident CTAs per SM (the kernel above is capped at 42 registers for 3):
+// 0.134 -> 0.112 ms (profiles/r2a_hexplane_time_check.txt).
+__global__ void __launch_bounds__(512, 2)
 hexplane_time_fwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const __grid_constant__ TimeRowSetup ts, long long P,
                           const float* __restrict__ pts, const unsigned int* __restrict__ order, float t,
                           const float* __restrict__ factor, float* __restrict__ feat, int tiled)
@@ -540,13 +540,12 @@ hexplane_time_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, const _
     }
 }
 
-// Opt-in variant ("hexplane_time_bwd" = 1 / 2, unmeasured): same arithmetic per element as the kernel above, but the level
-// count is a compile-time 2, so both levels' d_feature / factor / d_factor rows of a point group are requested before the
-// first one is used (the kernel above waits for one level's rows, works, then requests the next: two exposed memory
-// latencies per iteration -- 66 % of its stall samples are the first use of a load).  MINB = resident CTAs per SM the
-// register budget is set for (3: 85 registers, 2: 128 registers and a third fewer warps).
-template <int MINB>
-__global__ void __launch_bounds__(256, MINB)
+// 2 levels (the reference's configuration): same arithmetic per element as the kernel above, but the level count is a
+// compile-time 2, so both levels' d_feature / factor / d_factor rows of a point group are requested before the first one is
+// used (the kernel above waits for one level's rows, works, then requests the next: two exposed memory latencies per
+// iteration -- 66 % of its stall samples are the first use of a load).  The register budget is set for 2 resident CTAs per
+// SM (128 registers and a third fewer warps than 3 at 85 registers): 0.417 -> 0.354 ms (profiles/r2a_hexplane_time_check.txt).
+__global__ void __launch_bounds__(256, 2)
 hexplane_time_bwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const __grid_constant__ TimeRowSetup ts, long long P,
                           const float* __restrict__ pts, const unsigned int* __restrict__ order, float t,
                           const float* __restrict__ factor, float* __restrict__ dfactor, const float* __restrict__ dfeat,
@@ -865,17 +864,17 @@ int b200gs_hexplane_time_forward(const b200gs_hexplane_desc* desc, long long P, 
     if (!time_rows_setup(*desc, ts)) { set_error("hexplane_time_forward: time rows do not fit shared memory"); return -1; }
     if (P <= 0) return 0;
     const size_t smem = (size_t)ts.total * sizeof(float);
-    cudaFuncSetAttribute(hexplane_time_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     long long blocks = (P + 63) / 64;                // 16 warps x 4 point slots per block; the kernels are latency bound, so as many warps as fit
     const long long cap = (long long)NUM_SMS * (smem * 3 <= 220 * 1024 ? 3 : (smem * 2 <= 220 * 1024 ? 2 : 1));
     if (blocks > cap) blocks = cap;
-    if (g_opt_hexplane_time_fwd != 0 && desc->levels == 2) {            // opt-in variant, see hexplane_time_fwd2_kernel
-        auto kern = g_opt_hexplane_time_fwd == 2 ? hexplane_time_fwd2_kernel<2> : hexplane_time_fwd2_kernel<3>;
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (g_opt_hexplane_time_fwd == 2 && blocks > (long long)NUM_SMS * 2) blocks = (long long)NUM_SMS * 2;
-        kern<<<(unsigned)blocks, 512, smem, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, features, features_tiled);
-    } else
-    hexplane_time_fwd_kernel<<<(unsigned)blocks, 512, smem, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, features, features_tiled);
+    if (desc->levels == 2) {                         // see hexplane_time_fwd2_kernel: 2 resident CTAs per SM
+        cudaFuncSetAttribute(hexplane_time_fwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (blocks > (long long)NUM_SMS * 2) blocks = (long long)NUM_SMS * 2;
+        hexplane_time_fwd2_kernel<<<(unsigned)blocks, 512, smem, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, features, features_tiled);
+    } else {
+        cudaFuncSetAttribute(hexplane_time_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        hexplane_time_fwd_kernel<<<(unsigned)blocks, 512, smem, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, features, features_tiled);
+    }
     return check_launch("hexplane_time_forward");
 }
 
@@ -895,19 +894,19 @@ int b200gs_hexplane_time_backward(const b200gs_hexplane_desc* desc, long long P,
     if (replicas < 1) { set_error("hexplane_time_backward: scratch for at least one row replica is required"); return -1; }
     float* rows = (float*)time_row_scratch;
     cudaMemsetAsync(rows, 0, per * replicas, (cudaStream_t)stream);
-    cudaFuncSetAttribute(hexplane_time_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)per);
     long long blocks = (P + 31) / 32;
     const long long cap = (long long)NUM_SMS * (per * 3 <= 220 * 1024 ? 3 : (per * 2 <= 220 * 1024 ? 2 : 1));
     if (blocks > cap) blocks = cap;
-    if (g_opt_hexplane_time_bwd != 0 && desc->levels == 2) {            // opt-in variant, see hexplane_time_bwd2_kernel
-        auto kern = g_opt_hexplane_time_bwd == 2 ? hexplane_time_bwd2_kernel<2> : hexplane_time_bwd2_kernel<3>;
-        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)per);
-        if (g_opt_hexplane_time_bwd == 2 && blocks > (long long)NUM_SMS * 2) blocks = (long long)NUM_SMS * 2;
-        kern<<<(unsigned)blocks, 256, per, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, d_factor_accum,
-                                                                 d_features, d_pts, rows, replicas, d_features_tiled);
-    } else
-    hexplane_time_bwd_kernel<<<(unsigned)blocks, 256, per, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, d_factor_accum,
-                                                                                   d_features, d_pts, rows, replicas, d_features_tiled);
+    if (desc->levels == 2) {                         // see hexplane_time_bwd2_kernel: 2 resident CTAs per SM
+        cudaFuncSetAttribute(hexplane_time_bwd2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)per);
+        if (blocks > (long long)NUM_SMS * 2) blocks = (long long)NUM_SMS * 2;
+        hexplane_time_bwd2_kernel<<<(unsigned)blocks, 256, per, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, d_factor_accum,
+                                                                                        d_features, d_pts, rows, replicas, d_features_tiled);
+    } else {
+        cudaFuncSetAttribute(hexplane_time_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)per);
+        hexplane_time_bwd_kernel<<<(unsigned)blocks, 256, per, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, d_factor_accum,
+                                                                                       d_features, d_pts, rows, replicas, d_features_tiled);
+    }
     hexplane_time_rows_flush_kernel<<<(unsigned)((ts.total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(*desc, time_scalar, rows, replicas);
     return check_launch("hexplane_time_backward");
 }

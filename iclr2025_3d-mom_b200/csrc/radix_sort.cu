@@ -48,7 +48,8 @@ __global__ void __launch_bounds__(256) rs_scan_hist(u32* __restrict__ g_hist)
     h[threadIdx.x] = block_exclusive_scan_256(v, s_warp);
 }
 
-// LB_BATCH (option "lookback_parallel", default on: 111 -> 103 us per 1M-pair 32-bit sort): the decoupled look-back of a digit walks its predecessors' states LB_BATCH at a
+// LB_BATCH (8 while every tile is resident at once: 111 -> 103 us per 1M-pair 32-bit sort, profiles/r2a_sort_check.txt): the
+// decoupled look-back of a digit walks its predecessors' states LB_BATCH at a
 // time (independent volatile loads in flight together) instead of one dependent L2 round trip per predecessor -- with a
 // few hundred tiles resident at once the serial walk is what a pass on ~1M keys spends its time in.  Same sums, same result.
 template <bool HAS_VALS, int IPT, int LB_BATCH, int BALLOT>
@@ -81,24 +82,19 @@ rs_onesweep_pass(const u32* __restrict__ keys_in, const u32* __restrict__ vals_i
         u32 idx = wbase + i * 32 + lane;
         key[i] = idx < n ? __ldg(keys_in + idx) : 0xFFFFFFFFu;
     }
-    // Stable in-warp ranking: items are visited in index order (i-major, then lane).
     // Stable in-warp ranking: items are visited in index order (i-major, then lane).  The lanes that hold the same digit are found
-    // with one ballot per digit bit (BALLOT: VOTE + LOP3, a few cycles each and independent across the IPT items) or with
-    // MATCH.ANY (one instruction, but its latency is the top stall of this kernel, profiles/r2w_stalls_rs_onesweep_pass.txt).
+    // with one ballot per digit bit (VOTE + LOP3, a few cycles each and independent across the IPT items) rather than MATCH.ANY
+    // (one instruction, but its latency was the top stall of this kernel, profiles/r2w_stalls_rs_onesweep_pass.txt): 103 -> 87 us
+    // per 1M-pair 32-bit sort, 96 -> 79 us per 2.4M-pair 12-bit sort (profiles/r3h_sort_check.txt).
     const u32 lt = lanemask_lt();
 #pragma unroll
     for (int i = 0; i < IPT; ++i) {
         u32 d = (key[i] >> shift) & mask;
-        u32 peers;
-        if constexpr (BALLOT > 0) {          // BALLOT = how many digit bits this pass can have set (4 or 8)
-            peers = 0xffffffffu;
+        u32 peers = 0xffffffffu;
 #pragma unroll
-            for (int b = 0; b < BALLOT; ++b) {
-                const u32 vote = __ballot_sync(0xffffffffu, (d >> b) & 1u);
-                peers &= ((d >> b) & 1u) ? vote : ~vote;
-            }
-        } else {
-            peers = __match_any_sync(0xffffffffu, d);
+        for (int b = 0; b < BALLOT; ++b) {   // BALLOT = how many digit bits this pass can have set (4 or 8)
+            const u32 vote = __ballot_sync(0xffffffffu, (d >> b) & 1u);
+            peers &= ((d >> b) & 1u) ? vote : ~vote;
         }
         u32 before = s_warp_hist[warp][d];
         rank[i] = (unsigned short)(before + __popc(peers & lt));
@@ -216,7 +212,7 @@ int radix_sort_pairs(u32* keys_a, u32* vals_a, u32* keys_b, u32* vals_b, size_t 
             kin, HV ? vin : nullptr, kout, HV ? vout : nullptr, (u32)n, spec.shift[p], spec.mask[p], g_hist + p * RS_RADIX, lb, tickets + p)
         // batched look-back pays while every tile is resident at once (3 CTAs per SM: 80 registers); beyond one wave the tiles of
         // the next wave find inclusive prefixes waiting and the plain walk is shorter (2.4M pairs / 12 bits: 79 vs 85 us)
-        const bool hv = vals_a != nullptr, par = g_opt_lookback_parallel != 0 && tiles <= (size_t)3 * NUM_SMS;
+        const bool hv = vals_a != nullptr, par = tiles <= (size_t)3 * NUM_SMS;
         // (32 states per round trip for single-wave inputs was measured too: 112 vs 103 us per 1M-pair sort, not kept;
         //  so was __launch_bounds__(256, 4): 64 registers with 20-36 B of spills, 87 -> 95 us per 1M-pair sort, 79 -> 76 us at 2.4M)
 #define RS_PICK(BLV) do { constexpr int BL = BLV; \
@@ -224,7 +220,7 @@ int radix_sort_pairs(u32* keys_a, u32* vals_a, u32* keys_b, u32* vals_b, size_t 
         else if (hv) RS_LAUNCH(true, RS_IPT, 1); \
         else if (par) RS_LAUNCH(false, RS_IPT, 8); \
         else RS_LAUNCH(false, RS_IPT, 1); } while (0)
-        if (g_opt_sort_ballot_rank == 0) RS_PICK(0); else if (spec.mask[p] < 16u) RS_PICK(4); else RS_PICK(8);
+        if (spec.mask[p] < 16u) RS_PICK(4); else RS_PICK(8);
 #undef RS_PICK
 #undef RS_LAUNCH
         u32* t = kin; kin = kout; kout = t;

@@ -4,7 +4,7 @@
 // Behaviour follows RAST/cuda_rasterizer/backward.cu:415-590 (compositing),
 // :144-274 (cov2D), :346-412 (projection, depth), :20-139 (SH), :278-341 (cov3D).
 // The compositing kernel does not issue one global atomic per (pixel, Gaussian, value)
-// like the reference (10 REDG per pair): the 32 pixels of a warp visit the same splat in
+// like the reference (10 REDG per pair): the 64 pixels of a warp visit the same splat in
 // lock-step, so their 10 partial gradients are folded with a transposed butterfly
 // (14 shuffles), accumulated per batch slot in shared memory, and leave the SM as three
 // 128-bit vector reductions per (tile, splat) instance.
@@ -15,210 +15,27 @@ namespace b200gs {
 
 namespace {
 
-constexpr int CB = 256;
 constexpr int ACC = 12;   // floats per Gaussian in the accumulation arena (3 x float4)
 
-struct __align__(16) BStage { float4 A[CB]; float4 B[CB]; float4 C[CB]; u32 gid[CB]; };
-
-__device__ __forceinline__ void bstage_fill(BStage& st, const u32* __restrict__ list, u32 begin, u32 n_eff,
-                                            u32 first, const float4* __restrict__ recA,
-                                            const float4* __restrict__ recB, const float4* __restrict__ recC)
-{
-    // position `pos` counts from the BACK of the effective list [begin, begin + n_eff)
-    const u32 t = threadIdx.x;
-    const u32 pos = first + t;
-    if (pos < n_eff) {
-        const u32 g = __ldg(list + (begin + n_eff - 1 - pos));
-        st.gid[t] = g;
-        cp_async16(&st.A[t], recA + g);
-        cp_async16(&st.B[t], recB + g);
-        cp_async16(&st.C[t], recC + g);
-    }
-}
-
-__global__ void __launch_bounds__(TILE_PIXELS)
-composite_bwd_kernel(const uint2* __restrict__ ranges, const u32* __restrict__ list, int W, int H, int grid_x,
-                     const float4* __restrict__ recA, const float4* __restrict__ recB,
-                     const float4* __restrict__ recC, const float* __restrict__ bg,
-                     const float* __restrict__ final_T, const u32* __restrict__ n_contrib,
-                     const float* __restrict__ dL_dpix, const float* __restrict__ dL_dpix_depth,
-                     float* __restrict__ acc)
-{
-    __shared__ BStage stage[2];
-    __shared__ __align__(16) float s_acc[CB * ACC];
-    __shared__ u32 s_max[8];
-    const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const u32 tile = blockIdx.x;
-    const u32 tx = tile % (u32)grid_x, ty = tile / (u32)grid_x;
-    const u32 px = tx * TILE_X + (warp & 1) * 8 + (lane & 7);
-    const u32 py = ty * TILE_Y + (warp >> 1) * 4 + (lane >> 3);
-    const bool inside = px < (u32)W && py < (u32)H;
-    const float fxp = (float)px, fyp = (float)py;
-    const uint2 range = ranges[tile];
-    const size_t pid = (size_t)py * W + px;
-    const size_t HW = (size_t)H * W;
-
-    const u32 last_contributor = inside ? n_contrib[pid] : 0;
-    const float patch_x = (float)(tx * TILE_X + (warp & 1) * 8), patch_y = (float)(ty * TILE_Y + (warp >> 1) * 4);
-    // nothing behind the deepest contributor of the tile can receive gradient
-    u32 m = last_contributor;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
-    const u32 warp_last = m;
-    if (lane == 0) s_max[warp] = m;
-    for (u32 i = tid; i < CB * ACC; i += TILE_PIXELS) s_acc[i] = 0.f;
-    __syncthreads();
-    u32 n_eff = 0;
-#pragma unroll
-    for (int w = 0; w < 8; ++w) n_eff = max(n_eff, s_max[w]);
-    n_eff = min(n_eff, range.y - range.x);
-    if (n_eff == 0) return;
-    const int rounds = (int)((n_eff + CB - 1) / CB);
-
-    const float T_final = inside ? final_T[pid] : 0.f;
-    float T = T_final;
-    float dLp0 = 0.f, dLp1 = 0.f, dLp2 = 0.f, dLd = 0.f;
-    if (inside) {
-        dLp0 = dL_dpix[pid]; dLp1 = dL_dpix[HW + pid]; dLp2 = dL_dpix[2 * HW + pid];
-        dLd = dL_dpix_depth ? dL_dpix_depth[pid] : 0.f;
-    }
-    const float bg_dot = bg[0] * dLp0 + bg[1] * dLp1 + bg[2] * dLp2;
-    float rec0 = 0.f, rec1 = 0.f, rec2 = 0.f, recd = 0.f;
-    float last_alpha = 0.f, lc0 = 0.f, lc1 = 0.f, lc2 = 0.f, ld = 0.f;
-    const float ddelx_dx = 0.5f * W, ddely_dy = 0.5f * H;
-
-    bstage_fill(stage[0], list, range.x, n_eff, 0, recA, recB, recC);
-    cp_async_commit();
-    for (int r = 0; r < rounds; ++r) {
-        if (r + 1 < rounds) bstage_fill(stage[(r + 1) & 1], list, range.x, n_eff, (u32)(r + 1) * CB, recA, recB, recC);
-        cp_async_commit();
-        cp_async_wait<1>();
-        __syncthreads();
-        const BStage& st = stage[r & 1];
-        const int cnt = (int)min((u32)CB, n_eff - (u32)r * CB);
-        // per-warp culling against the 8x4 pixel patch (see splat_may_touch_patch) and against the
-        // deepest contributor of the warp's pixels; survivors are walked back to front in lock-step
-        u32 masks[CB / 32];
-#pragma unroll
-        for (int q = 0; q < CB / 32; ++q) {
-            const int j = q * 32 + (int)lane;
-            const u32 p = n_eff - 1u - ((u32)r * CB + (u32)j);          // 0-based list position of staged slot j
-            const bool keep = j < cnt && p < warp_last && splat_may_touch_patch(st.A[j], st.B[j], patch_x, patch_y);
-            masks[q] = __ballot_sync(0xffffffffu, keep);
-        }
-#pragma unroll
-        for (int q = 0; q < CB / 32; ++q) {
-          u32 mq = masks[q];
-          while (mq != 0) {
-            const int j = q * 32 + __ffs(mq) - 1;
-            mq &= mq - 1;
-            const u32 contributor = n_eff - 1u - ((u32)r * CB + (u32)j);
-            bool act = contributor < last_contributor;      // false for pixels outside the image
-            const float4 A = st.A[j];
-            const float4 B = st.B[j];
-            const float dx = A.x - fxp, dy = A.y - fyp;
-            const float power = -0.5f * (A.z * dx * dx + B.x * dy * dy) - A.w * dx * dy;
-            act = act && !(power > 0.0f) && !(power < B.w);
-            float G = 0.f, alpha = 0.f;
-            if (act) {
-                G = expf(power);
-                alpha = fminf(0.99f, B.y * G);
-                act = !(alpha < 1.0f / 255.0f);
-            }
-            if (!__any_sync(0xffffffffu, act)) continue;
-            float v0 = 0.f, v1 = 0.f, v2 = 0.f, v3 = 0.f, v4 = 0.f, v5 = 0.f, v6 = 0.f, v7 = 0.f, v8 = 0.f, v9 = 0.f;
-            if (act) {
-                const float4 Cc = st.C[j];
-                T = T / (1.f - alpha);
-                const float w = alpha * T;
-                float dL_dalpha;
-                rec0 = last_alpha * lc0 + (1.f - last_alpha) * rec0; lc0 = Cc.x;
-                rec1 = last_alpha * lc1 + (1.f - last_alpha) * rec1; lc1 = Cc.y;
-                rec2 = last_alpha * lc2 + (1.f - last_alpha) * rec2; lc2 = Cc.z;
-                recd = last_alpha * ld + (1.f - last_alpha) * recd; ld = B.z;
-                dL_dalpha = (Cc.x - rec0) * dLp0 + (Cc.y - rec1) * dLp1 + (Cc.z - rec2) * dLp2 + (B.z - recd) * dLd;
-                dL_dalpha *= T;
-                last_alpha = alpha;
-                dL_dalpha += (-T_final / (1.f - alpha)) * bg_dot;
-                const float dL_dG = B.y * dL_dalpha;
-                const float gdx = G * dx, gdy = G * dy;
-                const float dG_ddelx = -gdx * A.z - gdy * A.w;
-                const float dG_ddely = -gdy * B.x - gdx * A.w;
-                v0 = dL_dG * dG_ddelx * ddelx_dx;      // d mean2D.x
-                v1 = dL_dG * dG_ddely * ddely_dy;      // d mean2D.y
-                v2 = -0.5f * gdx * dx * dL_dG;         // d conic.a
-                v3 = -0.5f * gdx * dy * dL_dG;         // d conic.b
-                v4 = -0.5f * gdy * dy * dL_dG;         // d conic.c
-                v5 = G * dL_dalpha;                    // d opacity
-                v6 = w * dLd;                          // d depth
-                v7 = w * dLp0; v8 = w * dLp1; v9 = w * dLp2;   // d colour
-            }
-            // transposed butterfly: 8 values (v0..v7) -> lane>>2 owns value (lane>>2); v8,v9 -> lanes 0/16
-            {
-                const bool h16 = lane & 16, h8 = lane & 8, h4 = lane & 4;
-                float u0 = (h16 ? v4 : v0) + __shfl_xor_sync(0xffffffffu, h16 ? v0 : v4, 16);
-                float u1 = (h16 ? v5 : v1) + __shfl_xor_sync(0xffffffffu, h16 ? v1 : v5, 16);
-                float u2 = (h16 ? v6 : v2) + __shfl_xor_sync(0xffffffffu, h16 ? v2 : v6, 16);
-                float u3 = (h16 ? v7 : v3) + __shfl_xor_sync(0xffffffffu, h16 ? v3 : v7, 16);
-                float y = (h16 ? v9 : v8) + __shfl_xor_sync(0xffffffffu, h16 ? v8 : v9, 16);
-                float w0 = (h8 ? u2 : u0) + __shfl_xor_sync(0xffffffffu, h8 ? u0 : u2, 8);
-                float w1 = (h8 ? u3 : u1) + __shfl_xor_sync(0xffffffffu, h8 ? u1 : u3, 8);
-                y += __shfl_xor_sync(0xffffffffu, y, 8);
-                float x = (h4 ? w1 : w0) + __shfl_xor_sync(0xffffffffu, h4 ? w0 : w1, 4);
-                y += __shfl_xor_sync(0xffffffffu, y, 4);
-                x += __shfl_xor_sync(0xffffffffu, x, 2);
-                y += __shfl_xor_sync(0xffffffffu, y, 2);
-                x += __shfl_xor_sync(0xffffffffu, x, 1);
-                y += __shfl_xor_sync(0xffffffffu, y, 1);
-                // value index held by this lane's quad: bit4 -> +4, bit3 -> +2, bit2 -> +1
-                if ((lane & 3) == 0) {
-                    const int k = ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1);
-                    // arena order: [mx, my, ca, cb | cc, op, dd, 0 | r, g, b, 0]; k: 0..5 -> slots 0..5, 6 -> 6, 7 -> 8
-                    const int slot = (k == 7) ? 8 : k;
-                    if (x != 0.f) atomicAdd(&s_acc[j * ACC + slot], x);
-                }
-                if ((lane & 15) == 0) {
-                    const int slot = (lane & 16) ? 10 : 9;
-                    if (y != 0.f) atomicAdd(&s_acc[j * ACC + slot], y);
-                }
-            }
-          }
-        }
-        __syncthreads();
-        // flush this batch: one thread per instance, three 128-bit reductions
-        if ((int)tid < cnt) {
-            float4* sa = reinterpret_cast<float4*>(&s_acc[tid * ACC]);
-            const float4 a0 = sa[0], a1 = sa[1], a2 = sa[2];
-            float* dst = acc + (size_t)st.gid[tid] * ACC;
-            if (a0.x != 0.f || a0.y != 0.f || a0.z != 0.f || a0.w != 0.f) red_add_v4(dst, a0.x, a0.y, a0.z, a0.w);
-            if (a1.x != 0.f || a1.y != 0.f || a1.z != 0.f) red_add_v4(dst + 4, a1.x, a1.y, a1.z, 0.f);
-            if (a2.x != 0.f || a2.y != 0.f || a2.z != 0.f) red_add_v4(dst + 8, a2.x, a2.y, a2.z, 0.f);
-            const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-            sa[0] = z; sa[1] = z; sa[2] = z;
-        }
-        __syncthreads();
-    }
-    cp_async_wait<0>();
-}
-
-
-// ---- the same kernel with TWO pixels per lane and packed FP32 pairs (option "composite_pairs", default on) -------------------
-// The kernel above is issue-slot bound (ncu: 75 % of issue slots busy, FMA pipe 34 %; 88 instructions per (warp, splat) of which
+// ---- compositing backward: TWO pixels per lane and packed FP32 pairs ----------------------------------------------------------
+// One pixel per lane is issue-slot bound (ncu: 75 % of issue slots busy, FMA pipe 34 %; 88 instructions per (warp, splat) of which
 // ~44 are the butterfly).  Here a warp covers an 8x8 patch: lane (lx, ly) owns pixels (lx, ly) and (lx, ly + 4) and carries their
 // state as f32x2 pairs, so the per-pixel arithmetic is issued once for both (FFMA2 / FMUL2 / FADD2, splat constants as
-// scalar-broadcast operands) and the 10-value butterfly is paid once per 64 pixels instead of once per 32.
+// scalar-broadcast operands) and the 10-value butterfly is paid once per 64 pixels instead of once per 32: 0.765 -> 0.608 ms per
+// 1M-Gaussian 1280x720 view.
 //   * A pixel for which the splat is inactive takes part with alpha = G = 0: T / (1 - 0), w = 0 and every partial gradient are
 //     exact no-ops, and the "previous colour" recurrence  rec = la * lc + (1 - la) * rec  evaluated one splat early gives the same
 //     value one splat later (0 * C + 1 * rec), so no per-pixel selects are needed and the previous colour is warp-uniform.
 //   * 1 / (1 - alpha) uses MUFU.RCP (relative error ~1e-7 per pair, 1e-5 over a chain of 100 contributors; the bar for these
 //     gradients is 1e-3); exp stays the accurate sequence (see below).
 constexpr int CB2_THREADS = 128;
-// CB2 = splats per batch, MINB = CTAs per SM the register budget is set for: 256 / 5 (39 KB of shared memory per CTA), 224 / 6
-// (34 KB, <= 85 registers), 192 / 7 (29 KB, <= 73 registers)
-template <int CB2> struct __align__(16) BStage2 { float4 A[CB2]; float4 B[CB2]; float4 C[CB2]; u32 gid[CB2]; };
+// CB2 = splats per batch, with the register budget set for 6 CTAs per SM (34 KB of shared memory per CTA, <= 85 registers).
+// Measured at 1M / 1280x720 and 200k / 512^2 (profiles/r2y_composite_pairs_occupancy.txt), whole rasterizer backward:
+// 256 / 5 CTAs: 0.612 / 0.322 ms, 224 / 6: 0.594 / 0.298 ms, 192 / 7: 0.582 / 0.321 ms.
+constexpr int CB2 = 224;
+struct __align__(16) BStage2 { float4 A[CB2]; float4 B[CB2]; float4 C[CB2]; u32 gid[CB2]; };
 
-template <int CB2, int MINB>
-__global__ void __launch_bounds__(CB2_THREADS, MINB)
+__global__ void __launch_bounds__(CB2_THREADS, 6)
 composite_bwd2_kernel(const uint2* __restrict__ ranges, const u32* __restrict__ list, int W, int H, int grid_x,
                       const float4* __restrict__ recA, const float4* __restrict__ recB,
                       const float4* __restrict__ recC, const float* __restrict__ bg,
@@ -226,7 +43,7 @@ composite_bwd2_kernel(const uint2* __restrict__ ranges, const u32* __restrict__ 
                       const float* __restrict__ dL_dpix, const float* __restrict__ dL_dpix_depth,
                       float* __restrict__ acc)
 {
-    __shared__ BStage2<CB2> stage[2];
+    __shared__ BStage2 stage[2];
     __shared__ __align__(16) float s_acc[CB2 * ACC];
     __shared__ u32 s_max[4];
     const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -266,7 +83,7 @@ composite_bwd2_kernel(const uint2* __restrict__ ranges, const u32* __restrict__ 
     float lc0 = 0.f, lc1 = 0.f, lc2 = 0.f, ld = 0.f;          // colour / depth of the previous splat this warp processed
     const float ddelx_dx = 0.5f * W, ddely_dy = 0.5f * H;
 
-    auto fill = [&](BStage2<CB2>& st, u32 first) {
+    auto fill = [&](BStage2& st, u32 first) {
 #pragma unroll
         for (int h = 0; h < (CB2 + CB2_THREADS - 1) / CB2_THREADS; ++h) {
             const u32 t = tid + h * CB2_THREADS, pos = first + t;
@@ -286,7 +103,7 @@ composite_bwd2_kernel(const uint2* __restrict__ ranges, const u32* __restrict__ 
         cp_async_commit();
         cp_async_wait<1>();
         __syncthreads();
-        const BStage2<CB2>& st = stage[r & 1];
+        const BStage2& st = stage[r & 1];
         const int cnt = (int)min((u32)CB2, n_eff - (u32)r * CB2);
         u32 masks[CB2 / 32];
 #pragma unroll
@@ -743,16 +560,8 @@ int rast_backward(int P, int D, int M, long long R, int W, int H, const float* b
     {
         ProfScope prof(PROF_COMPOSITE_BWD, stream);
         cudaMemsetAsync(grad_arena, 0, (size_t)P * ACC * sizeof(float), stream);
-        if (R > 0 && g_opt_composite_pairs != 0) {
-            // measured at 1M / 1280x720 and 200k / 512^2 (profiles/r2y_composite_pairs_occupancy.txt): 256 / 5: 0.612 / 0.322 ms,
-            // 224 / 6: 0.594 / 0.298 ms, 192 / 7: 0.582 / 0.321 ms for the whole rasterizer backward
-            auto kern = composite_bwd2_kernel<224, 6>;
-            kern<<<(unsigned)tiles, CB2_THREADS, 0, stream>>>(
-                img.ranges, sorted_list, W, H, grid_x, g.recA, g.recB, g.recC, bg, img.final_T, img.n_contrib,
-                dL_dpix, dL_dpix_depth, grad_arena);
-        }
-        else if (R > 0)
-            composite_bwd_kernel<<<(unsigned)tiles, TILE_PIXELS, 0, stream>>>(
+        if (R > 0)
+            composite_bwd2_kernel<<<(unsigned)tiles, CB2_THREADS, 0, stream>>>(
                 img.ranges, sorted_list, W, H, grid_x, g.recA, g.recB, g.recC, bg, img.final_T, img.n_contrib,
                 dL_dpix, dL_dpix_depth, grad_arena);
     }

@@ -331,9 +331,8 @@ __global__ void __launch_bounds__(PRE_THREADS) preprocess_fwd_kernel(const PreAr
 // (2 / 4 Gaussians per thread -- a 2 / 4 times shorter look-back chain -- were measured: stage 2 0.405 / 0.412 vs 0.409 ms, not kept.)
 constexpr u64 EM_AGG = 1ull << 62, EM_INCL = 1ull << 63, EM_VALUE = (1ull << 62) - 1;
 
-// WARP_LB (opt-in "lookback_parallel"): warp 0 looks back over 32 predecessors per step (ballots over their states, one
-// shuffle reduction) instead of thread 0 walking them one dependent L2 round trip at a time.  Same prefix, same output.
-template <bool WARP_LB>
+// Warp 0 looks back over 32 predecessors per step (ballots over their states, one shuffle reduction) instead of thread 0
+// walking them one dependent L2 round trip at a time.  Same prefix, same output.
 __global__ void __launch_bounds__(256)
 emit_instances_kernel(const u32* __restrict__ sorted_idx, u32 n_vis, const u32* __restrict__ tiles_touched,
                       const uint2* __restrict__ rect, int grid_x, u32* __restrict__ out_tile,
@@ -360,7 +359,7 @@ emit_instances_kernel(const u32* __restrict__ sorted_idx, u32 n_vis, const u32* 
     u32 total;
     const u32 off = block_exclusive_scan_256(cnt, s_scan, &total);
     s_off[tid] = off; s_rect[tid] = rc; s_gid[tid] = gid;
-    if (WARP_LB && tid < 32) {
+    if (tid < 32) {
         const u32 lane = tid;
         u64 prefix = 0;
         if (lane == 0) {
@@ -387,23 +386,6 @@ emit_instances_kernel(const u32* __restrict__ sorted_idx, u32 n_vis, const u32* 
             if (tile != 0) st_volatile_u64(status + tile, (prefix + total) | EM_INCL);
             s_base = prefix;
         }
-    }
-    if (!WARP_LB && tid == 0) {
-        s_off[256] = total;
-        u64 prefix = 0;
-        if (tile == 0) {
-            st_volatile_u64(status, (u64)total | EM_INCL);
-        } else {
-            st_volatile_u64(status + tile, (u64)total | EM_AGG);
-            for (u32 t = tile; t-- > 0;) {
-                u64 v;
-                do { v = ld_volatile_u64(status + t); } while ((v & (EM_AGG | EM_INCL)) == 0);
-                prefix += v & EM_VALUE;
-                if (v & EM_INCL) break;
-            }
-            st_volatile_u64(status + tile, (prefix + total) | EM_INCL);
-        }
-        s_base = prefix;
     }
     __syncthreads();
     const u64 base = s_base;
@@ -679,12 +661,8 @@ int rast_forward_stage2(int P, long long R, long long n_visible, int W, int H, c
         ProfScope prof(PROF_EMIT, stream);
         cudaMemsetAsync(b.emit_status, 0, ((size_t)nblk + 1) * sizeof(u64), stream);
         cudaMemsetAsync(b.emit_ticket, 0, 64 * sizeof(u32), stream);
-        if (g_opt_lookback_parallel != 0)
-            emit_instances_kernel<true><<<nblk, 256, 0, stream>>>(sorted_gid, (u32)n_visible, g.tiles_touched, g.rect,
-                                                                  d.grid_x, b.ikeys_a, b.ivals_a, b.emit_status, b.emit_ticket);
-        else
-            emit_instances_kernel<false><<<nblk, 256, 0, stream>>>(sorted_gid, (u32)n_visible, g.tiles_touched, g.rect,
-                                                                   d.grid_x, b.ikeys_a, b.ivals_a, b.emit_status, b.emit_ticket);
+        emit_instances_kernel<<<nblk, 256, 0, stream>>>(sorted_gid, (u32)n_visible, g.tiles_touched, g.rect,
+                                                        d.grid_x, b.ikeys_a, b.ivals_a, b.emit_status, b.emit_ticket);
         }
         // 3. stable sort by tile id => (tile, depth, index) order
         {

@@ -10,7 +10,8 @@
  *  - Every function returns 0 on success and non-zero on error; b200gs_last_error() returns
  *    the message of the last error raised on the calling thread.
  *  - Ownership: the caller owns every buffer, scratch included. The library never allocates
- *    or frees device memory and keeps no global state besides the per-thread error string.
+ *    or frees device memory and keeps no global state besides the per-thread error string and the
+ *    process-wide settings of b200gs_set_option / b200gs_profile_enable.
  *  - No implicit device synchronisation except where stated (b200gs_rast_forward_stage1).
  *  - "null" for an optional tensor has the meaning of the reference's empty tensor.
  *  Citations: RAST = submodules/depth-diff-gaussian-rasterization, KNN = submodules/simple-knn.
@@ -29,37 +30,11 @@ typedef void* b200gs_stream_t; /* cudaStream_t */
 
 const char* b200gs_last_error(void);
 int b200gs_version(void);
-/* Kernel variants, process-wide. The defaults are the fastest variants that have passed tools/native/mlp_variant_check.cu on
- * a B200 (bit-identical outputs, gradients equal up to float-atomic order); 0 selects the first-generation kernel, the
- * environment variable B200GS_<NAME>=<integer> overrides the initial value:
- *   "mlp_bwd_v2"     deformation-MLP backward (default 87): bit 0 = alternating weight slots + elected MMA issuer + coalesced
- *                    gradient flush; bits 1-2 = how d_out reaches a phase (3 = prefetched into L2 one phase ahead); 55 = 7 +
- *                    ONE dY image in shared memory, read K-major by the dX chain and MN-major by the weight-gradient MMAs;
- *                    87 = 55 + stash / feature rows staged by 32 KB TMA bulk copies two phases ahead (tiled feature layout;
- *                    55 otherwise) (deform_mlp_bwd_tc5.cu).  Built values: 0, 1, 3, 5, 7, 55, 87; anything else is refused
- *   "mlp_fwd_elect"  deformation-MLP forward (default 2): 1 = elected MMA issuer, 2 = plus activation-stash stores deferred
- *                    past the next layer's MMA issue (deform_mlp_tc5.cu)
- *   "hexplane_time_fwd" time-row HexPlane forward (default 2): 1 / 2 = both levels' factor rows requested up front,
- *                    register budget for 3 / 2 resident CTAs per SM; bit-identical outputs
- *   "hexplane_time_bwd" time-row HexPlane backward (default 2): 1 / 2 = both levels' rows requested before the
- *                    first is used, register budget for 3 / 2 resident CTAs per SM (hexplane.cu: hexplane_time_bwd2_kernel)
- *   "lookback_parallel" chained scans of the radix sort passes and of the instance emission (default 1):
- *                    predecessors' states are read 8 (per digit) / 32 (per warp) at a time instead of one dependent L2 round
- *                    trip each (sort passes: only while all tiles are resident at once); identical results
- *   "sort_ballot_rank" radix sort passes (default 1): the lanes of a warp that hold the same digit are found with one ballot per
- *                    digit bit (4 or 8 VOTE + LOP3, independent across a thread's 16 keys) instead of MATCH.ANY, whose latency was
- *                    the kernel's top stall: 103 -> 87 us per 1M-pair 32-bit sort, 96 -> 79 us per 2.4M-pair 12-bit sort; identical results
+/* Process-wide launch settings (the library reads no environment variables):
  *   "mlp_fwd_sms" / "mlp_bwd_sms" (default 0 = all 148): CTAs of the persistent deformation-MLP kernels.  The view-pipelining trainer
  *                    sets 120 around a step so that the other stream's sorts / emission / preprocess find free SMs next to them
  *                    (377 -> 383 view-iterations/s; 96: slower again); same results up to the order of the weight-gradient flushes
- *   "composite_pairs" compositing backward (default 1): a lane owns TWO pixels of an 8x8 warp patch and carries their state as
- *                    packed FP32 pairs (FFMA2 / FMUL2 / FADD2), the gradient butterfly is paid once per 64 pixels: 0.765 -> 0.608 ms
- *                    per 1M-Gaussian 1280x720 view; 0 = the one-pixel-per-lane kernel (rast_backward.cu)
- * Measured on a B200 in round 2 (profiles/r2a_*.txt); the variants that lost ("sort_small_tiles", "sort_balanced_digits", the
- * resident-weight and double-buffered MLP backward kernels) were deleted.
- * Same arithmetic in every variant.  ("mlp_bwd_ablate" is a profiling aid, not a variant: it removes one part of the MLP
- * backward kernel -- WRONG RESULTS -- so that tools/native/mlp_variant_check can time what that part costs; it is refused
- * unless the environment has B200GS_PROFILING=1.)  set: 0 on success, non-zero for an unknown name; get: the value, or -1 for an unknown name. */
+ * set: 0 on success, non-zero for an unknown name; get: the value, or -1 for an unknown name. */
 int b200gs_set_option(const char* name, int value);
 int b200gs_get_option(const char* name);
 
@@ -265,6 +240,8 @@ typedef struct {
                                      4-point-group tile layout of the activation stash ([tile of 128][32 groups][16 chunks][4 points][4]),
                                      which is what b200gs_hexplane_time_forward / _backward produce / consume with tiled = 1 */
 } b200gs_mlp_weights;
+/* gradients of b200gs_mlp_weights' arrays.  With feat_dim 64, w1 and the w2[h] of every enabled head must be 16-byte aligned
+ * (they are accumulated with 128-bit vector reductions); b200gs_deform_mlp_backward refuses other pointers. */
 typedef struct { float* w1; float* b1; float* w2[3]; float* b2[3]; float* w3[3]; float* b3[3]; } b200gs_mlp_grads;
 
 /* floats of the buffer the forward leaves for the backward (opaque to the caller, who only allocates it and hands the same

@@ -90,23 +90,55 @@ def test_call_timer_table_names_are_abi_entries():
         assert hasattr(L, name), name
 
 
-def test_kernel_variant_options_defaults_and_toggle():
-    """Kernel variants (include/b200gs.h: b200gs_set_option): validated defaults unless the environment overrides them;
-    unknown names are an error."""
+RETIRED_OPTIONS = (b"mlp_bwd_v2", b"mlp_fwd_elect", b"mlp_bwd_ablate", b"hexplane_time_fwd", b"hexplane_time_bwd",
+                   b"lookback_parallel", b"sort_ballot_rank", b"composite_pairs", b"sort_small_tiles", b"sort_balanced_digits")
+
+
+def test_launch_settings_and_retired_option_names():
+    """Launch settings (include/b200gs.h: b200gs_set_option): the two MLP SM caps round-trip from their default 0; the
+    kernel-generation switches of earlier rounds are unknown names; the environment changes nothing."""
+    import subprocess
+    import sys
     from b200gs import _lib
     L = _lib.lib()
-    for name, dflt in ((b"mlp_bwd_v2", 87), (b"mlp_fwd_elect", 2), (b"hexplane_time_fwd", 2), (b"hexplane_time_bwd", 2), (b"lookback_parallel", 1), (b"composite_pairs", 1), (b"sort_ballot_rank", 1)):
-        env = os.environ.get("B200GS_" + name.decode().upper())
-        want = int(env) if env is not None and env[:1].isdigit() else dflt
-        assert L.b200gs_get_option(name) == want
+    for name in (b"mlp_fwd_sms", b"mlp_bwd_sms"):
+        assert L.b200gs_get_option(name) == 0
+        assert L.b200gs_set_option(name, 120) == 0 and L.b200gs_get_option(name) == 120
         assert L.b200gs_set_option(name, 0) == 0 and L.b200gs_get_option(name) == 0
-        assert L.b200gs_set_option(name, want) == 0 and L.b200gs_get_option(name) == want
-    assert L.b200gs_get_option(b"mlp_bwd_ablate") == 0
-    for name in (b"sort_small_tiles", b"sort_balanced_digits"):      # measured in round 2, lost, deleted
-        assert L.b200gs_get_option(name) == -1
-    if os.environ.get("B200GS_PROFILING") != "1":                  # the wrong-results profiling builds cannot be switched on by accident
-        assert L.b200gs_set_option(b"mlp_bwd_ablate", 2) != 0 and L.b200gs_get_option(b"mlp_bwd_ablate") == 0
-        keep = L.b200gs_get_option(b"mlp_bwd_v2")
-        assert L.b200gs_set_option(b"mlp_bwd_v2", 23) != 0 and L.b200gs_get_option(b"mlp_bwd_v2") == keep      # inexact on hardware: not built
-    assert L.b200gs_set_option(b"no_such_option", 1) != 0 and b"unknown option" in L.b200gs_last_error()
-    assert L.b200gs_get_option(b"no_such_option") == -1
+    for name in RETIRED_OPTIONS + (b"no_such_option",):
+        assert L.b200gs_get_option(name) == -1, name
+        assert L.b200gs_set_option(name, 1) != 0 and b"unknown option" in L.b200gs_last_error(), name
+        assert L.b200gs_get_option(name) == -1, name
+    # the library reads no environment variables: a process started with the old B200GS_* switches sees the same answers
+    names = [n.decode() for n in (b"mlp_fwd_sms", b"mlp_bwd_sms") + RETIRED_OPTIONS]
+    probe = ("import ctypes, sys; L = ctypes.CDLL(sys.argv[1]); "
+             "print([L.b200gs_get_option(n.encode()) for n in sys.argv[2:]])")
+    env = dict(os.environ, B200GS_MLP_BWD_V2="0", B200GS_MLP_FWD_ELECT="0", B200GS_MLP_FWD_SMS="100",
+               B200GS_MLP_BWD_SMS="100", B200GS_COMPOSITE_PAIRS="0", B200GS_SORT_BALLOT_RANK="0", B200GS_PROFILING="1")
+    r = subprocess.run([sys.executable, "-c", probe, _lib.LIB_PATH] + names, env=env, capture_output=True, text=True,
+                       timeout=120)
+    assert r.returncode == 0, r.stderr
+    assert r.stdout.strip() == str([0, 0] + [-1] * len(RETIRED_OPTIONS))
+
+
+def test_mlp_backward_refuses_misaligned_weight_gradients():
+    """The tcgen05 MLP backward (feat_dim 64) flushes the W1 / W2 gradients with 128-bit reductions: a gradient pointer
+    that is not 16-byte aligned is an error raised before anything touches the device."""
+    from b200gs import _lib
+    from b200gs.field import _MlpGrads, _MlpWeights
+    L = _lib.lib()
+    w = _MlpWeights(feat_dim=64, width=64, w1=0x10000, b1=0x20000)
+    for h in range(3):
+        w.w2[h], w.b2[h], w.w3[h], w.b3[h] = 0x30000 + 0x1000 * h, 0x40000, 0x50000, 0x60000
+    for bad in ("w1", "w2"):
+        gw = _MlpGrads(w1=0x70000, b1=0x80000)
+        for h in range(3):
+            gw.w2[h], gw.b2[h], gw.w3[h], gw.b3[h] = 0x90000 + 0x1000 * h, 0xa0000, 0xb0000, 0xc0000
+        if bad == "w1":
+            gw.w1 = 0x70004
+        else:
+            gw.w2[1] = 0x91008
+        rc = L.b200gs_deform_mlp_backward(ctypes.byref(w), ctypes.byref(gw), ctypes.c_longlong(1000), None, None, None,
+                                          None, None, None, None)
+        assert rc != 0, bad
+        assert b"16-byte aligned" in L.b200gs_last_error(), (bad, L.b200gs_last_error())

@@ -4,13 +4,11 @@
 TAG=${1:-rX}
 KRE=${2:-deform_mlp_bwd}
 mkdir -p gpurun_out
-# seconds each, no Python: kernel-variant parity + timing, rasterizer checksums + timing (diff two builds / option values)
+# seconds each, no Python: sort check + timing, rasterizer checksums + timing (diff two builds)
 tools/probe/umma_probe2 > gpurun_out/umma_probe2_$TAG.log 2>&1; cat gpurun_out/umma_probe2_$TAG.log
-make -s -C tools/native >/dev/null 2>&1; tools/native/mlp_variant_check 1000000 7,55,87 > gpurun_out/mlp_variant_check_$TAG.log 2>&1; grep -v '^    ' gpurun_out/mlp_variant_check_$TAG.log | head -40
-tools/native/mlp_variant_check 1000000 ablate > gpurun_out/mlp_bwd_ablate_$TAG.log 2>&1; cat gpurun_out/mlp_bwd_ablate_$TAG.log
+make -s -C tools/native >/dev/null 2>&1
 tools/native/sort_check 1000000 32 > gpurun_out/sort_check_$TAG.log 2>&1; tail -9 gpurun_out/sort_check_$TAG.log
 tools/native/sort_check 5100000 12 > gpurun_out/sort_check12_$TAG.log 2>&1; tail -9 gpurun_out/sort_check12_$TAG.log
-tools/native/hexplane_time_check > gpurun_out/hexplane_time_check_$TAG.log 2>&1; tail -4 gpurun_out/hexplane_time_check_$TAG.log
 tools/native/view_check 1000000 1280 720 0.01 8 > gpurun_out/view_check_$TAG.log 2>&1; tail -16 gpurun_out/view_check_$TAG.log
 tools/native/rast_check 1000000 1280 720 0.01 10 > gpurun_out/rast_check_$TAG.log 2>&1; sed -n 2,4p gpurun_out/rast_check_$TAG.log
 python -m pytest tests -m gpu -x -q > gpurun_out/pytest_$TAG.log 2>&1; echo "pytest rc=$?" ; tail -3 gpurun_out/pytest_$TAG.log

@@ -1,6 +1,5 @@
-// Standalone check of the radix sort variants through the C ABI: b200gs_sort_pairs_u32 with "lookback_parallel" off / on on the same
-// random (key, value) pairs -- results must be identical (the sort is stable, so the output is unique) and equal to std::stable_sort --
-// with the device time of each (CUDA events, 10 sorts after one warm-up).
+// Standalone check of the radix sort through the C ABI: b200gs_sort_pairs_u32 on random (key, value) pairs must equal
+// std::stable_sort (the sort is stable, so the output is unique), with its device time (CUDA events, 10 sorts after one warm-up).
 // run: tools/native/sort_check [n = 1000000] [bits = 32]
 #include <algorithm>
 #include <cstdint>
@@ -30,26 +29,21 @@ int main(int argc, char** argv)
     CK(cudaMemcpy(k0, keys.data(), n * 4, cudaMemcpyHostToDevice)); CK(cudaMemcpy(v0, vals.data(), n * 4, cudaMemcpyHostToDevice));
     cudaStream_t st; CK(cudaStreamCreate(&st));
     cudaEvent_t e0, e1; CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
-    bool ok = true;
-    for (int variant = 0; variant < 4; ++variant) {          // lookback_parallel off / on  x  sort_ballot_rank off / on
-        if (b200gs_set_option("lookback_parallel", variant & 1) || b200gs_set_option("sort_ballot_rank", variant >> 1)) { printf("%s\n", b200gs_last_error()); return 3; }
-        float total = 0; int side = 0;
-        for (int rep = -1; rep < 10; ++rep) {
-            CK(cudaMemcpyAsync(ka, k0, n * 4, cudaMemcpyDeviceToDevice, st)); CK(cudaMemcpyAsync(va, v0, n * 4, cudaMemcpyDeviceToDevice, st));
-            CK(cudaEventRecord(e0, st));
-            side = b200gs_sort_pairs_u32(ka, va, kb, vb, n, 0, bits, temp, tb, st);
-            CK(cudaEventRecord(e1, st)); CK(cudaStreamSynchronize(st));
-            if (side < 0) { printf("sort failed: %s\n", b200gs_last_error()); return 3; }
-            float ms; CK(cudaEventElapsedTime(&ms, e0, e1)); if (rep >= 0) total += ms;
-        }
-        std::vector<uint32_t> ok_k(n), ok_v(n);
-        CK(cudaMemcpy(ok_k.data(), side ? kb : ka, n * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(ok_v.data(), side ? vb : va, n * 4, cudaMemcpyDeviceToHost));
-        size_t bad = 0;
-        for (size_t i = 0; i < n; ++i) bad += ok_v[i] != order[i] || ok_k[i] != keys[order[i]];
-        printf("lookback_parallel = %d, sort_ballot_rank = %d: %.1f us per sort of %zu pairs on %d bits, %zu mismatches against std::stable_sort\n",
-               variant & 1, variant >> 1, 100.f * total, n, bits, bad);
-        ok &= bad == 0;
+    float total = 0; int side = 0;
+    for (int rep = -1; rep < 10; ++rep) {
+        CK(cudaMemcpyAsync(ka, k0, n * 4, cudaMemcpyDeviceToDevice, st)); CK(cudaMemcpyAsync(va, v0, n * 4, cudaMemcpyDeviceToDevice, st));
+        CK(cudaEventRecord(e0, st));
+        side = b200gs_sort_pairs_u32(ka, va, kb, vb, n, 0, bits, temp, tb, st);
+        CK(cudaEventRecord(e1, st)); CK(cudaStreamSynchronize(st));
+        if (side < 0) { printf("sort failed: %s\n", b200gs_last_error()); return 3; }
+        float ms; CK(cudaEventElapsedTime(&ms, e0, e1)); if (rep >= 0) total += ms;
     }
+    std::vector<uint32_t> ok_k(n), ok_v(n);
+    CK(cudaMemcpy(ok_k.data(), side ? kb : ka, n * 4, cudaMemcpyDeviceToHost)); CK(cudaMemcpy(ok_v.data(), side ? vb : va, n * 4, cudaMemcpyDeviceToHost));
+    size_t bad = 0;
+    for (size_t i = 0; i < n; ++i) bad += ok_v[i] != order[i] || ok_k[i] != keys[order[i]];
+    printf("%.1f us per sort of %zu pairs on %d bits, %zu mismatches against std::stable_sort\n", 100.f * total, n, bits, bad);
+    const bool ok = bad == 0;
     printf("RESULT: %s\n", ok ? "PASS" : "FAIL");
     return ok ? 0 : 1;
 }

@@ -3,9 +3,9 @@
 //   forward (stage 1 + 2) -> L1 loss + gradient -> rasterizer backward (SH gradient accumulated) -> activations backward ->
 //   deformation MLP backward -> time-row HexPlane backward
 // plus the per-step pieces once (spatial HexPlane forward / backward, plane regulariser).  Device time per entry point (CUDA
-// events on the launching stream) and per view, so that a kernel option can be A/B'd end to end in seconds:
+// events on the launching stream) and per view, so that two builds or launch settings can be A/B'd end to end in seconds:
 //     tools/native/view_check 1000000 1280 720 0.01 8
-//     tools/native/view_check 1000000 1280 720 0.01 8 lookback_parallel=0 mlp_bwd_v2=7
+//     tools/native/view_check 1000000 1280 720 0.01 8 mlp_fwd_sms=120 mlp_bwd_sms=120
 // Synthetic inputs with the distributions of b200gs/synthetic.py (not the same random stream), random-init field.  This is a
 // timing tool: results are summarised by checksums only (the parity tests live in tests/).
 #include <cmath>

@@ -1,9 +1,10 @@
 """Deformation-MLP kernels alone (C3 point count): device time per launch of b200gs_deform_mlp_forward / _backward through the
-C ABI, CUDA events on the launching stream, L2 flushed by the working set itself (1.4 / 1.6 GB per launch).  Run it once per
-variant (include/b200gs.h: b200gs_set_option; the environment gives the initial values):
-    python tools/time_mlp.py                                                  # defaults
-    B200GS_MLP_BWD_V2=0 B200GS_MLP_FWD_ELECT=0 python tools/time_mlp.py       # first-generation kernels
-(tools/native/mlp_variant_check does the same without Python and also compares the variants' results.)"""
+C ABI, CUDA events on the launching stream, L2 flushed by the working set itself (1.4 / 1.6 GB per launch).  Knobs:
+    P = point count (default 1000000)
+    MULTIRES = HexPlane level multipliers (default 1,2: 2 levels, feature dim 64, the reference's configuration;
+               1,2,4,8: 4 levels, feature dim 128)
+    python tools/time_mlp.py
+    MULTIRES=1,2,4,8 P=1000000 python tools/time_mlp.py"""
 import os
 import sys
 
@@ -15,7 +16,8 @@ import torch
 import test_field_parity as T
 
 P = int(os.environ.get("P", 1000000))
-net = T._model([1, 2], 50)
+MULTIRES = [int(m) for m in os.environ.get("MULTIRES", "1,2").split(",")]
+net = T._model(MULTIRES, 50)
 xyz, scales, rot, opacity, shs, flow = T._inputs(P)
 frame_num = torch.tensor(22, device="cuda")
 a = [t.clone().requires_grad_(True) for t in (xyz, scales, rot)]
@@ -37,6 +39,6 @@ with profile(activities=[ProfilerActivity.CUDA]) as prof:
         step()
     torch.cuda.synchronize()
 rows = [(e.key, e.device_time_total / max(e.count, 1), e.count) for e in prof.key_averages() if "deform_mlp" in e.key or "hexplane" in e.key]
-print("variants:", {k: v for k, v in os.environ.items() if k.startswith("B200GS_")})
+print(f"P = {P}, multires = {MULTIRES}")
 for k, us, n in sorted(rows, key=lambda r: -r[1]):
     print(f"{us:9.1f} us x{n:3d}  {k[:100]}")
