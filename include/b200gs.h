@@ -31,7 +31,8 @@ typedef void* b200gs_stream_t; /* cudaStream_t */
 const char* b200gs_last_error(void);
 int b200gs_version(void);
 /* Process-wide launch settings (the library reads no environment variables):
- *   "mlp_fwd_sms" / "mlp_bwd_sms" (default 0 = all 148): CTAs of the persistent deformation-MLP kernels.  The view-pipelining trainer
+ *   "mlp_fwd_sms" / "mlp_bwd_sms" (default 0 = all 148): CTAs of the persistent deformation-MLP kernels (mlp_bwd_sms caps the
+ *                    feature-dim-64 backward only: the feature-dim-128 backward always launches one CTA per SM).  The view-pipelining trainer
  *                    sets 120 around a step so that the other stream's sorts / emission / preprocess find free SMs next to them
  *                    (377 -> 383 view-iterations/s; 96: slower again); same results up to the order of the weight-gradient flushes
  * set: 0 on success, non-zero for an unknown name; get: the value, or -1 for an unknown name. */

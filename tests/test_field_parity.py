@@ -12,20 +12,20 @@ from oracle import field_torch as oracle
 pytestmark = pytest.mark.gpu
 
 
-def _args(multires, T):
+def _args(multires, T, no_dx=False, no_ds=False, no_dr=False):
     return types.SimpleNamespace(
         net_width=64, timebase_pe=4, defor_depth=0, posebase_pe=10, scale_rotation_pe=2, opacity_pe=2,
         timenet_width=64, timenet_output=32, bounds=1.6, grid_pe=0,
         kplanes_config={'grid_dimensions': 2, 'input_coordinate_dim': 4, 'output_coordinate_dim': 32,
                         'resolution': [64, 64, 64, T]},
-        multires=multires, no_dx=False, no_grid=False, no_ds=False, no_dr=False, no_do=True, no_dshs=True,
+        multires=multires, no_dx=no_dx, no_grid=False, no_ds=no_ds, no_dr=no_dr, no_do=True, no_dshs=True,
         empty_voxel=False, static_mlp=False, apply_rotation=False)
 
 
-def _model(multires, T, seed=0):
+def _model(multires, T, seed=0, **heads_off):
     from b200gs.field import deform_network
     torch.manual_seed(seed)
-    net = deform_network(_args(multires, T)).cuda()
+    net = deform_network(_args(multires, T, **heads_off)).cuda()
     with torch.no_grad():
         for p in net.deformation_net.grid.grids.parameters():
             p.add_(torch.randn_like(p) * 0.01)       # make the time planes non-trivial (SURVEY §8d)
@@ -54,14 +54,22 @@ def _rel(a, b):
 _FULL = [([1, 2], 50, 1000000)]      # BASELINE.json C3 point count (always on: seconds on a B200)
 
 
-@pytest.mark.parametrize("multires,T,P", [([1, 2], 50, 5000), ([1, 2], 50, 64), ([1, 2], 50, 1), ([1, 2, 4, 8], 25, 3001),
-                                          ([1, 2], 50, 40003), ([1, 2], 50, -5000), ([1, 2], 50, -40003)] + _FULL)   # >= 16384 points: cell-ordered traversal
-def test_deform_network_forward_backward(multires, T, P):
+_CASES = [([1, 2], 50, 5000), ([1, 2], 50, 64), ([1, 2], 50, 1), ([1, 2, 4, 8], 25, 3001),
+          ([1, 2], 50, 40003), ([1, 2], 50, -5000), ([1, 2], 50, -40003)] + _FULL      # >= 16384 points: cell-ordered traversal
+# disabled heads (no_dx / no_ds / no_dr): pass-through outputs, no stash-free inference, no gradient for the head's parameters
+_HEADS_OFF = [{"no_ds": True}, {"no_dx": True, "no_dr": True}]
+
+
+@pytest.mark.parametrize("multires,T,P,heads_off",
+                         [pytest.param(m, T, P, {}, id=f"multires{i}-{T}-{P}") for i, (m, T, P) in enumerate(_CASES)] +
+                         [pytest.param(m, T, P, off, id=f"multires{i}-{T}-{P}-" + "-".join(off)) for off in _HEADS_OFF
+                          for i, (m, T, P) in enumerate(_CASES) if P in (5000, 3001)])
+def test_deform_network_forward_backward(multires, T, P, heads_off):
     # P < 0: |P| points with a DIFFERENT timestamp per point (the general [P,1] tensor of gaussian_renderer/__init__.py:56);
     # otherwise the camera's one timestamp repeated, which field.DETECT_UNIFORM_TIME routes to the one-timestamp kernels
     per_point_time = P < 0
     P = abs(P)
-    net = _model(multires, T)
+    net = _model(multires, T, **heads_off)
     levels = len(multires)
     xyz, scales, rot, opacity, shs, flow = _inputs(P)
     time = torch.rand(P, 1, generator=torch.Generator().manual_seed(9)).cuda() if per_point_time else torch.full((P, 1), 0.37, device="cuda")
@@ -71,7 +79,7 @@ def test_deform_network_forward_backward(multires, T, P):
     a = [t.clone().requires_grad_(True) for t in (xyz, scales, rot)]
     pts, sc, rt, op, sh = net(a[0], a[1], a[2], opacity, shs, time, flow, frame_num, 1)
     b = [t.clone().requires_grad_(True) for t in (xyz, scales, rot)]
-    rp, rs, rr, ro, rsh = oracle.deform_forward(sd, levels, b[0], b[1], b[2], opacity, shs, time, flow, frame_num, 1)
+    rp, rs, rr, ro, rsh = oracle.deform_forward(sd, levels, b[0], b[1], b[2], opacity, shs, time, flow, frame_num, 1, **heads_off)
     assert _rel(pts, rp) < 2e-5 and _rel(sc, rs) < 2e-5 and _rel(rt, rr) < 2e-5
     assert torch.equal(op, ro) and sh is shs
 
@@ -100,7 +108,8 @@ def test_deform_network_forward_backward(multires, T, P):
         sd64 = {k: (v.detach().clone().to(dt) if v.dtype.is_floating_point else v.detach().clone()).contiguous().requires_grad_(v.dtype.is_floating_point)
                 for k, v in net.state_dict().items()}
         c = [t.clone().to(dt).requires_grad_(True) for t in (xyz, scales, rot)]
-        qp, qs, qr, _, _ = oracle.deform_forward(sd64, levels, c[0], c[1], c[2], opacity.to(dt), shs.to(dt), time.to(dt), flow.to(dt), frame_num, 1)
+        qp, qs, qr, _, _ = oracle.deform_forward(sd64, levels, c[0], c[1], c[2], opacity.to(dt), shs.to(dt), time.to(dt), flow.to(dt), frame_num, 1,
+                                                 **heads_off)
         ((qp * wp.to(dt)).sum() + (qs * ws.to(dt)).sum() + (qr * wr.to(dt)).sum()).backward()
     for k, v in sd.items():
         if not v.requires_grad or k.endswith("grid.aabb") or k not in params:
@@ -125,7 +134,7 @@ def test_deform_network_forward_backward(multires, T, P):
             worst = max(worst, e_ours)
         checked += 1
     print(f"worst parameter-gradient relative error: {worst:.2e}")
-    assert checked >= 2 + 12 + 6 * levels
+    assert checked >= 2 + 4 * (3 - len(heads_off)) + 6 * levels
     # never-used sub-networks get no gradient, exactly like the reference (Appendix C iii)
     assert all(p.grad is None for n, p in net.named_parameters() if n.startswith("timenet") or "opacity_deform" in n or "shs_deform" in n)
 
