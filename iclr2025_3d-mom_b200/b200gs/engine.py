@@ -48,7 +48,7 @@ def default_opt():
         position_lr_init=0.00016, position_lr_final=0.0000016, position_lr_delay_mult=0.01, position_lr_max_steps=20000,
         deformation_lr_init=0.00016, deformation_lr_final=0.0000016, deformation_lr_delay_mult=0.01,
         grid_lr_init=0.0016, grid_lr_final=0.000016, feature_lr=0.0025, opacity_lr=0.05, scaling_lr=0.005,
-        rotation_lr=0.001, percent_dense=0.01)
+        rotation_lr=0.001, percent_dense=0.01, lambda_dssim=0.0)
 
 
 def expon_lr(step, lr_init, lr_final, max_steps, lr_delay_steps=0, lr_delay_mult=1.0):
@@ -371,8 +371,10 @@ class ViewParallelTrainer:
     Same sums, same Adam arithmetic as one collective + one optimiser launch (tests/test_dist_gloo.py, tests/test_dist_nccl.py)."""
 
     def __init__(self, model, bg_color, stage="fine", process_group=None, world_size=1, rank=0, render_fn=None,
-                 regulation=None, regulation_fn=None, shared_shs=None, overlap_sh_reduce=None):
+                 regulation=None, regulation_fn=None, shared_shs=None, overlap_sh_reduce=None, lambda_dssim=0.0):
         self.model = model
+        # opt.lambda_dssim (arguments/__init__.py): loss += lambda_dssim * (1 - ssim(image, gt)), fused path only; 0 = no D-SSIM term
+        self.lambda_dssim = float(lambda_dssim)
         self.bg = bg_color
         self.stage = stage
         # (time_smoothness_weight, l1_time_planes, plane_tv_weight) of train_4DGS.py:215-218, or None to leave it out
@@ -531,7 +533,9 @@ class ViewParallelTrainer:
     def step(self, cams, gts, global_batch=None):
         """cams / gts: THIS rank's views; a ground-truth image is a float32 [3,H,W] tensor or the dataset's own uint8 [H,W,3]
         image (GPU path). Loss = mean over the GLOBAL batch of per-view L1 means (train_4DGS.py:205-210: l1 over the
-        concatenated [B,3,H,W] tensor). Returns the summed local loss (already scaled by 1/B) as a tensor."""
+        concatenated [B,3,H,W] tensor), plus lambda_dssim * (1 - ssim) of the same batch when lambda_dssim > 0 (train_4DGS.py's
+        opt.lambda_dssim term; the batch's SSIM is the mean of the per-view SSIMs since all views have the same size). Returns the
+        summed local loss (already scaled by 1/B) as a tensor."""
         B = global_batch or (len(cams) * self.world_size)
         self._bind()
         self._mark("step_start")
@@ -620,9 +624,14 @@ class ViewParallelTrainer:
                             img = pkg["render"]
                             self._sse_numel = img.numel()
                             d_img = fusedops.l1_loss_and_grad(img, gt, 1.0 / (img.numel() * B), total, self._sse[vi:])
+                            if self.lambda_dssim > 0.0:
+                                # + lambda_dssim * (1 - ssim) of this view's share, its gradient added into d_img
+                                fusedops.dssim_loss_and_grad(img, gt, self.lambda_dssim / B, total, d_img)
                             img.backward(d_img)
                             loss = None
                         else:
+                            if self.lambda_dssim > 0.0:
+                                raise NotImplementedError("lambda_dssim > 0 needs the fused path (our own render on the GPU)")
                             diff = pkg["render"] - gt
                             loss = diff.abs().mean() / B
                             sse_plain.append((diff.detach() ** 2).sum().reshape(1))

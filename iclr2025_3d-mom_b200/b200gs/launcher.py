@@ -9,7 +9,8 @@ reference's compiled extensions, (2) appends import shims for third-party module
 `GaussianModel` looks it up (scene/gaussian_model.py:21,53), (4) makes `training_setup` build the fused
 multi-tensor Adam from the very param groups the reference assembles (gaussian_model.py:197-209), and
 (5) installs the one-launch prune / cat bookkeeping (gaussian_model.py:424-482) and (6) routes
-`compute_regulation` (gaussian_model.py:768-769) to the fused plane-regulariser kernel. The reference tree is
+`compute_regulation` (gaussian_model.py:768-769) to the fused plane-regulariser kernel, and (7) routes
+`utils.loss_utils.ssim` (the opt.lambda_dssim term) to the fused SSIM kernels (patch_loss_utils). The reference tree is
 never modified.
 """
 import os
@@ -43,6 +44,44 @@ def _library_version_shims():
         return real(obj, mode, *a, **k)
     fromarray._b200gs_int8 = True
     Image.fromarray = fromarray
+
+
+def fused_ssim_supported(img1, img2, window_size=11, size_average=True):
+    """Whether fusedops.ssim computes what utils/loss_utils.py:ssim would for these arguments: window 11, two float32 CUDA
+    tensors of one shape [N,C,H,W] (or [C,H,W] with size_average, which the reference reduces with .mean() only), no
+    gradient wanted for img2.  Looks at metadata only; launches nothing."""
+    import torch
+    if window_size != 11 or not (isinstance(img1, torch.Tensor) and isinstance(img2, torch.Tensor)):
+        return False
+    if not (img1.is_cuda and img2.is_cuda and img1.device == img2.device):
+        return False
+    if img1.dtype != torch.float32 or img2.dtype != torch.float32 or img1.shape != img2.shape or img1.numel() == 0:
+        return False
+    if not (img1.dim() == 4 or (img1.dim() == 3 and size_average)):
+        return False
+    return not (img2.requires_grad and torch.is_grad_enabled())
+
+
+def patch_loss_utils(module):
+    """Replaces `module.ssim` (the reference's utils.loss_utils) by a wrapper that sends the calls fusedops.ssim covers
+    (fused_ssim_supported) to the fused kernels and every other call to the original function.  Idempotent.
+    B200GS_FUSED_SSIM=0 leaves the module as it is.  Returns the module."""
+    if os.environ.get("B200GS_FUSED_SSIM", "1") == "0":
+        return module
+    orig = getattr(module, "ssim", None)
+    if orig is None or getattr(orig, "_b200gs_fused", False):
+        return module
+
+    def ssim(img1, img2, window_size=11, size_average=True):
+        if fused_ssim_supported(img1, img2, window_size, size_average):
+            from . import fusedops
+            return fusedops.ssim(img1, img2, window_size, size_average)
+        return orig(img1, img2, window_size, size_average)
+    ssim._b200gs_fused = True
+    ssim._b200gs_original = orig
+    ssim.__doc__ = orig.__doc__
+    module.ssim = ssim
+    return module
 
 
 def install(reference_root):
@@ -106,6 +145,13 @@ def install(reference_root):
             return __orig(self, time_smoothness_weight, l1_time_planes_weight, plane_tv_weight)
         gm.GaussianModel.compute_regulation = compute_regulation
         gm.GaussianModel._b200gs_patched = True
+    # train_4DGS.py imports `ssim` from utils.loss_utils when it starts (after this point): the lambda_dssim term runs fused
+    try:
+        import utils.loss_utils as loss_utils
+    except ImportError:                     # a script that cannot import it cannot call its ssim either
+        loss_utils = None
+    if loss_utils is not None:
+        patch_loss_utils(loss_utils)
     return gm
 
 

@@ -331,6 +331,26 @@ int b200gs_l1_loss_fwd_bwd(long long n, const float* render, const float* target
 int b200gs_l1_loss_fwd_bwd_u8(int H, int W, const float* render_chw, const unsigned char* target_hwc, float scale, float* loss_accum,
                               float* sse_accum, float* d_render_chw, b200gs_stream_t stream);
 
+/* SSIM of utils/loss_utils.py:ssim (the 3DGS formulation: 11x11 Gaussian window, sigma 1.5, zero padding, C1 = 0.01^2,
+ * C2 = 0.03^2) with its gradient, for the D-SSIM term lambda_dssim * (1 - ssim) of train_4DGS.py.  x, y are [N,C,H,W] FP32
+ * (any N, C, H, W >= 1, N * C <= 65535); map(n,c,p) is the SSIM map of that pixel.
+ *   ssim_sum (may be null): ssim_sum[n] += value_offset + value_scale * sum_{c,p} map(n,c,p) for every image n, one FP32 add
+ *     of a value formed in FP64 (the map sums are accumulated in FP64 in the scratch).  value_offset 0, value_scale
+ *     1 / (C*H*W) on a zeroed ssim_sum gives each image's SSIM; offset w, scale -w / (C*H*W) adds w * (1 - SSIM) to a loss.
+ *   d_x (may be null = value only): d_x += weight * d(sum_{n,c,p} map)/dx, ADDED to what the buffer holds (so it can share
+ *     the buffer the L1 kernel wrote).  Forward, then backward launch; the map's partial derivatives pass between them
+ *     through the scratch.
+ *   scratch: b200gs_ssim_scratch_bytes(N, C, H, W, with_grad = d_x != null) bytes of device memory, no initial contents
+ *     (8 bytes per image, plus 12 bytes per element with the gradient).
+ * Returns 0 without launching when both ssim_sum and d_x are null. */
+size_t b200gs_ssim_scratch_bytes(int N, int C, int H, int W, int with_grad);
+int b200gs_ssim_fwd_bwd(int N, int C, int H, int W, const float* x, const float* y, float value_offset, float value_scale,
+                        float* ssim_sum, float weight, float* d_x, void* scratch, size_t scratch_bytes, b200gs_stream_t stream);
+/* The same for one [3,H,W] image against the uint8 [H,W,3] ground truth (N = 1, C = 3), converted on the device as
+ * float(u8) / 255.0f like b200gs_l1_loss_fwd_bwd_u8: identical results to the FP32 entry on the converted target. */
+int b200gs_ssim_fwd_bwd_u8(int H, int W, const float* x_chw, const unsigned char* y_hwc, float value_offset, float value_scale,
+                           float* ssim_sum, float weight, float* d_x_chw, void* scratch, size_t scratch_bytes, b200gs_stream_t stream);
+
 /* Is the [n] float tensor x one value repeated?  gaussian_renderer/__init__.py:56 hands the field the camera's single timestamp as
  * a materialised [P,1] tensor; when it is uniform the field takes its one-timestamp fast path (time planes from shared memory).
  * scratch_dev2: 8 bytes of device memory; host_pinned2: 8 bytes of PINNED host memory, on return [0] = 1 if uniform else 0,
