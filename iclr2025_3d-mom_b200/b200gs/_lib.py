@@ -115,7 +115,8 @@ class CallTimer:
     # kernels launched per call (for the launch count): see csrc/api.cu and the per-file launchers
     KERNELS = {"b200gs_rast_forward_stage1": 7, "b200gs_rast_forward_stage2": 7, "b200gs_rast_backward": 2, "b200gs_rast_backward_accumulate_sh": 2,
                "b200gs_hexplane_order": 6, "b200gs_hexplane_forward": 1, "b200gs_hexplane_forward_masked": 1, "b200gs_hexplane_backward_masked": 1, "b200gs_hexplane_time_forward": 1, "b200gs_hexplane_time_backward": 1, "b200gs_hexplane_backward": 1, "b200gs_hexplane_regulation": 1,
-               "b200gs_deform_mlp_forward": 1, "b200gs_deform_mlp_backward": 1, "b200gs_adam_multi": 1, "b200gs_adam_sh": 1,
+               "b200gs_deform_mlp_forward": 1, "b200gs_deform_mlp_backward": 1, "b200gs_deform_heads_forward": 1, "b200gs_deform_heads_backward": 1,
+               "b200gs_adam_multi": 1, "b200gs_adam_sh": 1,
                "b200gs_activations_forward": 1, "b200gs_activations_backward": 1, "b200gs_l1_loss_fwd_bwd": 1, "b200gs_l1_loss_fwd_bwd_u8": 1,
                "b200gs_ssim_fwd_bwd": 3, "b200gs_ssim_fwd_bwd_u8": 3,   # forward, backward, sum (the trainer always asks for the gradient)
                "b200gs_gather_rows_multi": 1, "b200gs_dist2": 8, "b200gs_mark_visible": 1, "b200gs_sort_pairs_u32": 6}

@@ -341,14 +341,24 @@ class LossRing:
         return float(self.host[i])
 
 
-def _receives_grad(name, stage):
-    """Parameters the reference's loss reaches (SURVEY.md Appendix C iii): timenet, the opacity /
-    SH heads and the aabb never do; in the coarse stage the whole deformation field is bypassed."""
+def _receives_grad(name, stage, no_do=True, no_dshs=True):
+    """Parameters the reference's loss reaches (SURVEY.md Appendix C iii): timenet and the aabb never do, the opacity / SH
+    heads only when they are on (no_do / no_dshs False); in the coarse stage the whole deformation field is bypassed."""
     if name.startswith("_deformation."):
         if stage == "coarse":
             return False
-        return not ("timenet" in name or "opacity_deform" in name or "shs_deform" in name or name.endswith("grid.aabb"))
+        if "opacity_deform" in name:
+            return not no_do
+        if "shs_deform" in name:
+            return not no_dshs
+        return not ("timenet" in name or name.endswith("grid.aabb"))
     return True
+
+
+def _head_flags(model):
+    """(no_do, no_dshs) of the model's deformation field; (True, True) for a model without one."""
+    args = getattr(getattr(getattr(model, "_deformation", None), "deformation_net", None), "args", None)
+    return bool(getattr(args, "no_do", True)), bool(getattr(args, "no_dshs", True))
 
 
 class ViewParallelTrainer:
@@ -425,7 +435,7 @@ class ViewParallelTrainer:
         # flat gradient arena: [every parameter the loss reaches except (shared_shs) the SH tensors | screen-space xy per
         # Gaussian]; p.grad are views into it, so autograd accumulates in place and ONE collective (fp32 sum over
         # NVLink/NVSwitch) reduces it. Parameters outside it keep grad None and the optimiser skips them, as torch does.
-        named = [(n, p) for n, p in model.named_parameters() if p.requires_grad and _receives_grad(n, stage)]
+        named = [(n, p) for n, p in model.named_parameters() if p.requires_grad and _receives_grad(n, stage, *_head_flags(model))]
         is_sh = lambda n: n in ("_features_dc", "_features_rest")
         self.sh_params = [p for n, p in named if is_sh(n)] if self.shared_shs else []
         if len(self.sh_params) != 2:
@@ -558,6 +568,9 @@ class ViewParallelTrainer:
             m._features_dc.grad = None
             m._features_rest.grad = None
         from . import field as _field
+        # SH head on: the rasterizer sees shs' (not the step's leaf), so its SH gradient goes back through autograd to the
+        # field, whose heads backward adds it into the step's SH buffer
+        sh_head = self.stage == "fine" and not _head_flags(m)[1]
         share_spatial = self.shared_shs and self.stage == "fine" and len(cams) > 1 and m._xyz.is_cuda
         if share_spatial:
             _field.begin_shared_step(m._deformation, m._xyz)
@@ -602,8 +615,10 @@ class ViewParallelTrainer:
                     torch.maximum(self.max_radii, pkg["radii"], out=self.max_radii)
                     _field.ACCUMULATE_INTO_GRAD = self.shared_shs     # p.grad are arena views: let the field kernels add into them
                     on_gpu = shs is not None and shs.is_cuda
-                    _rast.SH_GRAD_ACCUMULATOR = self.sh_grad if on_gpu else None
+                    _rast.SH_GRAD_ACCUMULATOR = self.sh_grad if on_gpu and not sh_head else None
                     _rast.SH_GRAD_OVERWRITE = first_sh
+                    _field.SH_GRAD_ACCUMULATOR = self.sh_grad if on_gpu and sh_head else None
+                    _field.SH_GRAD_OVERWRITE = first_sh
                     if on_gpu and self.overlap_sh_reduce and vi == len(cams) - 1:
                         # The SH tail starts from inside the LAST view's backward.  The SH gradient is complete as soon as the
                         # rasterizer backward has been queued, but the deformation-MLP backward that follows is a persistent kernel
@@ -611,7 +626,7 @@ class ViewParallelTrainer:
                         # delays those CTAs by the collective's whole duration (measured at N = 8: 0.60 -> 1.22 ms).  So the tail
                         # is started right AFTER the MLP backward has been queued and overlaps the time-plane / spatial HexPlane
                         # backward, the arena all-reduce and the regulariser instead -- ordinary kernels that share SMs gracefully.
-                        if self.stage == "fine" and hasattr(_field, "AFTER_MLP_BACKWARD") and not early:
+                        if self.stage == "fine" and hasattr(_field, "AFTER_MLP_BACKWARD") and (sh_head or not early):
                             _field.AFTER_MLP_BACKWARD = self._sh_tail
                         else:
                             _rast.AFTER_SH_ACCUMULATE = self._sh_tail
@@ -641,6 +656,8 @@ class ViewParallelTrainer:
                         _field.ACCUMULATE_INTO_GRAD = False
                         _rast.SH_GRAD_ACCUMULATOR = None
                         _rast.SH_GRAD_OVERWRITE = False
+                        _field.SH_GRAD_ACCUMULATOR = None
+                        _field.SH_GRAD_OVERWRITE = False
                         _rast.AFTER_SH_ACCUMULATE = None
                         _field.AFTER_MLP_BACKWARD = None
                     first_sh = False

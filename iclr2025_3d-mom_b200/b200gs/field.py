@@ -5,7 +5,8 @@ arguments, attribute paths, parameter names / shapes (so `state_dict()` keys suc
 `deformation_net.grid.grids.{level}.{plane}`, `deformation_net.grid.aabb`,
 `deformation_net.feature_out.0.weight`, `timenet.*`, `*_poc` match), same call signatures and
 return values — while forward and backward run the hand-written sm_100a kernels of
-libb200gs (csrc/hexplane.cu, csrc/deform_mlp.cu) through `torch.autograd.Function`s.
+libb200gs (csrc/hexplane.cu, csrc/deform_mlp*.cu and, with `no_do` / `no_dshs` False, csrc/deform_heads.cu for the
+opacity and SH heads) through `torch.autograd.Function`s.
 
 Differences that do not change results:
   * plane parameters keep their [1, 32, H, W] shape but use torch.channels_last strides (one
@@ -45,6 +46,16 @@ class _MlpWeights(ctypes.Structure):
 class _MlpGrads(ctypes.Structure):
     _fields_ = [("w1", ctypes.c_void_p), ("b1", ctypes.c_void_p), ("w2", ctypes.c_void_p * 3),
                 ("b2", ctypes.c_void_p * 3), ("w3", ctypes.c_void_p * 3), ("b3", ctypes.c_void_p * 3)]
+
+
+class _HeadsWeights(ctypes.Structure):
+    _fields_ = [("feat_dim", ctypes.c_int), ("width", ctypes.c_int), ("w1", ctypes.c_void_p), ("w2", ctypes.c_void_p * 2),
+                ("b2", ctypes.c_void_p * 2), ("w3", ctypes.c_void_p * 2), ("b3", ctypes.c_void_p * 2), ("feat_tiled", ctypes.c_int)]
+
+
+class _HeadsGrads(ctypes.Structure):
+    _fields_ = [("w1", ctypes.c_void_p), ("b1", ctypes.c_void_p), ("w2", ctypes.c_void_p * 2),
+                ("b2", ctypes.c_void_p * 2), ("w3", ctypes.c_void_p * 2), ("b3", ctypes.c_void_p * 2)]
 
 
 _P = ctypes.c_void_p
@@ -112,6 +123,12 @@ _lib.register("b200gs_deform_mlp_forward", ctypes.c_int,
                _P, _P, _P, _P, _P])
 _lib.register("b200gs_deform_mlp_backward", ctypes.c_int,
               [ctypes.POINTER(_MlpWeights), ctypes.POINTER(_MlpGrads), ctypes.c_longlong, _P, _P, _P, _P, _P, _P, _P])
+_lib.register("b200gs_deform_heads_saved_floats", ctypes.c_size_t, [ctypes.c_longlong])
+_lib.register("b200gs_deform_heads_forward", ctypes.c_int,
+              [ctypes.POINTER(_HeadsWeights), ctypes.c_longlong, ctypes.c_int, _P, _P, _P, _P, _P, _P, _P])
+_lib.register("b200gs_deform_heads_backward", ctypes.c_int,
+              [ctypes.POINTER(_HeadsWeights), ctypes.POINTER(_HeadsGrads), ctypes.c_longlong, ctypes.c_int, _P, _P, _P, _P, _P, _P,
+               _P, ctypes.c_int, _P])
 _lib.register("b200gs_hexplane_regulation", ctypes.c_int,
               [ctypes.POINTER(_HexDesc), ctypes.c_float, ctypes.c_float, ctypes.c_float, _P, _P])
 
@@ -233,6 +250,11 @@ ACCUMULATE_INTO_GRAD = False
 # Optional callable invoked right after the deformation-MLP backward kernel of a view has been queued (the trainer starts the SH
 # gradient's side-stream all-reduce + Adam there on the last view of a step); None = nothing.
 AFTER_MLP_BACKWARD = None
+# Set by the trainer for the duration of a view when the SH head is on: the [P,16,3] buffer the step's SH gradient collects in.
+# The heads backward adds d shs (= d shs', the identity path) into it -- writes it when SH_GRAD_OVERWRITE, the step's first
+# view -- and autograd gets None for `shs`.  None = the gradient goes to autograd.
+SH_GRAD_ACCUMULATOR = None
+SH_GRAD_OVERWRITE = False
 
 
 def _grad_target(param):
@@ -434,18 +456,21 @@ def _auto_spatial(xyz, grid):
 
 
 class _DeformFn(torch.autograd.Function):
-    """(pts, scales, rot) = field(xyz, scales, rot, t, scene_flow, frame_num, delta_scale).
+    """(pts, scales, rot[, opacity'][, shs']) = field(xyz, scales, rot, opacity, shs, t, scene_flow, frame_num, delta_scale).
 
-    inputs: xyz, scales, rot, times, scene_flow, frame_num, delta_scale, aabb, levels, res, heads, S_in,
-            w1, b1, (w2,b2,w3,b3) x 3 heads, *planes
+    inputs: xyz, scales, rot, opacity, shs, times, scene_flow, frame_num, delta_scale, aabb, levels, res, heads, S_in,
+            need_backward, w1, b1, (w2,b2,w3,b3) x 5 heads, *planes
+    heads: (pos, scales, rotations, opacity, shs) on / off.  opacity' / shs' are returned only for the heads that are on
+    (csrc/deform_heads.cu); opacity / shs may be None when their head is off.
     S_in: None, or the differentiable spatial product of _SpatialFn (then only the time planes are sampled here and
     dL/dS_in is returned for autograd to sum over the views of a batch).
     """
-    N_FIXED = 13
-    N_W = 14
+    N_FIXED = 15
+    N_W = 22
 
     @staticmethod
-    def forward(ctx, xyz, scales, rot, times, scene_flow, frame_num, delta_scale, aabb, levels, res, heads, S_in, need_backward, *rest):
+    def forward(ctx, xyz, scales, rot, opacity, shs, times, scene_flow, frame_num, delta_scale, aabb, levels, res, heads, S_in,
+                need_backward, *rest):
         weights, planes = rest[:_DeformFn.N_W], rest[_DeformFn.N_W:]
         xyz = xyz.contiguous(); scales = scales.contiguous(); rot = rot.contiguous(); scene_flow = scene_flow.contiguous()
         _check_cuda_f32(xyz, scales, rot, scene_flow, aabb, *planes, *[w for w in weights if w is not None])
@@ -490,8 +515,10 @@ class _DeformFn(torch.autograd.Function):
                   "hexplane_forward")
         mw = _DeformFn._weights_struct(weights, heads, 32 * levels)
         mw.feat_tiled = int(ctx.feat_tiled)
-        # inference (the caller knows no backward will follow: torch.no_grad() or nothing requires grad): no activation stash
-        stash = need_backward or not all(heads)
+        extra = heads[3] or heads[4]
+        # inference (the caller knows no backward will follow: torch.no_grad() or nothing requires grad): no activation stash,
+        # unless the opacity / SH heads run: they read relu(hidden) from it
+        stash = need_backward or not all(heads[:3]) or extra
         saved = torch.empty((L.b200gs_deform_mlp_saved_floats(P),), dtype=torch.float32, device=dev) if stash else None
         pts_o = torch.empty_like(xyz); scales_o = torch.empty_like(scales); rot_o = torch.empty_like(rot)
         if torch.is_tensor(frame_num):
@@ -503,13 +530,42 @@ class _DeformFn(torch.autograd.Function):
                                           rot.data_ptr(), scene_flow.data_ptr(), fn_val, fn_ptr, float(delta_scale),
                                           pts_o.data_ptr(), scales_o.data_ptr(), rot_o.data_ptr(), saved.data_ptr() if saved is not None else None, stream),
               "deform_mlp_forward")
+        outs = [pts_o, scales_o, rot_o]
+        hsaved = torch.empty(0, device=dev)
+        if extra:
+            op_in = opacity.contiguous() if heads[3] else None
+            sh_in = shs.contiguous() if heads[4] else None
+            _check_cuda_f32(op_in, sh_in)
+            if need_backward:
+                hsaved = torch.empty((L.b200gs_deform_heads_saved_floats(P),), dtype=torch.float32, device=dev)
+            op_o = torch.empty_like(op_in) if op_in is not None else None
+            sh_o = torch.empty_like(sh_in) if sh_in is not None else None
+            hw = _DeformFn._heads_struct(weights, heads, 32 * levels, ctx.feat_tiled)
+            check(L.b200gs_deform_heads_forward(ctypes.byref(hw), P, _sh_coeffs(sh_in), saved.data_ptr(), _lib.ptr(op_in),
+                                                _lib.ptr(sh_in), _lib.ptr(op_o), _lib.ptr(sh_o),
+                                                hsaved.data_ptr() if hsaved.numel() else None, stream), "deform_heads_forward")
+            _lib.COUNTERS["deform_heads_forward"] += 1
+            outs += [o for o in (op_o, sh_o) if o is not None]
         if saved is None:
             saved = torch.empty(0, device=dev)
-        ctx.save_for_backward(xyz, tt if tt is not None else torch.empty(0), aabb, feat, saved,
+        ctx.save_for_backward(xyz, tt if tt is not None else torch.empty(0), aabb, feat, saved, hsaved,
                               *[w if w is not None else torch.empty(0) for w in weights], *planes)
         ctx.meta = (levels, res, heads, ts, tt is not None)
         ctx.params = (weights, planes)          # the Parameter objects themselves (for _grad_target)
-        return pts_o, scales_o, rot_o
+        return tuple(outs)
+
+    @staticmethod
+    def _heads_struct(weights, heads, feat_dim, feat_tiled):
+        hw = _HeadsWeights()
+        hw.feat_dim = feat_dim
+        hw.width = int(weights[0].shape[0])
+        hw.w1 = weights[0].data_ptr()
+        hw.feat_tiled = int(feat_tiled)
+        for h in range(2):
+            if heads[3 + h]:
+                w2, b2, w3, b3 = weights[14 + 4 * h: 18 + 4 * h]
+                hw.w2[h], hw.b2[h], hw.w3[h], hw.b3[h] = w2.data_ptr(), b2.data_ptr(), w3.data_ptr(), b3.data_ptr()
+        return hw
 
     @staticmethod
     def _weights_struct(weights, heads, feat_dim):
@@ -527,8 +583,8 @@ class _DeformFn(torch.autograd.Function):
         return mw
 
     @staticmethod
-    def backward(ctx, d_pts, d_scales, d_rot):
-        xyz, tt, aabb, feat, saved, *rest = ctx.saved_tensors
+    def backward(ctx, d_pts, d_scales, d_rot, *d_extra):
+        xyz, tt, aabb, feat, saved, hsaved, *rest = ctx.saved_tensors
         weights, planes = rest[:_DeformFn.N_W], rest[_DeformFn.N_W:]
         levels, res, heads, ts, has_t = ctx.meta
         if saved.numel() == 0:
@@ -541,7 +597,10 @@ class _DeformFn(torch.autograd.Function):
         pw, pp = ctx.params
         direct_w = [_grad_target(q) if q is not None else None for q in pw]
         direct_p = [_grad_target(q) for q in pp]
-        gws = [(dw if dw is not None else torch.zeros_like(w)) if w.numel() else None for w, dw in zip(weights, direct_w)]
+        # (the weights of a disabled opacity / SH head get no buffer: with both off nothing is allocated beyond the three heads)
+        live = [i < 14 or heads[3 + (i - 14) // 4] for i in range(len(weights))]
+        gws = [(dw if dw is not None else torch.zeros_like(w)) if (w.numel() and on) else None
+               for w, dw, on in zip(weights, direct_w, live)]
         mg = _MlpGrads()
         mg.w1 = gws[0].data_ptr(); mg.b1 = gws[1].data_ptr()
         for h in range(3):
@@ -555,6 +614,30 @@ class _DeformFn(torch.autograd.Function):
         check(L.b200gs_deform_mlp_backward(ctypes.byref(mw), ctypes.byref(mg), P, feat.data_ptr(), saved.data_ptr(),
                                            cp(d_pts) if heads[0] else None, cp(d_scales) if heads[1] else None,
                                            cp(d_rot) if heads[2] else None, d_feat.data_ptr(), stream), "deform_mlp_backward")
+        d_op = d_sh = None
+        if heads[3] or heads[4]:
+            if hsaved.numel() == 0:
+                raise RuntimeError("deform_network: backward through a forward that ran in inference mode (no heads stash)")
+            # after the three-head backward (which WROTE d_feat, dW1, db1) and before the HexPlane backward reads d_feat
+            d_extra = [t.contiguous() if t is not None else None for t in d_extra]
+            d_op = d_extra[0] if heads[3] else None
+            d_sh = d_extra[-1] if heads[4] else None
+            acc = SH_GRAD_ACCUMULATOR
+            use_acc = (d_sh is not None and acc is not None and acc.shape == d_sh.shape and acc.is_contiguous()
+                       and acc.device == d_sh.device and acc.dtype == torch.float32)
+            hg = _HeadsGrads()
+            hg.w1 = gws[0].data_ptr(); hg.b1 = gws[1].data_ptr()
+            for h in range(2):
+                if heads[3 + h]:
+                    hg.w2[h], hg.b2[h], hg.w3[h], hg.b3[h] = (gws[i].data_ptr() for i in range(14 + 4 * h, 18 + 4 * h))
+            hw = _DeformFn._heads_struct(weights, heads, 32 * levels, ctx.feat_tiled)
+            check(L.b200gs_deform_heads_backward(ctypes.byref(hw), ctypes.byref(hg), P, _sh_coeffs(d_sh), feat.data_ptr(),
+                                                 saved.data_ptr(), hsaved.data_ptr(), cp(d_op), cp(d_sh), d_feat.data_ptr(),
+                                                 acc.data_ptr() if use_acc else None, int(use_acc and SH_GRAD_OVERWRITE), stream),
+                  "deform_heads_backward")
+            _lib.COUNTERS["deform_heads_backward"] += 1
+            if use_acc:
+                d_sh = None                     # already in the step's SH buffer
         if AFTER_MLP_BACKWARD is not None:
             AFTER_MLP_BACKWARD()
         sh = ctx.shared
@@ -594,12 +677,20 @@ class _DeformFn(torch.autograd.Function):
         # pts = xyz*1 + ..., scales = scales*1 + ds, rot = rot + dr: identity paths
         d_xyz = d_xyz_grid + d_pts if d_pts is not None else d_xyz_grid
         gw_out = [None if dw is not None else g for g, dw in zip(gws, direct_w)]      # accumulated in place -> nothing for autograd
-        for h in range(3):
+        for h in range(5):
             if not heads[h]:
                 for i in range(2 + 4 * h, 6 + 4 * h):
                     gw_out[i] = None
         gp_out = [None if dp is not None else g for g, dp in zip(gplanes, direct_p)]
-        return (d_xyz, d_scales, d_rot, None, None, None, None, None, None, None, None, d_S, None, *gw_out, *gp_out)
+        # opacity' = opacity * 1 + ..., shs' = shs * 1 + ...: identity paths
+        return (d_xyz, d_scales, d_rot, d_op, d_sh, None, None, None, None, None, None, None, None, d_S, None, *gw_out, *gp_out)
+
+
+def _sh_coeffs(shs):
+    """SH coefficients per point of a [P, M, 3] tensor (None: no SH head), -1 for any other shape (the kernels refuse it)."""
+    if shs is None:
+        return 16
+    return int(shs.shape[1]) if shs.dim() == 3 and shs.shape[2] == 3 else -1
 
 
 def _regulation_launch(field, weights, loss_accum, grads):
@@ -751,8 +842,6 @@ class Deformation(nn.Module):
         if args.static_mlp: unsupported.append("static_mlp")
         if grid_pe != 0: unsupported.append("grid_pe")
         if getattr(args, "apply_rotation", False): unsupported.append("apply_rotation")
-        if not args.no_do: unsupported.append("no_do=False")
-        if not args.no_dshs: unsupported.append("no_dshs=False")
         if D > 1: unsupported.append("defor_depth>1")
         if W != 64: unsupported.append("net_width!=64")
         if unsupported:
@@ -794,9 +883,9 @@ class Deformation(nn.Module):
     def forward_dynamic(self, rays_pts_emb, scales_emb, rotations_emb, opacity_emb, shs_emb, time_feature, time_emb,
                         scene_flow, frame_num, delta_scale):
         a = self.args
-        heads = (not a.no_dx, not a.no_ds, not a.no_dr)
+        heads = (not a.no_dx, not a.no_ds, not a.no_dr, not a.no_do, not a.no_dshs)
         weights = [self.feature_out[0].weight, self.feature_out[0].bias]
-        for m in (self.pos_deform, self.scales_deform, self.rotations_deform):
+        for m in (self.pos_deform, self.scales_deform, self.rotations_deform, self.opacity_deform, self.shs_deform):
             weights += [m[1].weight, m[1].bias, m[3].weight, m[3].bias]
         xyz = rays_pts_emb[:, :3]
         if scene_flow is None:
@@ -809,6 +898,7 @@ class Deformation(nn.Module):
         t_arg = time_emb[:, :1] if torch.is_tensor(time_emb) else float(time_emb)
         S_in = None
         need_backward = torch.is_grad_enabled() and (any(t.requires_grad for t in (rays_pts_emb, scales_emb, rotations_emb))
+                                                     or (heads[3] and opacity_emb.requires_grad) or (heads[4] and shs_emb.requires_grad)
                                                      or any(w.requires_grad for w in weights) or self.grid.grids[0][0].requires_grad)
         if torch.is_tensor(t_arg) and xyz.is_cuda:
             # the reference's render() hands over the camera's ONE timestamp as a [P,1] tensor (gaussian_renderer/__init__.py:56)
@@ -817,11 +907,15 @@ class Deformation(nn.Module):
         if (AUTOGRAD_SPATIAL_SHARING and not torch.is_tensor(t_arg) and xyz.is_cuda and torch.is_grad_enabled() and _SHARED is None
                 and self.grid._time_rows_supported() and (xyz.requires_grad or self.grid.grids[0][0].requires_grad)):
             S_in = _auto_spatial(xyz, self.grid)
-        pts, scales, rotations = _DeformFn.apply(xyz, scales_emb[:, :3], rotations_emb[:, :4], t_arg, scene_flow,
-                                                 frame_num, delta_scale, self.grid.aabb, len(self.grid.grids),
-                                                 tuple(self.grid._res), heads, S_in, need_backward, *weights, *self.grid._planes())
-        opacity = opacity_emb[:, :1]
-        shs = shs_emb
+        if heads[4] and not (shs_emb.dim() == 3 and tuple(shs_emb.shape[1:]) == (16, 3)):
+            raise NotImplementedError(f"b200gs Deformation: the SH head needs shs of shape [P,16,3], got {tuple(shs_emb.shape)}")
+        out = _DeformFn.apply(xyz, scales_emb[:, :3], rotations_emb[:, :4], opacity_emb[:, :1] if heads[3] else None,
+                              shs_emb if heads[4] else None, t_arg, scene_flow, frame_num, delta_scale, self.grid.aabb,
+                              len(self.grid.grids), tuple(self.grid._res), heads, S_in, need_backward, *weights,
+                              *self.grid._planes())
+        pts, scales, rotations = out[:3]
+        opacity = out[3] if heads[3] else opacity_emb[:, :1]
+        shs = out[-1] if heads[4] else shs_emb
         return pts, scales, rotations, opacity, shs
 
     def get_mlp_parameters(self):

@@ -266,6 +266,38 @@ int b200gs_deform_mlp_backward(const b200gs_mlp_weights* w /* host */, const b20
                                long long P, const float* features, const float* saved, const float* d_pts,
                                const float* d_scales, const float* d_rot, float* d_features, b200gs_stream_t stream);
 
+/* Opacity and SH deformation heads (no_do = False / no_dshs = False; deformation.py:97-153 with mask = ones):
+ *     opacity_out[P,1] = opacity * 1 + opacity_deform(hidden)      opacity_deform: ReLU, Linear(64,64), ReLU, Linear(64,1)
+ *     shs_out[P,16,3]  = shs * 1 + shs_deform(hidden)              shs_deform:     ReLU, Linear(64,64), ReLU, Linear(64,48)
+ * They run beside the three geometry heads and read relu(hidden) from the stash b200gs_deform_mlp_forward left (which must
+ * therefore have been given one).  w2[0] / w2[1] null = that head off; at least one must be on. */
+typedef struct {
+    int feat_dim;                 /* 64 or 128, as in b200gs_mlp_weights */
+    int width;                    /* net_width, 64 */
+    const float* w1;              /* feature_out.0 [64, feat_dim] (backward only: d_features += d_h W1) */
+    const float* w2[2]; const float* b2[2];     /* {opacity,shs}_deform.1  [64,64], [64] */
+    const float* w3[2]; const float* b3[2];     /* {opacity,shs}_deform.3  [k,64], [k], k = 1, 48 */
+    int feat_tiled;               /* layout of features / d_features, as in b200gs_mlp_weights */
+} b200gs_heads_weights;
+/* gradients of b200gs_heads_weights' arrays (w1 / b1: feature_out.0).  w1, the w2[h] of every enabled head and the SH head's
+ * w3 must be 16-byte aligned (128-bit vector reductions). */
+typedef struct { float* w1; float* b1; float* w2[2]; float* b2[2]; float* w3[2]; float* b3[2]; } b200gs_heads_grads;
+/* floats of the heads' own activation stash: relu(z_opacity), relu(z_sh) in the layout of the three-head stash */
+size_t b200gs_deform_heads_saved_floats(long long P);
+/* mlp_saved: the stash of the matching b200gs_deform_mlp_forward call.  opacity [P,1], shs [P,sh_coeffs,3] (sh_coeffs must
+ * be 16 when the SH head is on).  heads_saved: b200gs_deform_heads_saved_floats(P) floats for the backward, or NULL. */
+int b200gs_deform_heads_forward(const b200gs_heads_weights* w /* host */, long long P, int sh_coeffs, const float* mlp_saved,
+                                const float* opacity, const float* shs, float* opacity_out, float* shs_out, float* heads_saved,
+                                b200gs_stream_t stream);
+/* Run AFTER b200gs_deform_mlp_backward of the same view: ADDS the heads' share into d_features (same layout), gw->w1 and
+ * gw->b1, and accumulates the heads' own weight gradients.  d_opacity [P,1] / d_shs [P,16,3]: upstream gradients of the
+ * outputs (null = zero).  sh_grad (may be null): a [P,16,3] buffer that receives d_shs as well (the gradient of the `shs`
+ * input: an identity path), written instead of added to when sh_grad_overwrite != 0. */
+int b200gs_deform_heads_backward(const b200gs_heads_weights* w /* host */, const b200gs_heads_grads* gw /* host */, long long P,
+                                 int sh_coeffs, const float* features, const float* mlp_saved, const float* heads_saved,
+                                 const float* d_opacity, const float* d_shs, float* d_features, float* sh_grad,
+                                 int sh_grad_overwrite, b200gs_stream_t stream);
+
 /* Plane-subset variants: features = factor * prod_{k in plane_mask} plane_k (bit k of plane_mask = plane k; factor may be
  * null = 1).  With the spatial planes (0,1,3: mask 0x0B) evaluated once per optimiser step and handed back as `factor`,
  * each view of a multi-view batch only samples the time planes (2,4,5: mask 0x34): the Gaussians' xyz do not change
