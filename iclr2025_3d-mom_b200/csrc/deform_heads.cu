@@ -18,7 +18,7 @@
 // whole chain; weight gradients accumulate in fragments over every tile of a persistent CTA and are flushed once).  Same
 // rounding rules as the three-head backwards: the dX chain runs the full three-term split, dY stays exact (hi + lo) in the
 // weight gradients, X is rounded to TF32 once, bias gradients are FP32 sums.
-#include "tc5_common.cuh"
+#include "mma_tf32.cuh"
 #include "../../include/b200gs.h"
 
 namespace b200gs {
@@ -41,33 +41,6 @@ struct FwdArgs {
     float* saved;                         // 2 planes: relu(z_opacity), relu(z_sh); null = inference
 };
 
-// torch [N_real x K] row-major -> hi / lo K-major UMMA operands with N rows (zero padded)
-__device__ __forceinline__ void stage_kmajor(float* __restrict__ hi, float* __restrict__ lo, const float* __restrict__ w,
-                                             int N, int N_real, int K)
-{
-    for (int i = threadIdx.x; i < N * K; i += FT) {
-        const int n = i / K, k = i - n * K;
-        const float v = n < N_real ? __ldg(w + (size_t)n * K + k) : 0.f;
-        const u32 h = tc5::to_tf32(v), l = tc5::to_tf32(v - __uint_as_float(h));
-        const int off = (k >> 2) * (N * 4) + n * 4 + (k & 3);
-        hi[off] = __uint_as_float(h);
-        lo[off] = __uint_as_float(l);
-    }
-}
-
-// D (+)= (Ahi + Alo)(Bhi + Blo) without lo*lo, K = 64, small terms first
-__device__ __forceinline__ void issue_split(u32 d_tmem, u32 a_hi, u32 a_lo, u32 b_hi_smem, u32 b_lo_smem, int N)
-{
-    const u64 dh = tc5::kmajor_desc(b_hi_smem, N), dl = tc5::kmajor_desc(b_lo_smem, N);
-    const u64 step = (u64)((2 * N * 16) >> 4);
-    const u32 idesc = tc5::make_idesc(128, N);
-    for (int j = 0; j < MW / 8; ++j) {
-        tc5::mma_ts(d_tmem, a_lo + 8 * j, dh + step * j, idesc, j > 0);
-        tc5::mma_ts(d_tmem, a_hi + 8 * j, dl + step * j, idesc, 1u);
-        tc5::mma_ts(d_tmem, a_hi + 8 * j, dh + step * j, idesc, 1u);
-    }
-}
-
 __global__ void __launch_bounds__(FT, 1) deform_heads_fwd_kernel(const __grid_constant__ FwdArgs a)
 {
     using namespace tc5;
@@ -84,8 +57,8 @@ __global__ void __launch_bounds__(FT, 1) deform_heads_fwd_kernel(const __grid_co
 
     for (int h = 0; h < 2; ++h) {
         if (!on[h]) continue;
-        stage_kmajor(W2h + h * MW * MW, W2l + h * MW * MW, a.w.w2[h], MW, MW, MW);
-        stage_kmajor(W3h + h * 48 * MW, W3l + h * 48 * MW, a.w.w3[h], N3(h), KD(h), MW);
+        stage_kmajor<FT>(W2h + h * MW * MW, W2l + h * MW * MW, a.w.w2[h], MW, MW, MW);
+        stage_kmajor<FT>(W3h + h * 48 * MW, W3l + h * 48 * MW, a.w.w3[h], N3(h), KD(h), MW);
         for (int i = tid; i < MW; i += FT) bias[h * MW + i] = __ldg(a.w.b2[h] + i);
         for (int i = tid; i < KD(h); i += FT) bias[2 * MW + h * 48 + i] = __ldg(a.w.b3[h] + i);
     }
@@ -93,10 +66,7 @@ __global__ void __launch_bounds__(FT, 1) deform_heads_fwd_kernel(const __grid_co
         mbar_init(bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 0) tmem_alloc(tmem_slot, 512);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
     __syncthreads();
@@ -131,7 +101,7 @@ __global__ void __launch_bounds__(FT, 1) deform_heads_fwd_kernel(const __grid_co
         if (issuer()) {
             tc_fence_after();
             for (int h = 0; h < 2; ++h)
-                if (on[h]) issue_split(tbase + C_D2 + 64 * h, tbase, tbase + C_A_LO, smem_u32(W2h + h * MW * MW), smem_u32(W2l + h * MW * MW), MW);
+                if (on[h]) issue_layer(tbase + C_D2 + 64 * h, tbase, tbase + C_A_LO, smem_u32(W2h + h * MW * MW), smem_u32(W2l + h * MW * MW), MW, MW, make_idesc(128, MW));
             tc_commit(bar);
         }
         mbar_wait(bar, phase); phase ^= 1;
@@ -165,8 +135,8 @@ __global__ void __launch_bounds__(FT, 1) deform_heads_fwd_kernel(const __grid_co
         if (issuer()) {
             tc_fence_after();
             for (int h = 0; h < 2; ++h)
-                if (on[h]) issue_split(tbase + c_d3[h], tbase + C_Z + 128 * h, tbase + C_Z + 128 * h + 64,
-                                       smem_u32(W3h + h * 48 * MW), smem_u32(W3l + h * 48 * MW), N3(h));
+                if (on[h]) issue_layer(tbase + c_d3[h], tbase + C_Z + 128 * h, tbase + C_Z + 128 * h + 64,
+                                       smem_u32(W3h + h * 48 * MW), smem_u32(W3l + h * 48 * MW), N3(h), MW, make_idesc(128, N3(h)));
             tc_commit(bar);
         }
         mbar_wait(bar, phase); phase ^= 1;
@@ -206,9 +176,7 @@ __global__ void __launch_bounds__(FT, 1) deform_heads_fwd_kernel(const __grid_co
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tbase), "r"(512u) : "memory");
-    }
+    if (warp == 0) tmem_dealloc(tbase, 512);
 }
 
 constexpr size_t FWD_SMEM = (size_t)(4 * MW * MW + 4 * 48 * MW + 2 * MW + 96) * sizeof(float) + 128;
@@ -219,56 +187,7 @@ constexpr int BT = 256;                   // 8 warps x 16 points
 constexpr int LDS_T = MW + 8;             // row stride of the dz / d_h tile (conflict-free fragment loads)
 constexpr int LDO = 48 + 8;               // row stride of the upstream-gradient tile
 constexpr int RS2 = MW / 2 + 4;           // float4 row stride of a K = 64 operand
-
-__device__ __forceinline__ void split(float x, u32& hi, u32& lo)
-{
-    hi = tc5::to_tf32(x);
-    lo = tc5::to_tf32(x - __uint_as_float(hi));
-}
-__device__ __forceinline__ void mma(float c[4], const u32 a[4], u32 b0, u32 b1)
-{
-    asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-        : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
-// Pre-split operand for Y[rows][n] = sum_k X[rows][k] Wm[k][n], Wm[k][n] = w[k * sk + n]: entry (n, j, t) =
-// {hi Wm[8j+2t][n], hi Wm[8j+2t+1][n], lo, lo} at float4 index n * rs + 4j + t (the k order of an accumulator fragment
-// re-used as an A fragment: slot t <-> column 2t, slot t+4 <-> column 2t+1).
-__device__ __forceinline__ void stage_weight(float4* __restrict__ dst, const float* __restrict__ w, int K, int N, int K_real, int sk, int rs)
-{
-    for (int i = threadIdx.x; i < N * (K / 2); i += BT) {
-        const int n = i / (K / 2), kk = i - n * (K / 2);
-        const int k0 = 2 * kk, k1 = k0 + 1;
-        const float v0 = k0 < K_real ? __ldg(w + (size_t)k0 * sk + n) : 0.f;
-        const float v1 = k1 < K_real ? __ldg(w + (size_t)k1 * sk + n) : 0.f;
-        u32 h0, l0, h1, l1;
-        split(v0, h0, l0); split(v1, h1, l1);
-        dst[n * rs + kk] = make_float4(__uint_as_float(h0), __uint_as_float(h1), __uint_as_float(l0), __uint_as_float(l1));
-    }
-}
-
-// acc[nt] += A (k-step j) * B[:, n-tile nt], the three passes of the split issued pass-major over groups of four n-tiles
-template <int NT>
-__device__ __forceinline__ void kstep(float (*acc)[4], const float a[4], const float4* __restrict__ Bq, int rs, int j, int g, int t)
-{
-    u32 ahi[4], alo[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) split(a[i], ahi[i], alo[i]);
-    constexpr int G = NT < 4 ? NT : 4;
-#pragma unroll
-    for (int n0 = 0; n0 < NT; n0 += G) {
-        float4 b[G];
-#pragma unroll
-        for (int q = 0; q < G; ++q) b[q] = Bq[(8 * (n0 + q) + g) * rs + 4 * j + t];
-#pragma unroll
-        for (int q = 0; q < G; ++q) mma(acc[n0 + q], alo, __float_as_uint(b[q].x), __float_as_uint(b[q].y));
-#pragma unroll
-        for (int q = 0; q < G; ++q) mma(acc[n0 + q], ahi, __float_as_uint(b[q].z), __float_as_uint(b[q].w));
-#pragma unroll
-        for (int q = 0; q < G; ++q) mma(acc[n0 + q], ahi, __float_as_uint(b[q].x), __float_as_uint(b[q].y));
-    }
-}
+using tf32::split; using tf32::mma; using tf32::kstep;
 
 // acc[m][n] (16 out x 8 in) += sum over the tile's rows of dY[row][16 (m0+m) + .] * tf32(X[row][8 (n0+n) + .]);
 // dY from a row-major smem tile (stride lds; out rows >= n_out are zero), X from global memory (stash tiles or row-major).
@@ -339,11 +258,11 @@ __global__ void __launch_bounds__(BT, 1) deform_heads_bwd_kernel(const __grid_co
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
     const bool on[2] = {a.w.w2[0] != nullptr, a.w.w2[1] != nullptr};
 
-    stage_weight(W1b, a.w.w1, MW, F, MW, F, RS2);
+    tf32::stage_weight<BT>(W1b, a.w.w1, MW, F, MW, F, RS2);
     for (int h = 0; h < 2; ++h) {
         if (!on[h]) continue;
-        if (RESIDENT) stage_weight(W2b + h * MW * RS2, a.w.w2[h], MW, MW, MW, MW, RS2);
-        stage_weight(W3b[h], a.w.w3[h], h == 0 ? 8 : 48, MW, KD(h), MW, RS3[h]);
+        if (RESIDENT) tf32::stage_weight<BT>(W2b + h * MW * RS2, a.w.w2[h], MW, MW, MW, MW, RS2);
+        tf32::stage_weight<BT>(W3b[h], a.w.w3[h], h == 0 ? 8 : 48, MW, KD(h), MW, RS3[h]);
     }
     __syncthreads();
 
@@ -380,7 +299,7 @@ __global__ void __launch_bounds__(BT, 1) deform_heads_bwd_kernel(const __grid_co
             const float* zsv = a.saved + (size_t)h * stash_plane_floats(a.P);
             const float4* W2h = W2b + (RESIDENT ? h : 0) * MW * RS2;
             if (!RESIDENT) {                  // every warp is past the previous head's use of the slot (trailing barrier below)
-                stage_weight(W2b, a.w.w2[h], MW, MW, MW, MW, RS2);
+                tf32::stage_weight<BT>(W2b, a.w.w2[h], MW, MW, MW, MW, RS2);
                 __syncthreads();
             }
             // dz = (d_out W3) masked by relu(z) > 0; d_out also goes to the smem tile (dW3, db3) and, for the SH head, into the
@@ -561,9 +480,7 @@ int b200gs_deform_heads_forward(const b200gs_heads_weights* w, long long P, int 
     heads::FwdArgs a;
     a.w = *w; a.P = P; a.hidden = mlp_saved; a.opacity = opacity; a.shs = shs; a.opacity_out = opacity_out;
     a.shs_out = shs_out; a.saved = heads_saved;
-    const long long nblocks = (P + tc5::ROWS - 1) / tc5::ROWS;
-    const int sms = g_opt_mlp_fwd_sms > 0 && g_opt_mlp_fwd_sms < NUM_SMS ? g_opt_mlp_fwd_sms : NUM_SMS;
-    const int grid = (int)(nblocks < sms ? nblocks : sms);
+    const int grid = tc5::persistent_grid(P, g_opt_mlp_fwd_sms);
     cudaFuncSetAttribute(heads::deform_heads_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)heads::FWD_SMEM);
     heads::deform_heads_fwd_kernel<<<grid, heads::FT, heads::FWD_SMEM, (cudaStream_t)stream>>>(a);
     return check_launch("deform_heads_forward");
@@ -590,9 +507,7 @@ int b200gs_deform_heads_backward(const b200gs_heads_weights* w, const b200gs_hea
     a.w = *w; a.gw = *gw; a.P = P; a.feat = features; a.hidden = mlp_saved; a.saved = heads_saved;
     a.d_opacity = d_opacity; a.d_shs = d_shs; a.d_feat = d_features;
     a.sh_grad = w->w2[1] ? sh_grad : nullptr; a.sh_overwrite = sh_grad_overwrite;
-    const long long nblocks = (P + tc5::ROWS - 1) / tc5::ROWS;
-    const int sms = g_opt_mlp_bwd_sms > 0 && g_opt_mlp_bwd_sms < NUM_SMS ? g_opt_mlp_bwd_sms : NUM_SMS;
-    const int grid = (int)(nblocks < sms ? nblocks : sms);
+    const int grid = tc5::persistent_grid(P, g_opt_mlp_bwd_sms);
     const size_t smem = heads::bwd_smem(w->feat_dim);
     if (w->feat_dim == 64) {
         cudaFuncSetAttribute(heads::deform_heads_bwd_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -20,83 +20,19 @@
 // ReLU'd activations the backward needs (4 x 256 B per point, plain row-major) leave the SM.
 // The backward accumulates all weight gradients in register fragments across every tile a
 // persistent CTA processes and flushes them with one atomic per element per CTA.
-#include "tc5_common.cuh"
+#include "mma_tf32.cuh"
 #include "../../include/b200gs.h"
 
 namespace b200gs {
 
 namespace {
 
-constexpr bool USE_TCGEN05_BACKWARD = true;     // F = 64 only; F = 128 keeps the mma.sync kernel below
 using tc5::MW;                     // net_width
-using tc5::stash_off; using tc5::stash_plane_floats;
+using tc5::stash_off; using tc5::stash_plane_floats; using tc5::to_tf32;
+using tf32::split; using tf32::mma; using tf32::kstep; using tf32::stage_weight;
 constexpr int MT = 256;            // threads per CTA (8 warps x 16 points)
 using tc5::ROWS;                   // points per CTA iteration
 constexpr int LDS_T = MW + 8;      // row stride (floats) of the row-major smem tiles: conflict-free fragment loads
-
-__device__ __forceinline__ u32 to_tf32(float x) { u32 r; asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x)); return r; }
-__device__ __forceinline__ void split(float x, u32& hi, u32& lo)
-{
-    hi = to_tf32(x);
-    lo = to_tf32(x - __uint_as_float(hi));
-}
-__device__ __forceinline__ void mma(float c[4], const u32 a[4], u32 b0, u32 b1)
-{
-    asm("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-// c += (ahi + alo) * (bhi + blo) without the lo*lo term, small terms first; b = {hi0, hi1, lo0, lo1}
-__device__ __forceinline__ void mma3(float c[4], const u32 ahi[4], const u32 alo[4], const float4 b)
-{
-    mma(c, alo, __float_as_uint(b.x), __float_as_uint(b.y));
-    mma(c, ahi, __float_as_uint(b.z), __float_as_uint(b.w));
-    mma(c, ahi, __float_as_uint(b.x), __float_as_uint(b.y));
-}
-
-// Pre-split weight operand for  Y[rows][n] = sum_k X[rows][k] * Wm[k][n]:
-// entry (n, j, t) = {hi Wm[8j+2t][n], hi Wm[8j+2t+1][n], lo ..., lo ...}, float4 index n*rs + 4j + t,
-// rs = K/2 + 4 (== 4 mod 8 -> the 8 lanes of an LDS.128 phase hit disjoint banks).
-// `w` holds element Wm[k][n] at w[k*sk + n*sn]; K_real / N_real bound the non-zero part.
-__device__ __forceinline__ void stage_weight(float4* __restrict__ dst, const float* __restrict__ w, int K, int N,
-                                             int K_real, int N_real, int sk, int sn)
-{
-    const int rs = K / 2 + 4;
-    for (int i = threadIdx.x; i < N * (K / 2); i += MT) {
-        const int n = i / (K / 2), kk = i - n * (K / 2);      // kk = 4j + t
-        const int k0 = 2 * kk, k1 = k0 + 1;
-        const float v0 = (n < N_real && k0 < K_real) ? __ldg(w + (size_t)k0 * sk + (size_t)n * sn) : 0.f;
-        const float v1 = (n < N_real && k1 < K_real) ? __ldg(w + (size_t)k1 * sk + (size_t)n * sn) : 0.f;
-        u32 h0, l0, h1, l1;
-        split(v0, h0, l0); split(v1, h1, l1);
-        dst[n * rs + kk] = make_float4(__uint_as_float(h0), __uint_as_float(h1), __uint_as_float(l0), __uint_as_float(l1));
-    }
-}
-
-// acc[nt] += A(k-step j) * B[:, n-tile nt]  for nt in [0, NT); A given as its 4 fragment values.
-// The three passes of the split are issued pass-major over groups of four n-tiles, so that back-to-back
-// MMAs never depend on each other (a dependent HMMA would wait out the full pipe latency).
-template <int NT>
-__device__ __forceinline__ void kstep(float (*acc)[4], const float a[4], const float4* __restrict__ Bq, int rs, int j,
-                                      int g, int t)
-{
-    u32 ahi[4], alo[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) split(a[i], ahi[i], alo[i]);
-    constexpr int G = NT < 4 ? NT : 4;
-#pragma unroll
-    for (int n0 = 0; n0 < NT; n0 += G) {
-        float4 b[G];
-#pragma unroll
-        for (int q = 0; q < G; ++q) b[q] = Bq[(8 * (n0 + q) + g) * rs + 4 * j + t];
-#pragma unroll
-        for (int q = 0; q < G; ++q) mma(acc[n0 + q], alo, __float_as_uint(b[q].x), __float_as_uint(b[q].y));
-#pragma unroll
-        for (int q = 0; q < G; ++q) mma(acc[n0 + q], ahi, __float_as_uint(b[q].z), __float_as_uint(b[q].w));
-#pragma unroll
-        for (int q = 0; q < G; ++q) mma(acc[n0 + q], ahi, __float_as_uint(b[q].x), __float_as_uint(b[q].y));
-    }
-}
 
 // ---------------------------------------------------------------------------------------------
 struct BwdArgs {
@@ -144,27 +80,25 @@ __device__ __forceinline__ void dw_accumulate(float (*acc)[4], const float* __re
     }
 }
 
-template <int F>
+template <int F>      // F = 128 (feature dim 64 runs the tcgen05 backward)
 __global__ void __launch_bounds__(MT, 1) deform_mlp_bwd_kernel(const __grid_constant__ BwdArgs a)
 {
     extern __shared__ __align__(16) float4 smem4[];
     constexpr int RS2 = MW / 2 + 4;            // K = 64 operands
     constexpr int RS3 = 4;                     // K = 8 operand (W3): 4 float4 per row, contiguous -> conflict-free
-    constexpr bool RESIDENT = (F == 64);       // F = 128: one W2 slot, re-staged per head (shared memory budget)
     constexpr int NT1 = F / 8;                 // n-tiles of d_feature / in-features of W1
     float4* W3b = smem4;                       // [3][64][RS3]   Wm[k=out(pad 8)][n=in 64]  = W3[k][n]
-    float4* W2b = W3b + 3 * MW * RS3;          // [3][64][RS2]   Wm[k=out][n=in]            = W2[k][n]
-    float4* W1b = W2b + (RESIDENT ? 3 : 1) * MW * RS2;   // [F][RS2]  Wm[k=out 64][n=in F]       = W1[k][n]
+    float4* W2b = W3b + 3 * MW * RS3;          // [64][RS2]      Wm[k=out][n=in]            = W2[k][n], one slot re-staged per head
+    float4* W1b = W2b + MW * RS2;              // [F][RS2]       Wm[k=out 64][n=in F]       = W1[k][n]
     float* Ds = reinterpret_cast<float*>(W1b + F * RS2);          // [ROWS][LDS_T]  dz / d hidden, row-major
     float* Dout = Ds + ROWS * LDS_T;                              // [ROWS][8]      upstream gradient of the head
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, t = lane & 3;
     const int kdim[3] = {3, 3, 4};
 
-    // backward dX = dY W: Wm[k][n] = W_torch[k][n] -> sk = row length, sn = 1
-    stage_weight(W1b, a.w.w1, MW, F, MW, F, F, 1);
+    // backward dX = dY W: Wm[k][n] = W_torch[k][n] -> sk = row length
+    stage_weight<MT>(W1b, a.w.w1, MW, F, MW, F, RS2);
     for (int h = 0; h < 3; ++h) {
         if (!a.w.w2[h]) continue;
-        if (RESIDENT) stage_weight(W2b + h * MW * RS2, a.w.w2[h], MW, MW, MW, MW, MW, 1);
         for (int i = tid; i < MW * 4; i += MT) {                     // K = 8 (padded outputs), rs = 4
             const int n = i >> 2, kk = i & 3, k0 = 2 * kk, k1 = k0 + 1;
             const float v0 = k0 < kdim[h] ? __ldg(a.w.w3[h] + k0 * MW + n) : 0.f;
@@ -216,11 +150,9 @@ __global__ void __launch_bounds__(MT, 1) deform_mlp_bwd_kernel(const __grid_cons
             const int kd = kdim[h];
             const float* dsrc = h == 0 ? a.d_pts : (h == 1 ? a.d_scales : a.d_rot);
             const float* zsv = a.saved + (size_t)(1 + h) * stash_plane_floats(a.P);
-            const float4* W2h = W2b + (RESIDENT ? h : 0) * MW * RS2;
-            if (!RESIDENT) {            // every warp is past the previous head's use of the slot (trailing barrier below)
-                stage_weight(W2b, a.w.w2[h], MW, MW, MW, MW, MW, 1);
-                __syncthreads();
-            }
+            // every warp is past the previous head's use of the slot (trailing barrier below)
+            stage_weight<MT>(W2b, a.w.w2[h], MW, MW, MW, MW, RS2);
+            __syncthreads();
             // upstream gradient as an A fragment (one k-step, columns >= kd are zero) and as a smem tile
             float df[4];
             {
@@ -252,7 +184,7 @@ __global__ void __launch_bounds__(MT, 1) deform_mlp_bwd_kernel(const __grid_cons
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 const float af[4] = {dz[j][0], dz[j][2], dz[j][1], dz[j][3]};
-                kstep<8>(dRh, af, W2h, RS2, j, g, t);
+                kstep<8>(dRh, af, W2b, RS2, j, g, t);
             }
             __syncthreads();                                             // dz and d_out tiles complete
             dw_accumulate<4, true>(gW2[h], Ds, mt, a.saved, MW, row0, a.P, ntb, g, t);            // dW2 += dz^T relu(h)
@@ -347,11 +279,8 @@ __global__ void __launch_bounds__(MT, 1) deform_mlp_bwd_kernel(const __grid_cons
     }
 }
 
-size_t bwd_smem(int F)
-{
-    return (size_t)(3 * MW * 4 + (F == 64 ? 3 : 1) * MW * (MW / 2 + 4) + F * (MW / 2 + 4)) * sizeof(float4) +
-           (size_t)(ROWS * LDS_T + ROWS * 8) * sizeof(float);
-}
+constexpr size_t BWD_SMEM = (size_t)(3 * MW * 4 + MW * (MW / 2 + 4) + 128 * (MW / 2 + 4)) * sizeof(float4) +
+                            (size_t)(ROWS * LDS_T + ROWS * 8) * sizeof(float);
 
 int check_weights(const b200gs_mlp_weights* w)
 {
@@ -402,21 +331,14 @@ int b200gs_deform_mlp_backward(const b200gs_mlp_weights* w, const b200gs_mlp_gra
     if (check_weights(w)) return -1;
     if (!gw) { set_error("deform_mlp_backward: null gradient table"); return -1; }
     if (P <= 0) return 0;
-    if (USE_TCGEN05_BACKWARD && w->feat_dim == 64)
+    if (w->feat_dim == 64)
         return deform_mlp_backward_tc5(w, gw, P, feat, saved, d_pts, d_scales, d_rot, d_feat, (cudaStream_t)stream);
     BwdArgs a;
     a.w = *w; a.gw = *gw; a.P = P; a.feat = feat; a.saved = saved; a.d_pts = d_pts; a.d_scales = d_scales;
     a.d_rot = d_rot; a.d_feat = d_feat;
-    const long long nblocks = (P + ROWS - 1) / ROWS;
-    const int grid = (int)(nblocks < NUM_SMS ? nblocks : NUM_SMS);
-    const size_t smem = bwd_smem(w->feat_dim);
-    if (w->feat_dim == 64) {
-        cudaFuncSetAttribute(deform_mlp_bwd_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        deform_mlp_bwd_kernel<64><<<grid, MT, smem, (cudaStream_t)stream>>>(a);
-    } else {
-        cudaFuncSetAttribute(deform_mlp_bwd_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        deform_mlp_bwd_kernel<128><<<grid, MT, smem, (cudaStream_t)stream>>>(a);
-    }
+    const int grid = tc5::persistent_grid(P, 0);       // no CTA cap: this kernel does not take mlp_bwd_sms
+    cudaFuncSetAttribute(deform_mlp_bwd_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)BWD_SMEM);
+    deform_mlp_bwd_kernel<128><<<grid, MT, BWD_SMEM, (cudaStream_t)stream>>>(a);
     return check_launch("deform_mlp_backward");
 }
 

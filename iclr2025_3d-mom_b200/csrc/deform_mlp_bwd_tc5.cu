@@ -122,10 +122,7 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
         if constexpr (TMA) { mbar_init(bar + 1, 1); mbar_init(bar + 2, 1); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 0) tmem_alloc(tmem_slot, 512);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
     __syncthreads();
@@ -499,9 +496,7 @@ __global__ void __launch_bounds__(BT, 1) deform_mlp_bwd_tc5_kernel(const __grid_
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tbase), "r"(512u) : "memory");
-    }
+    if (warp == 0) tmem_dealloc(tbase, 512);
 }
 
 size_t bwd_smem() { return (size_t)(2 * MW * MW + 2 * MW * MW) * 4 + 98304 + 2 * KPLANE + 64; }
@@ -519,9 +514,7 @@ int deform_mlp_backward_tc5(const b200gs_mlp_weights* w, const b200gs_mlp_grads*
     tc5::BwdArgs a;
     a.w = *w; a.gw = *gw; a.P = P; a.feat = feat; a.saved = saved; a.d_pts = d_pts; a.d_scales = d_scales; a.d_rot = d_rot;
     a.d_feat = d_feat; a.dy_sbo = 512u;
-    const long long nblocks = (P + tc5::ROWS - 1) / tc5::ROWS;
-    const int sms = g_opt_mlp_bwd_sms > 0 && g_opt_mlp_bwd_sms < NUM_SMS ? g_opt_mlp_bwd_sms : NUM_SMS;          // option: leave a few SMs to a concurrent stream
-    const int grid = (int)(nblocks < sms ? nblocks : sms);
+    const int grid = tc5::persistent_grid(P, g_opt_mlp_bwd_sms);
     const size_t smem = tc5::bwd_smem();
     // the TMA staging needs the tiled feature layout (one contiguous 32 KB tile per phase)
     void (*kern)(tc5::BwdArgs) = w->feat_tiled ? tc5::deform_mlp_bwd_tc5_kernel<true> : tc5::deform_mlp_bwd_tc5_kernel<false>;

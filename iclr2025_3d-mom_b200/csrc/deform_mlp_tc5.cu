@@ -23,32 +23,6 @@ namespace tc5 {
 
 constexpr int NT = 128;            // threads per CTA
 
-// weights: torch [N_real x K] row-major -> hi / lo K-major UMMA operands with N rows (zero padded)
-__device__ __forceinline__ void stage_kmajor(float* __restrict__ hi, float* __restrict__ lo, const float* __restrict__ w,
-                                             int N, int N_real, int K)
-{
-    for (int i = threadIdx.x; i < N * K; i += NT) {
-        const int n = i / K, k = i - n * K;
-        const float v = n < N_real ? __ldg(w + (size_t)n * K + k) : 0.f;
-        const u32 h = to_tf32(v), l = to_tf32(v - __uint_as_float(h));
-        const int off = (k >> 2) * (N * 4) + n * 4 + (k & 3);
-        hi[off] = __uint_as_float(h);
-        lo[off] = __uint_as_float(l);
-    }
-}
-
-// 3 x (K/8) MMAs: D = (Ahi + Alo) (Bhi + Blo) without lo*lo, small terms first
-__device__ __forceinline__ void issue_layer(u32 d_tmem, u32 a_hi, u32 a_lo, u32 b_hi_smem, u32 b_lo_smem, int N, int K, u32 idesc)
-{
-    const u64 dh = kmajor_desc(b_hi_smem, N), dl = kmajor_desc(b_lo_smem, N);
-    const u64 step = (u64)((2 * N * 16) >> 4);         // two 16-byte K chunks per instruction
-    for (int j = 0; j < K / 8; ++j) {
-        mma_ts(d_tmem, a_lo + 8 * j, dh + step * j, idesc, j > 0);
-        mma_ts(d_tmem, a_hi + 8 * j, dl + step * j, idesc, 1u);
-        mma_ts(d_tmem, a_hi + 8 * j, dh + step * j, idesc, 1u);
-    }
-}
-
 struct FwdArgs {
     b200gs_mlp_weights w;
     long long P;
@@ -75,12 +49,12 @@ __global__ void __launch_bounds__(NT, 1) deform_mlp_fwd_tc5_kernel(const __grid_
     const int tid = threadIdx.x, warp = tid >> 5;
     const int kdim[3] = {3, 3, 4};
 
-    stage_kmajor(W1h, W1l, a.w.w1, MW, MW, F);
+    stage_kmajor<NT>(W1h, W1l, a.w.w1, MW, MW, F);
     for (int i = tid; i < MW; i += NT) bias[i] = __ldg(a.w.b1 + i);
     for (int h = 0; h < 3; ++h) {
         if (!a.w.w2[h]) continue;
-        stage_kmajor(W2h + h * MW * MW, W2l + h * MW * MW, a.w.w2[h], MW, MW, MW);
-        stage_kmajor(W3h + h * 16 * MW, W3l + h * 16 * MW, a.w.w3[h], 16, kdim[h], MW);
+        stage_kmajor<NT>(W2h + h * MW * MW, W2l + h * MW * MW, a.w.w2[h], MW, MW, MW);
+        stage_kmajor<NT>(W3h + h * 16 * MW, W3l + h * 16 * MW, a.w.w3[h], 16, kdim[h], MW);
         for (int i = tid; i < MW; i += NT) bias[MW + h * MW + i] = __ldg(a.w.b2[h] + i);
         if (tid < 16) bias[4 * MW + h * 16 + tid] = tid < kdim[h] ? __ldg(a.w.b3[h] + tid) : 0.f;
     }
@@ -94,10 +68,7 @@ __global__ void __launch_bounds__(NT, 1) deform_mlp_fwd_tc5_kernel(const __grid_
         mbar_init(bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 0) tmem_alloc(tmem_slot, 512);
     // make the generic-proxy weight writes visible to the tensor-core (async) proxy
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
@@ -243,9 +214,7 @@ __global__ void __launch_bounds__(NT, 1) deform_mlp_fwd_tc5_kernel(const __grid_
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tbase), "r"(512u) : "memory");
-    }
+    if (warp == 0) tmem_dealloc(tbase, 512);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -263,19 +232,6 @@ __global__ void __launch_bounds__(NT, 1) deform_mlp_fwd_tc5_kernel(const __grid_
 // (F = 128: the feature lo half overlaps Z, it is dead once layer 1 has completed); D2 [256,448) the three
 // heads' accumulators (layer 1 accumulates into the first 64 of them); D3 [448,496) the head outputs.
 constexpr int NT2 = 256;
-
-__device__ __forceinline__ void stage_kmajor2(float* __restrict__ hi, float* __restrict__ lo, const float* __restrict__ w,
-                                              int N, int N_real, int K)
-{
-    for (int i = threadIdx.x; i < N * K; i += NT2) {
-        const int n = i / K, k = i - n * K;
-        const float v = n < N_real ? __ldg(w + (size_t)n * K + k) : 0.f;
-        const u32 h = to_tf32(v), l = to_tf32(v - __uint_as_float(h));
-        const int off = (k >> 2) * (N * 4) + n * 4 + (k & 3);
-        hi[off] = __uint_as_float(h);
-        lo[off] = __uint_as_float(l);
-    }
-}
 
 // The MMAs are issued from a warp-uniform branch by the elected lane of warp 0 (tc5_common.cuh elect_one): `if (tid == 0)`
 // makes the compiler wrap every tcgen05.mma in an ELECT / BRA.U.ANY loop.  The activation-stash stores of a layer are issued
@@ -299,11 +255,11 @@ __global__ void __launch_bounds__(NT2, 1) deform_mlp_fwd_tc5v2_kernel(const __gr
     const int pT = (warp & 3) * 32 + lane, cT = warp >> 2;
     const int kdim[3] = {3, 3, 4};
 
-    stage_kmajor2(W1h, W1l, a.w.w1, MW, MW, F);
+    stage_kmajor<NT2>(W1h, W1l, a.w.w1, MW, MW, F);
     for (int i = tid; i < MW; i += NT2) bias[i] = __ldg(a.w.b1 + i);
     for (int h = 0; h < 3; ++h) {
-        stage_kmajor2(W2h + h * MW * MW, W2l + h * MW * MW, a.w.w2[h], MW, MW, MW);
-        stage_kmajor2(W3h + h * 16 * MW, W3l + h * 16 * MW, a.w.w3[h], 16, kdim[h], MW);
+        stage_kmajor<NT2>(W2h + h * MW * MW, W2l + h * MW * MW, a.w.w2[h], MW, MW, MW);
+        stage_kmajor<NT2>(W3h + h * 16 * MW, W3l + h * 16 * MW, a.w.w3[h], 16, kdim[h], MW);
         for (int i = tid; i < MW; i += NT2) bias[MW + h * MW + i] = __ldg(a.w.b2[h] + i);
         if (tid < 16) bias[4 * MW + h * 16 + tid] = tid < kdim[h] ? __ldg(a.w.b3[h] + tid) : 0.f;
     }
@@ -318,10 +274,7 @@ __global__ void __launch_bounds__(NT2, 1) deform_mlp_fwd_tc5v2_kernel(const __gr
         for (int i = 0; i < 7; ++i) mbar_init(bars + i, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 0) tmem_alloc(tmem_slot, 512);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
     __syncthreads();
@@ -482,9 +435,7 @@ __global__ void __launch_bounds__(NT2, 1) deform_mlp_fwd_tc5v2_kernel(const __gr
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tbase), "r"(512u) : "memory");
-    }
+    if (warp == 0) tmem_dealloc(tbase, 512);
 }
 
 size_t fwd_smem(int F) { return (size_t)(2 * MW * F + 6 * MW * MW + 6 * 16 * MW + 4 * MW + 48) * sizeof(float) + 128; }
@@ -500,9 +451,7 @@ int deform_mlp_forward_tc5(const b200gs_mlp_weights* w, long long P, const float
     a.w = *w; a.P = P; a.feat = feat; a.xyz = xyz; a.scales = scales; a.rot = rot; a.scene_flow = scene_flow;
     a.frame_num = frame_num; a.frame_num_dev = frame_num_dev; a.delta_scale = delta_scale; a.pts_out = pts_out;
     a.scales_out = scales_out; a.rot_out = rot_out; a.saved = saved;
-    const long long nblocks = (P + tc5::ROWS - 1) / tc5::ROWS;
-    const int sms = g_opt_mlp_fwd_sms > 0 && g_opt_mlp_fwd_sms < NUM_SMS ? g_opt_mlp_fwd_sms : NUM_SMS;          // option: leave a few SMs to a concurrent stream
-    const int grid = (int)(nblocks < sms ? nblocks : sms);
+    const int grid = tc5::persistent_grid(P, g_opt_mlp_fwd_sms);
     const size_t smem = tc5::fwd_smem(w->feat_dim);
     if (!saved && !(w->w2[0] && w->w2[1] && w->w2[2])) {
         set_error("deform_mlp_forward: saved == NULL (inference, nothing stashed) needs all three heads enabled");

@@ -8,6 +8,14 @@ namespace tc5 {
 constexpr int MW = 64;
 constexpr int ROWS = 128;
 
+__device__ __forceinline__ u32 smem_u32(const void* p) { return (u32)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ u32 to_tf32(float x) { u32 r; asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x)); return r; }
+// Exact two-term split for tcgen05.mma.kind::tf32. The tensor core TRUNCATES an FP32 container to TF32 (it ignores the low
+// 13 mantissa bits; measured with tools/probe/umma_probe.cu), so the "hi" operand can be the raw value itself and
+// lo = x - trunc(x) is exact (13 significant bits, of which the hardware keeps 10): hi + lo reproduces x to 2^-21 relative
+// with two instructions instead of the five of a round / subtract / round split.
+__device__ __forceinline__ float tf32_lo(float x) { return x - __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
+
 // Activation stash layout (forward -> backward, opaque to callers): 4 planes (relu(hidden), relu(z_pos),
 // relu(z_scale), relu(z_rot)) of ceil(P/128) tiles; a tile is [32 groups of 4 points][16 column chunks][4 points]
 // [4 floats].  The backward reads 8 chunks x 4 points per warp instruction = one contiguous 512-byte run; the
@@ -18,6 +26,15 @@ __host__ __device__ __forceinline__ size_t stash_off(long long row, int col)
     return (size_t)(row >> 7) * (ROWS * MW) + (size_t)((row & 127) >> 2) * 256 + (size_t)(col >> 2) * 16 + (size_t)(row & 3) * 4 + (col & 3);
 }
 
+// Grid of a persistent kernel walking the ceil(P/128) tiles: one CTA per SM, at most `cap` when 0 < cap < NUM_SMS (the
+// b200gs_set_option CTA caps, which leave SMs to a concurrent stream), never more CTAs than tiles.
+inline int persistent_grid(long long P, int cap)
+{
+    const long long nblocks = (P + ROWS - 1) / ROWS;
+    const int sms = cap > 0 && cap < NUM_SMS ? cap : NUM_SMS;
+    return (int)(nblocks < sms ? nblocks : sms);
+}
+
 // Behind the four stash planes the forward leaves, for the tcgen05 backward (feature dim 64), the transposed weights as
 // ready-to-copy K-major UMMA B operands [N = in][K = out] in TF32 hi / lo pairs: W2^T of the three heads, then W1^T
 // (8 images of 64 x 64 floats). The backward streams the current head's pair into shared memory with cp.async instead
@@ -25,7 +42,6 @@ __host__ __device__ __forceinline__ size_t stash_off(long long row, int col)
 // three-term split (a rounded weight operand left up to 2 % error on a few per-point xyz gradients at 1M points).
 constexpr size_t BWD_W_IMAGE_FLOATS = 8 * MW * MW;
 __host__ __device__ __forceinline__ size_t stash_total_floats(long long P) { return 4 * stash_plane_floats(P) + BWD_W_IMAGE_FLOATS; }
-__device__ __forceinline__ u32 to_tf32(float x);
 // image m (0..2: W2 of head m, 3: W1), plane 0 = hi, 1 = lo; w = torch [out 64][in 64] row-major
 __device__ __forceinline__ void write_bwd_weight_image(float* __restrict__ images, int m, const float* __restrict__ w, int nthreads)
 {
@@ -40,14 +56,6 @@ __device__ __forceinline__ void write_bwd_weight_image(float* __restrict__ image
         lo[off] = __uint_as_float(to_tf32(v - h));
     }
 }
-
-__device__ __forceinline__ u32 smem_u32(const void* p) { return (u32)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ u32 to_tf32(float x) { u32 r; asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x)); return r; }
-// Exact two-term split for tcgen05.mma.kind::tf32. The tensor core TRUNCATES an FP32 container to TF32 (it ignores the low
-// 13 mantissa bits; measured with tools/probe/umma_probe.cu), so the "hi" operand can be the raw value itself and
-// lo = x - trunc(x) is exact (13 significant bits, of which the hardware keeps 10): hi + lo reproduces x to 2^-21 relative
-// with two instructions instead of the five of a round / subtract / round split.
-__device__ __forceinline__ float tf32_lo(float x) { return x - __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
 
 __device__ __forceinline__ void mbar_init(u64* bar, u32 count)
 {
@@ -119,6 +127,17 @@ __device__ __forceinline__ void tmem_st32(u32 addr, const u32* v)
     asm volatile("tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};"
                  :: "r"(addr), W8(v, 0), W8(v, 8), W8(v, 16), W8(v, 24) : "memory");
 }
+// Warp-collective: `cols` TMEM columns, base address written to *slot; the allocation permit is given up at once so that
+// the CTA never blocks another one's allocation on the same SM.  Freed by tmem_dealloc from one warp before the CTA exits.
+__device__ __forceinline__ void tmem_alloc(u32* slot, u32 cols)
+{
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(slot)), "r"(cols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc(u32 base, u32 cols)
+{
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(base), "r"(cols) : "memory");
+}
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
@@ -140,6 +159,33 @@ __device__ __forceinline__ u64 smem_desc(u32 smem_addr, u32 lbo_bytes, u32 sbo_b
     return (u64)((smem_addr >> 4) & 0x3FFF) | ((u64)(lbo_bytes >> 4) << 16) | ((u64)(sbo_bytes >> 4) << 32) | (1ull << 46);
 }
 constexpr u32 IDESC_A_MN = 1u << 15, IDESC_B_MN = 1u << 16;
+
+// weights: torch [N_real x K] row-major -> hi / lo K-major UMMA operands with N rows (zero padded), by a block of NTHREADS
+template <int NTHREADS>
+__device__ __forceinline__ void stage_kmajor(float* __restrict__ hi, float* __restrict__ lo, const float* __restrict__ w,
+                                             int N, int N_real, int K)
+{
+    for (int i = threadIdx.x; i < N * K; i += NTHREADS) {
+        const int n = i / K, k = i - n * K;
+        const float v = n < N_real ? __ldg(w + (size_t)n * K + k) : 0.f;
+        const u32 h = to_tf32(v), l = to_tf32(v - __uint_as_float(h));
+        const int off = (k >> 2) * (N * 4) + n * 4 + (k & 3);
+        hi[off] = __uint_as_float(h);
+        lo[off] = __uint_as_float(l);
+    }
+}
+
+// 3 x (K/8) MMAs: D = (Ahi + Alo) (Bhi + Blo) without lo*lo, small terms first
+__device__ __forceinline__ void issue_layer(u32 d_tmem, u32 a_hi, u32 a_lo, u32 b_hi_smem, u32 b_lo_smem, int N, int K, u32 idesc)
+{
+    const u64 dh = kmajor_desc(b_hi_smem, N), dl = kmajor_desc(b_lo_smem, N);
+    const u64 step = (u64)((2 * N * 16) >> 4);         // two 16-byte K chunks per instruction
+    for (int j = 0; j < K / 8; ++j) {
+        mma_ts(d_tmem, a_lo + 8 * j, dh + step * j, idesc, j > 0);
+        mma_ts(d_tmem, a_hi + 8 * j, dl + step * j, idesc, 1u);
+        mma_ts(d_tmem, a_hi + 8 * j, dh + step * j, idesc, 1u);
+    }
+}
 
 }  // namespace tc5
 }  // namespace b200gs
