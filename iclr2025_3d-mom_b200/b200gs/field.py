@@ -9,12 +9,14 @@ libb200gs (csrc/hexplane.cu, csrc/deform_mlp*.cu and, with `no_do` / `no_dshs` F
 opacity and SH heads) through `torch.autograd.Function`s.
 
 Differences that do not change results:
-  * plane parameters keep their [1, 32, H, W] shape but use torch.channels_last strides (one
-    coalesced 128-byte line per texel in the kernels);
+  * plane parameters keep their [1, C, H, W] shape (C = 16 or 32) but use torch.channels_last strides
+    (one coalesced line of C floats per texel in the kernels);
   * the sin/cos positional encodings the reference computes and then slices away
     (deformation.py:205-207 vs :107-135) are not computed.
 Configurations the reference can express but does not train with are rejected loudly
-(NotImplementedError) instead of silently falling back to PyTorch operators.
+(NotImplementedError) instead of silently falling back to PyTorch operators.  `HexPlaneField` takes 16 or 32 channels at
+1-4 levels; `Deformation` (the fused MLP) needs 32 channels at 2 or 4 levels.  `HexPlaneField` alone can therefore serve
+as the grid of the reference's own `scene.deformation.Deformation` (b200gs.launcher.patch_hexplane).
 """
 import contextlib
 import ctypes
@@ -97,7 +99,11 @@ def _cell_order(pts, aabb):
     """Cell-sorted visiting order of the query points (a locality HINT for the sampling kernels: any permutation gives the
     same results).  Cached per device on the storage: within one training iteration every view and the backward pass query
     the same positions, and across iterations the Gaussians move by a small fraction of a cell, so the order is re-sorted
-    only every ORDER_MAX_AGE parameter updates (FusedAdam bumps `_version` per step) or when the tensor / aabb changes."""
+    only every ORDER_MAX_AGE parameter updates (FusedAdam bumps `_version` per step) or when the tensor / aabb changes.
+    The entry holds the tensor it was sorted for: while it lives, its memory cannot be handed to a different tensor, so an
+    address match always means the same points.  A per-call copy (the `pts.contiguous()` of the [:, :3] slice the reference's
+    Deformation passes) is therefore sorted on every call; a freed copy's recycled address, at version 0, must not pass for
+    the same points."""
     P = int(pts.shape[0])
     if P < ORDER_MIN_POINTS:
         return None
@@ -111,7 +117,8 @@ def _cell_order(pts, aabb):
     scratch = torch.empty((nbytes,), dtype=torch.uint8, device=pts.device)
     check(L.b200gs_hexplane_order(P, pts.data_ptr(), aabb.data_ptr(), order.data_ptr(), scratch.data_ptr(), nbytes,
                                   current_stream()), "hexplane_order")
-    _ORDER_CACHE[pts.device] = (key, order, pts._version)
+    _lib.COUNTERS["cell_order_sorts"] += 1
+    _ORDER_CACHE[pts.device] = (key, order, pts._version, pts)
     return order
 
 
@@ -214,7 +221,7 @@ class _HexPlaneFn(torch.autograd.Function):
         _check_cuda_f32(pts, aabb, *planes)
         P = int(pts.shape[0])
         tt, ts = _times_arg(times, P)
-        feat = torch.empty((P, 32 * levels), dtype=torch.float32, device=pts.device)
+        feat = torch.empty((P, int(planes[0].shape[1]) * levels), dtype=torch.float32, device=pts.device)
         d = _hex_desc(aabb, planes, levels, res)
         order = _cell_order(pts, aabb)
         check(_lib.lib().b200gs_hexplane_forward(ctypes.byref(d), P, pts.data_ptr(), _optr(order),
@@ -235,6 +242,15 @@ class _HexPlaneFn(torch.autograd.Function):
         d_pts = torch.empty_like(pts) if ctx.needs_input_grad[0] else None
         d = _hex_desc(aabb, planes, levels, res, grads)
         d_feat = d_feat.contiguous()          # kept alive in this frame until the launch has been queued
+        if d.channels == 16 and not has_t:
+            # One timestamp for the whole call (the reference's render() passes the camera's one time): every point adds into
+            # the same two rows of each time plane, so their gradient is reduced through replicated 1-D rows first.
+            scratch, nbytes = _time_row_scratch(d, pts.device)
+            check(_lib.lib().b200gs_hexplane_backward_masked(ctypes.byref(d), P, pts.data_ptr(), _optr(ctx.order), None, ts, MASK_ALL,
+                                                             None, None, d_feat.data_ptr(),
+                                                             d_pts.data_ptr() if d_pts is not None else None, scratch.data_ptr(),
+                                                             nbytes, current_stream()), "hexplane_backward")
+            return (d_pts, None, None, None, None, *grads)
         check(_lib.lib().b200gs_hexplane_backward(ctypes.byref(d), P, pts.data_ptr(), _optr(ctx.order),
                                                   tt.data_ptr() if has_t else None, ts, d_feat.data_ptr(),
                                                   d_pts.data_ptr() if d_pts is not None else None, current_stream()),
@@ -766,12 +782,10 @@ class HexPlaneField(nn.Module):
         self.multiscale_res_multipliers = multires
         self.concat_features = True
         cfg0 = self.grid_config[0]
-        if cfg0["grid_dimensions"] != 2 or cfg0["input_coordinate_dim"] != 4:
-            raise NotImplementedError("b200gs HexPlaneField supports 2-D planes over (x, y, z, t) only")
-        if cfg0["output_coordinate_dim"] != 32:
-            raise NotImplementedError("b200gs HexPlaneField supports 32 channels per plane")
-        if len(multires) not in (2, 4):
-            raise NotImplementedError("b200gs HexPlaneField is built for 2 or 4 resolution levels")
+        if not HexPlaneField.supports(planeconfig, multires):
+            raise NotImplementedError("b200gs HexPlaneField supports 2-D planes over (x, y, z, t) with 16 or 32 channels at "
+                                      f"1-{MAX_LEVELS} levels (got {cfg0['grid_dimensions']}-D over {cfg0['input_coordinate_dim']} "
+                                      f"coordinates, {cfg0['output_coordinate_dim']} channels, {len(multires)} levels)")
         self.grids = nn.ModuleList()
         self.feat_dim = 0
         self._res = []
@@ -784,6 +798,13 @@ class HexPlaneField(nn.Module):
             self.grids.append(gp)
             self._res.append(tuple(int(r) for r in config["resolution"]))
         print("feature_dim:", self.feat_dim)
+
+    @staticmethod
+    def supports(planeconfig, multires):
+        """Whether the kernels cover this (kplanes_config, multires): 2-D planes over (x, y, z, t), 16 or 32 channels,
+        1-4 levels."""
+        return (planeconfig["grid_dimensions"] == 2 and planeconfig["input_coordinate_dim"] == 4
+                and planeconfig["output_coordinate_dim"] in (16, 32) and 1 <= len(multires) <= MAX_LEVELS)
 
     @property
     def get_aabb(self):
@@ -834,6 +855,11 @@ class Deformation(nn.Module):
         self.skips = skips
         self.grid_pe = grid_pe
         self.no_grid = args.no_grid
+        # the MLP kernels take a 64- or 128-wide feature row: 32 channels at 2 or 4 levels (checked before the grid consumes
+        # any random numbers)
+        if args.kplanes_config["output_coordinate_dim"] != 32 or len(args.multires) not in (2, 4):
+            raise NotImplementedError("b200gs Deformation: the fused MLP needs 32 channels per plane at 2 or 4 levels (got "
+                                      f"{args.kplanes_config['output_coordinate_dim']} channels, {len(args.multires)} levels)")
         self.grid = HexPlaneField(args.bounds, args.kplanes_config, args.multires)
         self.args = args
         unsupported = []

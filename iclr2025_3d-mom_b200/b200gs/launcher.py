@@ -8,10 +8,11 @@ reference's compiled extensions, (2) appends import shims for third-party module
 (compat/, SURVEY.md Appendix E), (3) swaps `deform_network` for the fused-kernel module where
 `GaussianModel` looks it up (scene/gaussian_model.py:21,53), (4) makes `training_setup` build the fused
 multi-tensor Adam from the very param groups the reference assembles (gaussian_model.py:197-209), and
-(5) installs the one-launch prune / cat bookkeeping (gaussian_model.py:424-482) and (6) routes
-`compute_regulation` (gaussian_model.py:768-769) to the fused plane-regulariser kernel, and (7) routes
-`utils.loss_utils.ssim` (the opt.lambda_dssim term) to the fused SSIM kernels (patch_loss_utils). The reference tree is
-never modified.
+(5) installs the one-launch prune / cat bookkeeping (gaussian_model.py:424-482), (6) routes
+`compute_regulation` (gaussian_model.py:768-769) to the fused plane-regulariser kernel, (7) routes
+`utils.loss_utils.ssim` (the opt.lambda_dssim term) to the fused SSIM kernels (patch_loss_utils), and (8) gives the
+reference's own `Deformation` -- built for the configurations (3) leaves to it -- our `HexPlaneField` as its grid
+(patch_hexplane), so only its MLP stays in PyTorch. The reference tree is never modified.
 """
 import os
 import runpy
@@ -84,6 +85,28 @@ def patch_loss_utils(module):
     return module
 
 
+def patch_hexplane(module):
+    """Replaces `module.HexPlaneField` (the name the reference's scene/deformation.py constructs `Deformation.grid` with) by a
+    factory that returns b200gs.field.HexPlaneField for the configurations its kernels cover (16 or 32 channels, 1-4 levels,
+    2-D planes over x, y, z, t) and the module's original class for any other, with one line on stderr.  Same constructor
+    arguments, `feat_dim`, attribute paths and state_dict keys either way.  Idempotent.  Returns the module."""
+    orig = getattr(module, "HexPlaneField", None)
+    if orig is None or getattr(orig, "_b200gs_factory", False):
+        return module
+    from . import field
+
+    def HexPlaneField(bounds, planeconfig, multires):
+        if field.HexPlaneField.supports(planeconfig, multires):
+            return field.HexPlaneField(bounds, planeconfig, multires)
+        print(f"[b200gs] HexPlane grid {planeconfig} x {len(multires)} levels is outside the kernels' scope; using the "
+              f"reference's {orig.__module__}.HexPlaneField", file=sys.stderr)
+        return orig(bounds, planeconfig, multires)
+    HexPlaneField._b200gs_factory = True
+    HexPlaneField._b200gs_original = orig
+    module.HexPlaneField = HexPlaneField
+    return module
+
+
 def install(reference_root):
     reference_root = os.path.abspath(reference_root)
     _library_version_shims()
@@ -119,6 +142,9 @@ def install(reference_root):
             return reference_deform_network(args)
     if getattr(reference_deform_network, "__name__", "") != "make_deform_network":
         gm.deform_network = make_deform_network
+    # the reference's Deformation (the fallback above) builds its grid from this module's namespace
+    import scene.deformation
+    patch_hexplane(scene.deformation)
     densify.patch_gaussian_model(gm.GaussianModel)
     if not getattr(gm.GaussianModel, "_b200gs_patched", False):
         for name in ("training_setup", "training_setup_jih"):

@@ -11,9 +11,9 @@
 //   ix     = clamp(((x + 1) / 2) * (W - 1), 0, W - 1)               same for iy
 //   value  = nw*w_nw + ne*w_ne + sw*w_sw + se*w_se                   corner order of ATen
 //   feature[level] = 1 * v0 * v1 * v2 * v3 * v4 * v5                 (left to right), levels concatenated
-// Planes are read CHANNELS-LAST ([H][W][32] in memory; the nn.Parameter keeps its
-// [1,32,H,W] shape with torch.channels_last strides): one warp handles one point with one
-// lane per channel, so every texel fetch is a single coalesced 128-byte line.
+// Planes are read CHANNELS-LAST ([H][W][C] in memory, C = 16 or 32; the nn.Parameter keeps its
+// [1,C,H,W] shape with torch.channels_last strides): C/4 lanes serve one point with four channels
+// each, so every texel fetch is one coalesced line of C floats (128 bytes at C = 32, 64 at C = 16).
 #include "common.cuh"
 #include "radix_sort.cuh"
 #include "tc5_common.cuh"
@@ -23,8 +23,15 @@ namespace b200gs {
 
 namespace {
 
-constexpr int HP_C = 32;                 // channels per plane (output_coordinate_dim)
 constexpr int HP_MAXL = B200GS_HEXPLANE_MAX_LEVELS;
+constexpr int TR_C = 32;                 // channels of the pre-blended time-row kernels (32-channel planes only)
+
+// Channel layout of the six-plane kernels: a point slot is C/4 lanes x 4 channels, so one LDG.128 per lane fetches a whole
+// texel; C = 32: 8 lanes, 4 slots per warp; C = 16: 4 lanes, 8 slots per warp.
+template <int C> struct Lanes {
+    static_assert(C == 16 || C == 32, "HexPlane planes have 16 or 32 channels");
+    static constexpr int per_slot = C / 4, slots = 32 / per_slot;
+};
 
 
 struct Bilinear {
@@ -67,13 +74,14 @@ __device__ __forceinline__ Bilinear bilinear_setup(float x, float y, int W, int 
     return b;
 }
 
-// ---- 128-bit path: a warp serves FOUR points at once; the 8 lanes of a point slot own 4 channels
-// each, so one LDG.128 per lane fetches a whole 128-byte texel per slot. Points are visited in
+// ---- 128-bit path: a warp serves 32/(C/4) points at once (4 at C = 32, 8 at C = 16); the C/4 lanes of a point slot own 4
+// channels each, so one LDG.128 per lane fetches a whole texel per slot. Points are visited in
 // `order` (a cell-sorted permutation, see hexplane_order below) so that neighbouring warps touch
 // the same few texels and the gathers are served by L1 instead of L2.
+template <int C>
 __device__ __forceinline__ float4 ld4(const float* __restrict__ plane, int texel, int cg)
 {
-    return texel >= 0 ? __ldg(reinterpret_cast<const float4*>(plane + (size_t)texel * HP_C) + cg)
+    return texel >= 0 ? __ldg(reinterpret_cast<const float4*>(plane + (size_t)texel * C) + cg)
                       : make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
@@ -125,12 +133,12 @@ template <> struct Pair<3> { static constexpr int a = 1, b = 2; };
 template <> struct Pair<4> { static constexpr int a = 1, b = 3; };
 template <> struct Pair<5> { static constexpr int a = 2, b = 3; };
 
-template <int K>
+template <int C, int K>
 __device__ __forceinline__ float4 sample_plane(const b200gs_hexplane_desc& d, int l, const float c[4], int cg, Bilinear& b)
 {
     b = bilinear_setup(c[Pair<K>::a], c[Pair<K>::b], d.res[l][Pair<K>::a], d.res[l][Pair<K>::b]);
     const float* plane = d.plane[l][K];
-    return interp4(ld4(plane, b.o_nw, cg), ld4(plane, b.o_ne, cg), ld4(plane, b.o_sw, cg), ld4(plane, b.o_se, cg), b);
+    return interp4(ld4<C>(plane, b.o_nw, cg), ld4<C>(plane, b.o_ne, cg), ld4<C>(plane, b.o_sw, cg), ld4<C>(plane, b.o_se, cg), b);
 }
 
 __device__ __forceinline__ float4 mul4(const float4 a, const float4 b)
@@ -138,20 +146,24 @@ __device__ __forceinline__ float4 mul4(const float4 a, const float4 b)
     return make_float4(__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y), __fmul_rn(a.z, b.z), __fmul_rn(a.w, b.w));
 }
 
-__global__ void __launch_bounds__(256)
+// C = 16: five resident CTAs requested explicitly; without the bound ptxas keeps the same 48 registers but spills the aabb
+// origin to the stack and reloads it per point.  C = 32 keeps the plain bound (its code is unchanged by the 16-channel layout).
+template <int C>
+__global__ void __launch_bounds__(256, C == 16 ? 5 : 0)
 hexplane_fwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, long long P, const float* __restrict__ pts,
                     const unsigned int* __restrict__ order, const float* __restrict__ times, float time_scalar,
                     int mask, const float* __restrict__ factor, float* __restrict__ feat)
 {
-    const int lane = threadIdx.x & 31, slot = lane >> 3, cg = lane & 7;
+    constexpr int LPS = Lanes<C>::per_slot, SPW = Lanes<C>::slots;
+    const int lane = threadIdx.x & 31, slot = lane / LPS, cg = lane % LPS;
     const AabbNorm an = aabb_norm(d.aabb);
-    const int F = d.levels * HP_C;
+    const int F = d.levels * C;
     // blocked assignment: a CTA walks ONE contiguous run of the (cell-sorted) order, so the texels of a small 3-D
     // region stay in its SM's L1 from one iteration to the next (a grid-stride walk re-fetched them from L2)
-    const long long ppi = (long long)(blockDim.x >> 5) * 4;                      // points per CTA iteration
+    const long long ppi = (long long)(blockDim.x >> 5) * SPW;                    // points per CTA iteration
     const long long chunk = ((P + gridDim.x - 1) / gridDim.x + ppi - 1) / ppi * ppi;
     const long long begin = (long long)blockIdx.x * chunk, end = begin + chunk < P ? begin + chunk : P;
-    for (long long base = begin + (long long)(threadIdx.x >> 5) * 4; base < end; base += ppi) {
+    for (long long base = begin + (long long)(threadIdx.x >> 5) * SPW; base < end; base += ppi) {
         const long long i = base + slot;
         if (i >= end) continue;
         const size_t g = order ? (size_t)__ldg(order + i) : (size_t)i;
@@ -161,14 +173,14 @@ hexplane_fwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, long long P,
             Bilinear b;
             // feature = factor * prod_{k in mask} plane_k; mask = all six planes and no factor is the reference's
             // left-to-right product (hexplane.py:87-96)
-            float4 f = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * HP_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
-            if (mask & 1) f = mul4(f, sample_plane<0>(d, l, c, cg, b));
-            if (mask & 2) f = mul4(f, sample_plane<1>(d, l, c, cg, b));
-            if (mask & 4) f = mul4(f, sample_plane<2>(d, l, c, cg, b));
-            if (mask & 8) f = mul4(f, sample_plane<3>(d, l, c, cg, b));
-            if (mask & 16) f = mul4(f, sample_plane<4>(d, l, c, cg, b));
-            if (mask & 32) f = mul4(f, sample_plane<5>(d, l, c, cg, b));
-            *reinterpret_cast<float4*>(feat + g * F + l * HP_C + cg * 4) = f;
+            float4 f = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
+            if (mask & 1) f = mul4(f, sample_plane<C, 0>(d, l, c, cg, b));
+            if (mask & 2) f = mul4(f, sample_plane<C, 1>(d, l, c, cg, b));
+            if (mask & 4) f = mul4(f, sample_plane<C, 2>(d, l, c, cg, b));
+            if (mask & 8) f = mul4(f, sample_plane<C, 3>(d, l, c, cg, b));
+            if (mask & 16) f = mul4(f, sample_plane<C, 4>(d, l, c, cg, b));
+            if (mask & 32) f = mul4(f, sample_plane<C, 5>(d, l, c, cg, b));
+            *reinterpret_cast<float4*>(feat + g * F + l * C + cg * 4) = f;
         }
     }
 }
@@ -181,13 +193,13 @@ hexplane_fwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, long long P,
 // per point) and drops the second bilinear set-up.
 struct PlaneSample { float4 v, dx, dy; float ix, iy; };
 
-template <int K>
+template <int C, int K>
 __device__ __forceinline__ void sample_plane_full(const b200gs_hexplane_desc& d, int l, const float c[4], int cg, PlaneSample& s)
 {
     const int W = d.res[l][Pair<K>::a], H = d.res[l][Pair<K>::b];
     const Bilinear b = bilinear_setup(c[Pair<K>::a], c[Pair<K>::b], W, H);
     const float* plane = d.plane[l][K];
-    const float4 nw = ld4(plane, b.o_nw, cg), ne = ld4(plane, b.o_ne, cg), sw = ld4(plane, b.o_sw, cg), se = ld4(plane, b.o_se, cg);
+    const float4 nw = ld4<C>(plane, b.o_nw, cg), ne = ld4<C>(plane, b.o_ne, cg), sw = ld4<C>(plane, b.o_sw, cg), se = ld4<C>(plane, b.o_se, cg);
     s.v = interp4(nw, ne, sw, se, b);
     const float fx = (float)b.ix_nw, fy = (float)b.iy_nw;
     const float wx1 = (fx + 1.f) - b.ix, wx0 = b.ix - fx, wy1 = (fy + 1.f) - b.iy, wy0 = b.iy - fy;
@@ -200,16 +212,18 @@ __device__ __forceinline__ void sample_plane_full(const b200gs_hexplane_desc& d,
 }
 
 // Offset (floats) of the 1-D gradient row of time plane (a, t) of level l inside one replica of the row scratch.
+template <int C>
 __device__ __host__ __forceinline__ size_t time_row_offset(const b200gs_hexplane_desc& d, int l, int a)
 {
     size_t o = 0;
     for (int ll = 0; ll < l; ++ll) o += (size_t)(d.res[ll][0] + d.res[ll][1] + d.res[ll][2]);
     for (int aa = 0; aa < a; ++aa) o += (size_t)d.res[l][aa];
-    return o * HP_C;
+    return o * C;
 }
-__device__ __host__ __forceinline__ size_t time_row_floats(const b200gs_hexplane_desc& d) { return time_row_offset(d, d.levels, 0); }
+template <int C>
+__device__ __host__ __forceinline__ size_t time_row_floats(const b200gs_hexplane_desc& d) { return time_row_offset<C>(d, d.levels, 0); }
 
-template <int K>
+template <int C, int K>
 __device__ __forceinline__ void plane_backward_full(const b200gs_hexplane_desc& d, int l, int cg, const PlaneSample& s,
                                                     const float4 gv, float gc[3], float* __restrict__ rows)
 {
@@ -223,20 +237,20 @@ __device__ __forceinline__ void plane_backward_full(const b200gs_hexplane_desc& 
         // (weights wx1 / wx0); hexplane_time_rows_flush then adds wy1 / wy0 times the replica sum to the two plane rows.
         if (gp != nullptr && (gv.x != 0.f || gv.y != 0.f || gv.z != 0.f || gv.w != 0.f)) {
             const float wx1 = (fx + 1.f) - s.ix, wx0 = s.ix - fx;
-            float* base = rows + time_row_offset(d, l, Pair<K>::a) + (size_t)ixn * HP_C + cg * 4;
+            float* base = rows + time_row_offset<C>(d, l, Pair<K>::a) + (size_t)ixn * C + cg * 4;
             red_add_v4(base, gv.x * wx1, gv.y * wx1, gv.z * wx1, gv.w * wx1);
-            if (ixn + 1 < W) red_add_v4(base + HP_C, gv.x * wx0, gv.y * wx0, gv.z * wx0, gv.w * wx0);
+            if (ixn + 1 < W) red_add_v4(base + C, gv.x * wx0, gv.y * wx0, gv.z * wx0, gv.w * wx0);
         }
     } else
     if (gp != nullptr && (gv.x != 0.f || gv.y != 0.f || gv.z != 0.f || gv.w != 0.f)) {
         const float wx1 = (fx + 1.f) - s.ix, wx0 = s.ix - fx, wy1 = (fy + 1.f) - s.iy, wy0 = s.iy - fy;
         const float w_nw = wx1 * wy1, w_ne = wx0 * wy1, w_sw = wx1 * wy0, w_se = wx0 * wy0;
         const bool x1 = ixn + 1 < W, y1 = iyn + 1 < H;            // (ixn, iyn) itself is always inside: the coordinates are clamped
-        float* base = gp + ((size_t)iyn * W + ixn) * HP_C + cg * 4;
+        float* base = gp + ((size_t)iyn * W + ixn) * C + cg * 4;
         red_add_v4(base, gv.x * w_nw, gv.y * w_nw, gv.z * w_nw, gv.w * w_nw);
-        if (x1) red_add_v4(base + HP_C, gv.x * w_ne, gv.y * w_ne, gv.z * w_ne, gv.w * w_ne);
-        if (y1) red_add_v4(base + (size_t)W * HP_C, gv.x * w_sw, gv.y * w_sw, gv.z * w_sw, gv.w * w_sw);
-        if (x1 && y1) red_add_v4(base + (size_t)(W + 1) * HP_C, gv.x * w_se, gv.y * w_se, gv.z * w_se, gv.w * w_se);
+        if (x1) red_add_v4(base + C, gv.x * w_ne, gv.y * w_ne, gv.z * w_ne, gv.w * w_ne);
+        if (y1) red_add_v4(base + (size_t)W * C, gv.x * w_sw, gv.y * w_sw, gv.z * w_sw, gv.w * w_sw);
+        if (x1 && y1) red_add_v4(base + (size_t)(W + 1) * C, gv.x * w_se, gv.y * w_se, gv.z * w_se, gv.w * w_se);
     }
     // clip_coordinates_set_grad: the coordinate gradient vanishes where the border clamp is active
     if (Pair<K>::a < 3) {
@@ -249,6 +263,7 @@ __device__ __forceinline__ void plane_backward_full(const b200gs_hexplane_desc& 
     }
 }
 
+template <int C>
 __global__ void __launch_bounds__(128, 3)
 hexplane_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, long long P, const float* __restrict__ pts,
                     const unsigned int* __restrict__ order, const float* __restrict__ times, float time_scalar,
@@ -256,14 +271,15 @@ hexplane_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, long long P,
                     const float* __restrict__ dfeat, float* __restrict__ dpts /* [P,3], written */,
                     float* __restrict__ time_rows /* [replicas][time_row_floats], or null */, int replicas)
 {
-    float* rows = time_rows ? time_rows + (size_t)(blockIdx.x % replicas) * time_row_floats(d) : nullptr;
-    const int lane = threadIdx.x & 31, slot = lane >> 3, cg = lane & 7;
+    constexpr int LPS = Lanes<C>::per_slot, SPW = Lanes<C>::slots;
+    float* rows = time_rows ? time_rows + (size_t)(blockIdx.x % replicas) * time_row_floats<C>(d) : nullptr;
+    const int lane = threadIdx.x & 31, slot = lane / LPS, cg = lane % LPS;
     const AabbNorm an = aabb_norm(d.aabb);
-    const int F = d.levels * HP_C;
-    const long long ppi = (long long)(blockDim.x >> 5) * 4;                      // blocked assignment, see the forward
+    const int F = d.levels * C;
+    const long long ppi = (long long)(blockDim.x >> 5) * SPW;                    // blocked assignment, see the forward
     const long long chunk = ((P + gridDim.x - 1) / gridDim.x + ppi - 1) / ppi * ppi;
     const long long begin = (long long)blockIdx.x * chunk, end = begin + chunk < P ? begin + chunk : P;
-    for (long long base = begin + (long long)(threadIdx.x >> 5) * 4; base < end; base += ppi) {
+    for (long long base = begin + (long long)(threadIdx.x >> 5) * SPW; base < end; base += ppi) {
         const long long i = base + slot;
         const bool valid = i < end;
         const size_t g = valid ? (order ? (size_t)__ldg(order + i) : (size_t)i) : 0;
@@ -272,30 +288,30 @@ hexplane_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, long long P,
         float gc[3] = {0.f, 0.f, 0.f};
         if (valid) {
             for (int l = 0; l < d.levels; ++l) {
-                const float4 gout = __ldg(reinterpret_cast<const float4*>(dfeat + g * F + l * HP_C + cg * 4));
+                const float4 gout = __ldg(reinterpret_cast<const float4*>(dfeat + g * F + l * C + cg * 4));
                 auto mul = [](const float4 a, const float4 b) { return make_float4(a.x * b.x, a.y * b.y, a.z * b.z, a.w * b.w); };
                 // planes outside `mask` count as the constant 1 (their factor arrives through `factor` instead)
                 const float4 ones = make_float4(1.f, 1.f, 1.f, 1.f);
                 PlaneSample s0, s1, s2, s3, s4, s5;
                 s0.v = s1.v = s2.v = s3.v = s4.v = s5.v = ones;
-                if (mask & 1) sample_plane_full<0>(d, l, c, cg, s0);
-                if (mask & 2) sample_plane_full<1>(d, l, c, cg, s1);
-                if (mask & 4) sample_plane_full<2>(d, l, c, cg, s2);
-                if (mask & 8) sample_plane_full<3>(d, l, c, cg, s3);
-                if (mask & 16) sample_plane_full<4>(d, l, c, cg, s4);
-                if (mask & 32) sample_plane_full<5>(d, l, c, cg, s5);
-                const float4 go = factor ? mul(gout, __ldg(reinterpret_cast<const float4*>(factor + g * F + l * HP_C + cg * 4))) : gout;
+                if (mask & 1) sample_plane_full<C, 0>(d, l, c, cg, s0);
+                if (mask & 2) sample_plane_full<C, 1>(d, l, c, cg, s1);
+                if (mask & 4) sample_plane_full<C, 2>(d, l, c, cg, s2);
+                if (mask & 8) sample_plane_full<C, 3>(d, l, c, cg, s3);
+                if (mask & 16) sample_plane_full<C, 4>(d, l, c, cg, s4);
+                if (mask & 32) sample_plane_full<C, 5>(d, l, c, cg, s5);
+                const float4 go = factor ? mul(gout, __ldg(reinterpret_cast<const float4*>(factor + g * F + l * C + cg * 4))) : gout;
                 // prefix / suffix products of the six factors (the forward multiplies left to right)
                 const float4 p1 = s0.v, p2 = mul(p1, s1.v), p3 = mul(p2, s2.v), p4 = mul(p3, s3.v), p5 = mul(p4, s4.v);
                 const float4 q4 = s5.v, q3 = mul(q4, s4.v), q2 = mul(q3, s3.v), q1 = mul(q2, s2.v), q0 = mul(q1, s1.v);
-                if (mask & 1) plane_backward_full<0>(d, l, cg, s0, mul(go, q0), gc, rows);
-                if (mask & 2) plane_backward_full<1>(d, l, cg, s1, mul(go, mul(p1, q1)), gc, rows);
-                if (mask & 4) plane_backward_full<2>(d, l, cg, s2, mul(go, mul(p2, q2)), gc, rows);
-                if (mask & 8) plane_backward_full<3>(d, l, cg, s3, mul(go, mul(p3, q3)), gc, rows);
-                if (mask & 16) plane_backward_full<4>(d, l, cg, s4, mul(go, mul(p4, q4)), gc, rows);
-                if (mask & 32) plane_backward_full<5>(d, l, cg, s5, mul(go, p5), gc, rows);
+                if (mask & 1) plane_backward_full<C, 0>(d, l, cg, s0, mul(go, q0), gc, rows);
+                if (mask & 2) plane_backward_full<C, 1>(d, l, cg, s1, mul(go, mul(p1, q1)), gc, rows);
+                if (mask & 4) plane_backward_full<C, 2>(d, l, cg, s2, mul(go, mul(p2, q2)), gc, rows);
+                if (mask & 8) plane_backward_full<C, 3>(d, l, cg, s3, mul(go, mul(p3, q3)), gc, rows);
+                if (mask & 16) plane_backward_full<C, 4>(d, l, cg, s4, mul(go, mul(p4, q4)), gc, rows);
+                if (mask & 32) plane_backward_full<C, 5>(d, l, cg, s5, mul(go, p5), gc, rows);
                 if (dfactor) {                       // d factor += d feature * prod_{k in mask} plane_k
-                    float4* da = reinterpret_cast<float4*>(dfactor + g * F + l * HP_C + cg * 4);
+                    float4* da = reinterpret_cast<float4*>(dfactor + g * F + l * C + cg * 4);
                     const float4 prod = mul(p5, s5.v), old = *da;
                     *da = make_float4(old.x + gout.x * prod.x, old.y + gout.y * prod.y, old.z + gout.z * prod.z, old.w + gout.w * prod.w);
                 }
@@ -305,9 +321,8 @@ hexplane_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, long long P,
 #pragma unroll
             for (int a = 0; a < 3; ++a) {
                 float s = gc[a];
-                s += __shfl_xor_sync(0xffffffffu, s, 1);
-                s += __shfl_xor_sync(0xffffffffu, s, 2);
-                s += __shfl_xor_sync(0xffffffffu, s, 4);
+#pragma unroll
+                for (int o = 1; o < LPS; o <<= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
                 gc[a] = s * scale[a];
             }
             if (valid && cg < 3) dpts[3 * g + cg] = cg == 0 ? gc[0] : (cg == 1 ? gc[1] : gc[2]);
@@ -316,21 +331,22 @@ hexplane_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, long long P,
 }
 
 // Adds the replica-summed 1-D rows to the two time rows of every time plane: G[t0][x] += wy1 * r[x], G[t1][x] += wy0 * r[x].
+template <int C>
 __global__ void __launch_bounds__(256)
 hexplane_time_rows_flush_kernel(const __grid_constant__ b200gs_hexplane_desc d, float time_scalar, const float* __restrict__ rows, int replicas)
 {
-    const size_t total = time_row_floats(d);
+    const size_t total = time_row_floats<C>(d);
     const size_t i = (size_t)blockIdx.x * 256 + threadIdx.x;
     if (i >= total) return;
     int l = 0, a = 0;
-    size_t rem = i / HP_C;                                   // texel index over all (level, axis) rows
+    size_t rem = i / C;                                      // texel index over all (level, axis) rows
     for (;; ) {
         const size_t n = (size_t)d.res[l][a];
         if (rem < n) break;
         rem -= n;
         if (++a == 3) { a = 0; ++l; }
     }
-    const int K = a == 0 ? 2 : (a == 1 ? 4 : 5), ch = (int)(i % HP_C), x = (int)rem;
+    const int K = a == 0 ? 2 : (a == 1 ? 4 : 5), ch = (int)(i % C), x = (int)rem;
     float* gp = d.grad_plane[l][K];
     if (gp == nullptr) return;
     float sum = 0.f;
@@ -341,8 +357,8 @@ hexplane_time_rows_flush_kernel(const __grid_constant__ b200gs_hexplane_desc d, 
     const float fy = floorf(iy);
     const int iyn = (int)fy;
     const float wy1 = (fy + 1.f) - iy, wy0 = iy - fy;
-    gp[((size_t)iyn * W + x) * HP_C + ch] += sum * wy1;
-    if (iyn + 1 < H) gp[((size_t)(iyn + 1) * W + x) * HP_C + ch] += sum * wy0;
+    gp[((size_t)iyn * W + x) * C + ch] += sum * wy1;
+    if (iyn + 1 < H) gp[((size_t)(iyn + 1) * W + x) * C + ch] += sum * wy0;
 }
 
 
@@ -368,11 +384,11 @@ __device__ __forceinline__ void time_rows_prepare(const b200gs_hexplane_desc& d,
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
             const int K = a == 0 ? 2 : (a == 1 ? 4 : 5), W = d.res[l][a];
-            const float* g0 = d.plane[l][K] + (size_t)iyn * W * HP_C;
-            const float* g1 = g0 + (size_t)W * HP_C;
+            const float* g0 = d.plane[l][K] + (size_t)iyn * W * TR_C;
+            const float* g1 = g0 + (size_t)W * TR_C;
             // 128-bit loads, four in flight per thread: this runs before every CTA's main loop, so its latency is exposed
 #pragma unroll 4
-            for (int i = threadIdx.x; i < W * (HP_C / 4); i += blockDim.x) {
+            for (int i = threadIdx.x; i < W * (TR_C / 4); i += blockDim.x) {
                 const float4 p0 = __ldg(reinterpret_cast<const float4*>(g0) + i);
                 const float4 p1 = y1 ? __ldg(reinterpret_cast<const float4*>(g1) + i) : make_float4(0.f, 0.f, 0.f, 0.f);
                 reinterpret_cast<float4*>(R + ts.off[l][a])[i] =
@@ -393,8 +409,8 @@ __device__ __forceinline__ RowSample row_sample(const float* __restrict__ row, f
     r.x0 = (int)fx;
     r.x1 = r.x0 + 1 < W ? r.x0 + 1 : r.x0;          // out of range on the right edge: its weight is exactly 0
     r.wx1 = (fx + 1.f) - ix; r.wx0 = ix - fx;
-    const float4 a = *reinterpret_cast<const float4*>(row + r.x0 * HP_C + cg * 4);
-    const float4 b = *reinterpret_cast<const float4*>(row + r.x1 * HP_C + cg * 4);
+    const float4 a = *reinterpret_cast<const float4*>(row + r.x0 * TR_C + cg * 4);
+    const float4 b = *reinterpret_cast<const float4*>(row + r.x1 * TR_C + cg * 4);
     r.v = make_float4(__fmaf_rn(b.x, r.wx0, __fmul_rn(a.x, r.wx1)), __fmaf_rn(b.y, r.wx0, __fmul_rn(a.y, r.wx1)),
                       __fmaf_rn(b.z, r.wx0, __fmul_rn(a.z, r.wx1)), __fmaf_rn(b.w, r.wx0, __fmul_rn(a.w, r.wx1)));
     r.dv = make_float4(b.x - a.x, b.y - a.y, b.z - a.z, b.w - a.w);
@@ -411,7 +427,7 @@ hexplane_time_fwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, const _
     __syncthreads();
     const int lane = threadIdx.x & 31, slot = lane >> 3, cg = lane & 7;
     const AabbNorm an = aabb_norm(d.aabb);
-    const int F = d.levels * HP_C;
+    const int F = d.levels * TR_C;
     const long long ppi = (long long)(blockDim.x >> 5) * 4;
     const long long chunk = ((P + gridDim.x - 1) / gridDim.x + ppi - 1) / ppi * ppi;
     const long long begin = (long long)blockIdx.x * chunk, end = begin + chunk < P ? begin + chunk : P;
@@ -422,10 +438,10 @@ hexplane_time_fwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, const _
         float c[4], scale[3];
         normalized_coords(pts, nullptr, t, an, g, c, scale);
         for (int l = 0; l < d.levels; ++l) {
-            float4 f = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * HP_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
+            float4 f = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * TR_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
 #pragma unroll
             for (int a = 0; a < 3; ++a) f = mul4(f, row_sample(R + ts.off[l][a], c[a], d.res[l][a], cg).v);
-            *reinterpret_cast<float4*>(feat + (tiled ? tc5::stash_off((long long)g, l * HP_C + cg * 4) : g * F + l * HP_C + cg * 4)) = f;
+            *reinterpret_cast<float4*>(feat + (tiled ? tc5::stash_off((long long)g, l * TR_C + cg * 4) : g * F + l * TR_C + cg * 4)) = f;
         }
     }
 }
@@ -439,7 +455,7 @@ hexplane_time_fwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const 
                           const float* __restrict__ pts, const unsigned int* __restrict__ order, float t,
                           const float* __restrict__ factor, float* __restrict__ feat, int tiled)
 {
-    constexpr int L = 2, F = L * HP_C;
+    constexpr int L = 2, F = L * TR_C;
     extern __shared__ float R[];
     time_rows_prepare(d, t, R, ts);
     __syncthreads();
@@ -455,7 +471,7 @@ hexplane_time_fwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const 
         float4 f[L];
 #pragma unroll
         for (int l = 0; l < L; ++l)
-            f[l] = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * HP_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
+            f[l] = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * TR_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
         float c[4], scale[3];
         normalized_coords(pts, nullptr, t, an, g, c, scale);
 #pragma unroll
@@ -465,7 +481,7 @@ hexplane_time_fwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const 
         }
 #pragma unroll
         for (int l = 0; l < L; ++l)
-            *reinterpret_cast<float4*>(feat + (tiled ? tc5::stash_off((long long)g, l * HP_C + cg * 4) : g * F + l * HP_C + cg * 4)) = f[l];
+            *reinterpret_cast<float4*>(feat + (tiled ? tc5::stash_off((long long)g, l * TR_C + cg * 4) : g * F + l * TR_C + cg * 4)) = f[l];
     }
 }
 
@@ -484,7 +500,7 @@ hexplane_time_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, const _
     __syncthreads();
     const int lane = threadIdx.x & 31, slot = lane >> 3, cg = lane & 7;
     const AabbNorm an = aabb_norm(d.aabb);
-    const int F = d.levels * HP_C;
+    const int F = d.levels * TR_C;
     const long long ppi = (long long)(blockDim.x >> 5) * 4;
     const long long chunk = ((P + gridDim.x - 1) / gridDim.x + ppi - 1) / ppi * ppi;
     const long long begin = (long long)blockIdx.x * chunk, end = begin + chunk < P ? begin + chunk : P;
@@ -497,14 +513,14 @@ hexplane_time_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, const _
         float gc[3] = {0.f, 0.f, 0.f};
         if (valid) {
             for (int l = 0; l < d.levels; ++l) {
-                const float4 gout = __ldg(reinterpret_cast<const float4*>(dfeat + (tiled ? tc5::stash_off((long long)g, l * HP_C + cg * 4) : g * F + l * HP_C + cg * 4)));
-                const float4 fac = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * HP_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
+                const float4 gout = __ldg(reinterpret_cast<const float4*>(dfeat + (tiled ? tc5::stash_off((long long)g, l * TR_C + cg * 4) : g * F + l * TR_C + cg * 4)));
+                const float4 fac = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * TR_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
                 RowSample r[3];
 #pragma unroll
                 for (int a = 0; a < 3; ++a) r[a] = row_sample(R + ts.off[l][a], c[a], d.res[l][a], cg);
                 const float4 go = mul4(gout, fac);
                 if (dfactor) {                       // d S += d feature * T
-                    float4* da = reinterpret_cast<float4*>(dfactor + g * F + l * HP_C + cg * 4);
+                    float4* da = reinterpret_cast<float4*>(dfactor + g * F + l * TR_C + cg * 4);
                     const float4 T = mul4(mul4(r[0].v, r[1].v), r[2].v), old = overwrite ? make_float4(0.f, 0.f, 0.f, 0.f) : *da;
                     *da = make_float4(old.x + gout.x * T.x, old.y + gout.y * T.y, old.z + gout.z * T.z, old.w + gout.w * T.w);
                 }
@@ -515,10 +531,10 @@ hexplane_time_bwd_kernel(const __grid_constant__ b200gs_hexplane_desc d, const _
                         const float4 gv = mul4(go, oth);
                         // (shared-memory float atomics are compare-and-swap loops on this architecture; the vector reductions to
                         //  this CTA's replica of the global row buffer are native and four channels wide)
-                        float* g0 = rows + ts.off[l][a] + r[a].x0 * HP_C + cg * 4;
+                        float* g0 = rows + ts.off[l][a] + r[a].x0 * TR_C + cg * 4;
                         red_add_v4(g0, gv.x * r[a].wx1, gv.y * r[a].wx1, gv.z * r[a].wx1, gv.w * r[a].wx1);
                         if (r[a].x1 != r[a].x0) {
-                            float* g1 = rows + ts.off[l][a] + r[a].x1 * HP_C + cg * 4;
+                            float* g1 = rows + ts.off[l][a] + r[a].x1 * TR_C + cg * 4;
                             red_add_v4(g1, gv.x * r[a].wx0, gv.y * r[a].wx0, gv.z * r[a].wx0, gv.w * r[a].wx0);
                         }
                         gc[a] += r[a].mult * (gv.x * r[a].dv.x + gv.y * r[a].dv.y + gv.z * r[a].dv.z + gv.w * r[a].dv.w);
@@ -551,7 +567,7 @@ hexplane_time_bwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const 
                           const float* __restrict__ factor, float* __restrict__ dfactor, const float* __restrict__ dfeat,
                           float* __restrict__ dpts, float* __restrict__ time_rows, int replicas, int tiled_flags)
 {
-    constexpr int L = 2, F = L * HP_C;
+    constexpr int L = 2, F = L * TR_C;
     const int tiled = tiled_flags & 1;
     const bool overwrite = (tiled_flags & 2) != 0;          // d_factor is WRITTEN, not accumulated (a fresh buffer: no read, no memset)
     extern __shared__ float R[];
@@ -572,9 +588,9 @@ hexplane_time_bwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const 
         if (valid) {
 #pragma unroll
             for (int l = 0; l < L; ++l) {
-                gout[l] = __ldg(reinterpret_cast<const float4*>(dfeat + (tiled ? tc5::stash_off((long long)g, l * HP_C + cg * 4) : g * F + l * HP_C + cg * 4)));
-                fac[l] = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * HP_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
-                old[l] = (dfactor && !overwrite) ? *reinterpret_cast<const float4*>(dfactor + g * F + l * HP_C + cg * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
+                gout[l] = __ldg(reinterpret_cast<const float4*>(dfeat + (tiled ? tc5::stash_off((long long)g, l * TR_C + cg * 4) : g * F + l * TR_C + cg * 4)));
+                fac[l] = factor ? __ldg(reinterpret_cast<const float4*>(factor + g * F + l * TR_C + cg * 4)) : make_float4(1.f, 1.f, 1.f, 1.f);
+                old[l] = (dfactor && !overwrite) ? *reinterpret_cast<const float4*>(dfactor + g * F + l * TR_C + cg * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
             }
         }
         float c[4], scale[3];
@@ -589,7 +605,7 @@ hexplane_time_bwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const 
                 const float4 go = mul4(gout[l], fac[l]);
                 if (dfactor) {                       // d S += d feature * T
                     const float4 T = mul4(mul4(r[0].v, r[1].v), r[2].v);
-                    *reinterpret_cast<float4*>(dfactor + g * F + l * HP_C + cg * 4) =
+                    *reinterpret_cast<float4*>(dfactor + g * F + l * TR_C + cg * 4) =
                         make_float4(old[l].x + gout[l].x * T.x, old[l].y + gout[l].y * T.y, old[l].z + gout[l].z * T.z, old[l].w + gout[l].w * T.w);
                 }
                 if (go.x != 0.f || go.y != 0.f || go.z != 0.f || go.w != 0.f) {
@@ -597,10 +613,10 @@ hexplane_time_bwd2_kernel(const __grid_constant__ b200gs_hexplane_desc d, const 
                     for (int a = 0; a < 3; ++a) {
                         const float4 oth = mul4(r[(a + 1) % 3].v, r[(a + 2) % 3].v);
                         const float4 gv = mul4(go, oth);
-                        float* g0 = rows + ts.off[l][a] + r[a].x0 * HP_C + cg * 4;
+                        float* g0 = rows + ts.off[l][a] + r[a].x0 * TR_C + cg * 4;
                         red_add_v4(g0, gv.x * r[a].wx1, gv.y * r[a].wx1, gv.z * r[a].wx1, gv.w * r[a].wx1);
                         if (r[a].x1 != r[a].x0) {
-                            float* g1 = rows + ts.off[l][a] + r[a].x1 * HP_C + cg * 4;
+                            float* g1 = rows + ts.off[l][a] + r[a].x1 * TR_C + cg * 4;
                             red_add_v4(g1, gv.x * r[a].wx0, gv.y * r[a].wx0, gv.z * r[a].wx0, gv.w * r[a].wx0);
                         }
                         gc[a] += r[a].mult * (gv.x * r[a].dv.x + gv.y * r[a].dv.y + gv.z * r[a].dv.z + gv.w * r[a].dv.w);
@@ -626,7 +642,7 @@ bool time_rows_setup(const b200gs_hexplane_desc& d, TimeRowSetup& ts)
 {
     int o = 0;
     for (int l = 0; l < d.levels; ++l)
-        for (int a = 0; a < 3; ++a) { ts.off[l][a] = o; o += d.res[l][a] * HP_C; }
+        for (int a = 0; a < 3; ++a) { ts.off[l][a] = o; o += d.res[l][a] * TR_C; }
     ts.total = o;
     return (size_t)o * sizeof(float) <= 200 * 1024;             // the pre-blended rows must fit one CTA's shared memory
 }
@@ -667,6 +683,7 @@ hexplane_cellkey_kernel(long long P, const float* __restrict__ pts, const float*
 // One thread owns one (x, 4-channel) column of a channels-last plane and walks it top to bottom with the three
 // live second differences in registers: value and gradient in one pass, 8 B/parameter (+4 when the L1 term reads it
 // anyway).  dS/dG[j] = (2/N) (d[j] - 2 d[j-1] + d[j-2]),  d[i] defined for 0 <= i <= H-3.
+template <int C>
 __global__ void __launch_bounds__(128)
 hexplane_regulation_kernel(const __grid_constant__ b200gs_hexplane_desc d, float w_plane, float w_time, float w_l1,
                            float* __restrict__ loss)
@@ -680,12 +697,12 @@ hexplane_regulation_kernel(const __grid_constant__ b200gs_hexplane_desc d, float
     float* __restrict__ gG = d.grad_plane[l][k];
     const int col = blockIdx.x * 128 + threadIdx.x;            // (x, channel quad)
     float acc = 0.f;
-    if (col < W * 8) {
-        const size_t stride = (size_t)W * 8;                   // float4 units per row
+    if (col < W * (C / 4)) {
+        const size_t stride = (size_t)W * (C / 4);             // float4 units per row
         const float4* g4 = reinterpret_cast<const float4*>(G) + col;
         float4* o4 = gG ? reinterpret_cast<float4*>(gG) + col : nullptr;
-        const float cs = H > 2 ? w_s * 2.f / ((float)HP_C * (float)(H - 2) * (float)W) : 0.f;     // 2 w / N
-        const float cl = is_time ? w_l1 / ((float)HP_C * (float)H * (float)W) : 0.f;
+        const float cs = H > 2 ? w_s * 2.f / ((float)C * (float)(H - 2) * (float)W) : 0.f;        // 2 w / N
+        const float cl = is_time ? w_l1 / ((float)C * (float)H * (float)W) : 0.f;
         float sq = 0.f, l1 = 0.f;
         float4 t0 = H > 0 ? __ldg(g4) : make_float4(0.f, 0.f, 0.f, 0.f);
         float4 t1 = H > 1 ? __ldg(g4 + stride) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -724,11 +741,18 @@ hexplane_regulation_kernel(const __grid_constant__ b200gs_hexplane_desc d, float
     }
 }
 
-int validate(const b200gs_hexplane_desc* d)
+// Channel counts an entry point accepts (a set of these bits): 16 and 32 are the only layouts compiled.
+constexpr unsigned CH16 = 1, CH32 = 2;
+
+int validate(const b200gs_hexplane_desc* d, unsigned channels)
 {
     if (!d) { set_error("hexplane: null descriptor"); return -1; }
     if (d->levels < 1 || d->levels > HP_MAXL) { set_error("hexplane: levels=%d unsupported (1..%d)", d->levels, HP_MAXL); return -1; }
-    if (d->channels != HP_C) { set_error("hexplane: %d channels per plane unsupported (need %d)", d->channels, HP_C); return -1; }
+    if (!((d->channels == 16 && (channels & CH16)) || (d->channels == 32 && (channels & CH32)))) {
+        set_error("hexplane: %d channels per plane unsupported (this entry point takes %s)", d->channels,
+                  channels == CH32 ? "32" : "16 or 32");
+        return -1;
+    }
     if (!d->aabb) { set_error("hexplane: aabb is null"); return -1; }
     for (int l = 0; l < d->levels; ++l) {
         for (int a = 0; a < 4; ++a) if (d->res[l][a] < 1) { set_error("hexplane: bad resolution"); return -1; }
@@ -737,13 +761,46 @@ int validate(const b200gs_hexplane_desc* d)
     return 0;
 }
 
+template <int C>
 int grid_for(long long P)
 {
-    long long blocks = (P + 31) / 32;                // 8 warps x 4 point slots per block
+    constexpr long long per_block = 8 * Lanes<C>::slots;
+    long long blocks = (P + per_block - 1) / per_block;     // 8 warps x 4 (C = 32) or 8 (C = 16) point slots per block
     const long long cap = (long long)NUM_SMS * 8;    // persistent-style cap: 8 resident blocks per SM
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
     return (int)blocks;
+}
+
+// The six-plane backward of b200gs_hexplane_backward_masked for C channels (desc validated, P > 0).
+template <int C>
+int backward_masked(const b200gs_hexplane_desc& d, long long P, const float* pts, const unsigned int* order, const float* times,
+                    float time_scalar, int plane_mask, const float* factor, float* d_factor_accum, const float* d_features, float* d_pts,
+                    void* time_row_scratch, size_t time_row_scratch_bytes, cudaStream_t stream)
+{
+    // uniform-time fast path for the time planes' gradient: needs one shared timestamp (times == null) and scratch
+    float* rows = nullptr;
+    int replicas = 0;
+    if (times == nullptr && time_row_scratch != nullptr && (plane_mask & 0x34)) {
+        const size_t per = time_row_floats<C>(d) * sizeof(float);
+        replicas = (int)(time_row_scratch_bytes / per);
+        if (replicas > 64) replicas = 64;
+        if (replicas >= 1) {
+            rows = (float*)time_row_scratch;
+            cudaMemsetAsync(rows, 0, per * replicas, stream);
+        }
+    }
+    // 4 warps x 4 (C = 32) or 8 (C = 16) point slots per block, 3 blocks resident per SM (170 registers)
+    constexpr long long per_block = 4 * Lanes<C>::slots;
+    long long blocks = (P + per_block - 1) / per_block;
+    if (blocks > (long long)NUM_SMS * 12) blocks = (long long)NUM_SMS * 12;
+    hexplane_bwd_kernel<C><<<(unsigned)blocks, 128, 0, stream>>>(d, P, pts, order, times, time_scalar, plane_mask & 63, factor,
+                                                                 d_factor_accum, d_features, d_pts, rows, replicas);
+    if (rows) {
+        const size_t total = time_row_floats<C>(d);
+        hexplane_time_rows_flush_kernel<C><<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(d, time_scalar, rows, replicas);
+    }
+    return check_launch("hexplane_backward");
 }
 
 }  // namespace
@@ -780,9 +837,12 @@ int b200gs_hexplane_forward_masked(const b200gs_hexplane_desc* desc, long long P
                                    const float* times, float time_scalar, int plane_mask, const float* factor, float* features,
                                    b200gs_stream_t stream)
 {
-    if (validate(desc)) return -1;
+    if (validate(desc, CH16 | CH32)) return -1;
     if (P <= 0) return 0;
-    hexplane_fwd_kernel<<<grid_for(P), 256, 0, (cudaStream_t)stream>>>(*desc, P, pts, order, times, time_scalar, plane_mask & 63, factor, features);
+    if (desc->channels == 16)
+        hexplane_fwd_kernel<16><<<grid_for<16>(P), 256, 0, (cudaStream_t)stream>>>(*desc, P, pts, order, times, time_scalar, plane_mask & 63, factor, features);
+    else
+        hexplane_fwd_kernel<32><<<grid_for<32>(P), 256, 0, (cudaStream_t)stream>>>(*desc, P, pts, order, times, time_scalar, plane_mask & 63, factor, features);
     return check_launch("hexplane_forward");
 }
 
@@ -797,35 +857,21 @@ int b200gs_hexplane_backward_masked(const b200gs_hexplane_desc* desc, long long 
                                     const float* d_features, float* d_pts, void* time_row_scratch, size_t time_row_scratch_bytes,
                                     b200gs_stream_t stream)
 {
-    if (validate(desc)) return -1;
+    if (validate(desc, CH16 | CH32)) return -1;
     if (P <= 0) return 0;
-    // uniform-time fast path for the time planes' gradient: needs one shared timestamp (times == null) and scratch
-    float* rows = nullptr;
-    int replicas = 0;
-    if (times == nullptr && time_row_scratch != nullptr && (plane_mask & 0x34)) {
-        const size_t per = time_row_floats(*desc) * sizeof(float);
-        replicas = (int)(time_row_scratch_bytes / per);
-        if (replicas > 64) replicas = 64;
-        if (replicas >= 1) {
-            rows = (float*)time_row_scratch;
-            cudaMemsetAsync(rows, 0, per * replicas, (cudaStream_t)stream);
-        }
-    }
-    long long blocks = (P + 15) / 16;                // 4 warps x 4 point slots per block, 3 blocks resident per SM (170 registers)
-    if (blocks > (long long)NUM_SMS * 12) blocks = (long long)NUM_SMS * 12;
-    hexplane_bwd_kernel<<<(unsigned)blocks, 128, 0, (cudaStream_t)stream>>>(*desc, P, pts, order, times, time_scalar, plane_mask & 63, factor,
-                                                                            d_factor_accum, d_features, d_pts, rows, replicas);
-    if (rows) {
-        const size_t total = time_row_floats(*desc);
-        hexplane_time_rows_flush_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(*desc, time_scalar, rows, replicas);
-    }
-    return check_launch("hexplane_backward");
+    return desc->channels == 16
+        ? backward_masked<16>(*desc, P, pts, order, times, time_scalar, plane_mask, factor, d_factor_accum, d_features, d_pts,
+                              time_row_scratch, time_row_scratch_bytes, (cudaStream_t)stream)
+        : backward_masked<32>(*desc, P, pts, order, times, time_scalar, plane_mask, factor, d_factor_accum, d_features, d_pts,
+                              time_row_scratch, time_row_scratch_bytes, (cudaStream_t)stream);
 }
 
 size_t b200gs_hexplane_time_row_scratch_bytes(const b200gs_hexplane_desc* desc, int replicas)
 {
     if (!desc || desc->levels < 1 || desc->levels > HP_MAXL || replicas < 1) return 0;
-    return time_row_floats(*desc) * sizeof(float) * (size_t)replicas;
+    if (desc->channels == 16) return time_row_floats<16>(*desc) * sizeof(float) * (size_t)replicas;
+    if (desc->channels == 32) return time_row_floats<32>(*desc) * sizeof(float) * (size_t)replicas;
+    return 0;
 }
 
 int b200gs_hexplane_backward(const b200gs_hexplane_desc* desc, long long P, const float* pts, const unsigned int* order,
@@ -838,19 +884,24 @@ int b200gs_hexplane_backward(const b200gs_hexplane_desc* desc, long long P, cons
 int b200gs_hexplane_regulation(const b200gs_hexplane_desc* desc, float plane_tv_weight, float time_smoothness_weight,
                                float l1_time_planes_weight, float* loss_accum, b200gs_stream_t stream)
 {
-    if (validate(desc)) return -1;
+    if (validate(desc, CH16 | CH32)) return -1;
     int wmax = 1;
     for (int l = 0; l < desc->levels; ++l)
         for (int a = 0; a < 3; ++a) wmax = desc->res[l][a] > wmax ? desc->res[l][a] : wmax;
-    dim3 grid((unsigned)((wmax * 8 + 127) / 128), (unsigned)(desc->levels * 6));
-    hexplane_regulation_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(*desc, plane_tv_weight, time_smoothness_weight,
-                                                                        l1_time_planes_weight, loss_accum);
+    const int quads = desc->channels / 4;            // one thread per (x, 4-channel) column
+    dim3 grid((unsigned)((wmax * quads + 127) / 128), (unsigned)(desc->levels * 6));
+    if (desc->channels == 16)
+        hexplane_regulation_kernel<16><<<grid, 128, 0, (cudaStream_t)stream>>>(*desc, plane_tv_weight, time_smoothness_weight,
+                                                                                l1_time_planes_weight, loss_accum);
+    else
+        hexplane_regulation_kernel<32><<<grid, 128, 0, (cudaStream_t)stream>>>(*desc, plane_tv_weight, time_smoothness_weight,
+                                                                                l1_time_planes_weight, loss_accum);
     return check_launch("hexplane_regulation");
 }
 
 int b200gs_hexplane_time_supported(const b200gs_hexplane_desc* desc)
 {
-    if (validate(desc)) return 0;
+    if (validate(desc, CH32)) return 0;
     TimeRowSetup ts;
     return time_rows_setup(*desc, ts) ? 1 : 0;
 }
@@ -858,7 +909,7 @@ int b200gs_hexplane_time_supported(const b200gs_hexplane_desc* desc)
 int b200gs_hexplane_time_forward(const b200gs_hexplane_desc* desc, long long P, const float* pts, const unsigned int* order,
                                  float time_scalar, const float* factor, float* features, int features_tiled, b200gs_stream_t stream)
 {
-    if (validate(desc)) return -1;
+    if (validate(desc, CH32)) return -1;
     if (features_tiled && desc->levels != 2) { set_error("hexplane_time_forward: tiled features need 2 levels (64 columns)"); return -1; }
     TimeRowSetup ts;
     if (!time_rows_setup(*desc, ts)) { set_error("hexplane_time_forward: time rows do not fit shared memory"); return -1; }
@@ -883,7 +934,7 @@ int b200gs_hexplane_time_backward(const b200gs_hexplane_desc* desc, long long P,
                                   float* d_pts, void* time_row_scratch, size_t time_row_scratch_bytes, int d_features_tiled,
                                   b200gs_stream_t stream)
 {
-    if (validate(desc)) return -1;
+    if (validate(desc, CH32)) return -1;
     if ((d_features_tiled & 1) && desc->levels != 2) { set_error("hexplane_time_backward: tiled d_features need 2 levels (64 columns)"); return -1; }
     TimeRowSetup ts;
     if (!time_rows_setup(*desc, ts)) { set_error("hexplane_time_backward: time rows do not fit shared memory"); return -1; }
@@ -907,7 +958,7 @@ int b200gs_hexplane_time_backward(const b200gs_hexplane_desc* desc, long long P,
         hexplane_time_bwd_kernel<<<(unsigned)blocks, 256, per, (cudaStream_t)stream>>>(*desc, ts, P, pts, order, time_scalar, factor, d_factor_accum,
                                                                                        d_features, d_pts, rows, replicas, d_features_tiled);
     }
-    hexplane_time_rows_flush_kernel<<<(unsigned)((ts.total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(*desc, time_scalar, rows, replicas);
+    hexplane_time_rows_flush_kernel<TR_C><<<(unsigned)((ts.total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(*desc, time_scalar, rows, replicas);
     return check_launch("hexplane_time_backward");
 }
 

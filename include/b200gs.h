@@ -203,13 +203,17 @@ int b200gs_reset_opacity(long long N, const float* opacity_raw, float* out, b200
  * scene/hexplane.py::HexPlaneField.forward (:177, interpolate_ms_features :73-106: 6*levels
  * F.grid_sample + products + cat) and scene/deformation.py::Deformation.forward_dynamic
  * (:97-153: feature_out Linear + three ReLU-Linear-ReLU-Linear heads on cuBLAS), forward and
- * backward. Planes are CHANNELS-LAST: plane[l][k] points at [res_b][res_a][32] floats for the
+ * backward. Planes are CHANNELS-LAST: plane[l][k] points at [res_b][res_a][channels] floats for the
  * coordinate pair k = (a,b) in (0,1)(0,2)(0,3)(1,2)(1,3)(2,3); res[l] = resolution of x,y,z,t.
  * ------------------------------------------------------------------------------------- */
 #define B200GS_HEXPLANE_MAX_LEVELS 4
 typedef struct {
     int levels;
-    int channels;                                   /* 32 */
+    int channels;                                   /* 16 or 32 (output_coordinate_dim). 16 is taken by the six-plane
+                                                       entry points (_forward, _backward, their _masked variants, the
+                                                       time-row scratch size, _regulation); the pre-blended time-row
+                                                       entry points (_time_forward / _time_backward) take 32 only and
+                                                       _time_supported returns 0 for 16. Other counts are refused. */
     int res[B200GS_HEXPLANE_MAX_LEVELS][4];
     const float* plane[B200GS_HEXPLANE_MAX_LEVELS][6];
     float* grad_plane[B200GS_HEXPLANE_MAX_LEVELS][6]; /* backward: accumulated into (caller zero-fills); null = skip */
@@ -222,17 +226,17 @@ typedef struct {
 size_t b200gs_hexplane_order_scratch_bytes(long long P);
 int b200gs_hexplane_order(long long P, const float* pts, const float* aabb, unsigned int* order, void* scratch,
                           size_t scratch_bytes, b200gs_stream_t stream);
-/* features[P, 32*levels] = HexPlaneField(pts[P,3], t). times[P] may be null -> time_scalar for all. */
+/* features[P, channels*levels] = HexPlaneField(pts[P,3], t). times[P] may be null -> time_scalar for all. */
 int b200gs_hexplane_forward(const b200gs_hexplane_desc* desc /* host */, long long P, const float* pts,
                             const unsigned int* order, const float* times, float time_scalar, float* features,
                             b200gs_stream_t stream);
-/* plane gradients are ACCUMULATED into desc->grad_plane; d_pts[P,3] (may be null) is written. */
+/* plane gradients are ACCUMULATED into desc->grad_plane; d_pts[P,3] (may be null) is written; d_features[P, channels*levels]. */
 int b200gs_hexplane_backward(const b200gs_hexplane_desc* desc /* host */, long long P, const float* pts,
                              const unsigned int* order, const float* times, float time_scalar,
                              const float* d_features, float* d_pts, b200gs_stream_t stream);
 
 typedef struct {
-    int feat_dim;                 /* 32 * levels (64 or 128) */
+    int feat_dim;                 /* the grid's channels * levels; these kernels take 64 or 128 (32 channels, 2 or 4 levels) */
     int width;                    /* net_width, 64 */
     const float* w1; const float* b1;           /* feature_out.0  [64, feat_dim], [64] */
     const float* w2[3]; const float* b2[3];     /* {pos,scales,rotations}_deform.1  [64,64],[64]; null = head off (no_dx/no_ds/no_dr) */
@@ -303,7 +307,8 @@ int b200gs_deform_heads_backward(const b200gs_heads_weights* w /* host */, const
  * each view of a multi-view batch only samples the time planes (2,4,5: mask 0x34): the Gaussians' xyz do not change
  * within a step, so the spatial product is shared by all its views.  The backward additionally ACCUMULATES
  * d_factor_accum[P,F] += d_features * prod_{k in plane_mask} plane_k (null = skip), which is the upstream gradient of the
- * deferred spatial pass.  mask 0x3F with null factor is exactly b200gs_hexplane_forward / _backward. */
+ * deferred spatial pass.  factor / d_factor_accum / features / d_features are [P, channels*levels].  mask 0x3F with null factor
+ * is exactly b200gs_hexplane_forward / _backward. */
 int b200gs_hexplane_forward_masked(const b200gs_hexplane_desc* desc, long long P, const float* pts, const unsigned int* order,
                                    const float* times, float time_scalar, int plane_mask, const float* factor, float* features,
                                    b200gs_stream_t stream);
@@ -313,14 +318,17 @@ int b200gs_hexplane_backward_masked(const b200gs_hexplane_desc* desc, long long 
                                     b200gs_stream_t stream);
 /* Optional scratch for the backward above when the whole launch shares ONE timestamp (times == null): the time planes'
  * gradient is then reduced along x into up to 64 replicas of a 1-D row per plane (so the few hundred hot 128-byte lines of
- * the two touched time rows do not serialise in L2) and added to the planes by a small follow-up kernel. null = classic path. */
+ * the two touched time rows do not serialise in L2) and added to the planes by a small follow-up kernel. null = classic path.
+ * The size depends on desc->channels (0 for a count other than 16 or 32). */
 size_t b200gs_hexplane_time_row_scratch_bytes(const b200gs_hexplane_desc* desc, int replicas);
 
 /* Time planes only (mask 0x34), ONE timestamp for the whole launch, served from shared memory: every CTA pre-blends the two
  * touched time rows of each (x,t) / (y,t) / (z,t) plane into a 1-D row, samples become 1-D lerps without global texel traffic,
  * and the backward reduces the row gradients into replicated 1-D rows (time_row_scratch, as for the _masked variant; required). Same contract as the
  * _masked variants with plane_mask = 0x34 and times = null (results differ from them by FP32 re-association only).
- * b200gs_hexplane_time_supported: 1 when the rows of this descriptor fit one CTA's shared memory (2 levels at 64 / 128).
+ * 32-channel planes only: the forward and backward refuse 16 channels before any launch.
+ * b200gs_hexplane_time_supported: 1 when the descriptor has 32 channels and its rows fit one CTA's shared memory (2 levels at
+ * 64 / 128), else 0.
  * d_features_tiled of the backward is a flag word: bit 0 = d_features in the MLP kernels' tiled layout, bit 1 = d_factor_accum is
  * WRITTEN instead of accumulated (a fresh per-view buffer under autograd: saves its zero fill and the read). */
 int b200gs_hexplane_time_supported(const b200gs_hexplane_desc* desc);
