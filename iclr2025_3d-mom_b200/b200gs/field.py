@@ -75,6 +75,24 @@ _lib.register("b200gs_hexplane_time_forward", ctypes.c_int,
               [ctypes.POINTER(_HexDesc), ctypes.c_longlong, _P, _P, ctypes.c_float, _P, _P, ctypes.c_int, _P])
 _lib.register("b200gs_hexplane_time_backward", ctypes.c_int,
               [ctypes.POINTER(_HexDesc), ctypes.c_longlong, _P, _P, ctypes.c_float, _P, _P, _P, _P, _P, ctypes.c_size_t, ctypes.c_int, _P])
+_lib.register("b200gs_hexplane_order_scratch_bytes", ctypes.c_size_t, [ctypes.c_longlong])
+_lib.register("b200gs_hexplane_order", ctypes.c_int, [ctypes.c_longlong, _P, _P, _P, _P, ctypes.c_size_t, _P])
+_lib.register("b200gs_hexplane_regulation", ctypes.c_int,
+              [ctypes.POINTER(_HexDesc), ctypes.c_float, ctypes.c_float, ctypes.c_float, _P, _P])
+_lib.register("b200gs_uniform_value", ctypes.c_int, [ctypes.c_longlong, _P, _P, _P, _P])
+_lib.register("b200gs_deform_mlp_saved_floats", ctypes.c_size_t, [ctypes.c_longlong])
+_lib.register("b200gs_deform_mlp_forward", ctypes.c_int,
+              [ctypes.POINTER(_MlpWeights), ctypes.c_longlong, _P, _P, _P, _P, _P, ctypes.c_float, _P, ctypes.c_float,
+               _P, _P, _P, _P, _P])
+_lib.register("b200gs_deform_mlp_backward", ctypes.c_int,
+              [ctypes.POINTER(_MlpWeights), ctypes.POINTER(_MlpGrads), ctypes.c_longlong, _P, _P, _P, _P, _P, _P, _P])
+_lib.register("b200gs_deform_heads_saved_floats", ctypes.c_size_t, [ctypes.c_longlong])
+_lib.register("b200gs_deform_heads_forward", ctypes.c_int,
+              [ctypes.POINTER(_HeadsWeights), ctypes.c_longlong, ctypes.c_int, _P, _P, _P, _P, _P, _P, _P])
+_lib.register("b200gs_deform_heads_backward", ctypes.c_int,
+              [ctypes.POINTER(_HeadsWeights), ctypes.POINTER(_HeadsGrads), ctypes.c_longlong, ctypes.c_int, _P, _P, _P, _P, _P, _P,
+               _P, ctypes.c_int, _P])
+
 _ROW_SCRATCH = {}
 TIME_ROW_REPLICAS = 64
 
@@ -87,8 +105,7 @@ def _time_row_scratch(d, device):
         t = torch.empty((n,), dtype=torch.uint8, device=device)
         _ROW_SCRATCH[device] = t
     return t, n
-_lib.register("b200gs_hexplane_order_scratch_bytes", ctypes.c_size_t, [ctypes.c_longlong])
-_lib.register("b200gs_hexplane_order", ctypes.c_int, [ctypes.c_longlong, _P, _P, _P, _P, ctypes.c_size_t, _P])
+
 
 _ORDER_CACHE = {}
 ORDER_MIN_POINTS = 1 << 14
@@ -120,24 +137,6 @@ def _cell_order(pts, aabb):
     _lib.COUNTERS["cell_order_sorts"] += 1
     _ORDER_CACHE[pts.device] = (key, order, pts._version, pts)
     return order
-
-
-def _optr(order):
-    return order.data_ptr() if order is not None else None
-_lib.register("b200gs_deform_mlp_saved_floats", ctypes.c_size_t, [ctypes.c_longlong])
-_lib.register("b200gs_deform_mlp_forward", ctypes.c_int,
-              [ctypes.POINTER(_MlpWeights), ctypes.c_longlong, _P, _P, _P, _P, _P, ctypes.c_float, _P, ctypes.c_float,
-               _P, _P, _P, _P, _P])
-_lib.register("b200gs_deform_mlp_backward", ctypes.c_int,
-              [ctypes.POINTER(_MlpWeights), ctypes.POINTER(_MlpGrads), ctypes.c_longlong, _P, _P, _P, _P, _P, _P, _P])
-_lib.register("b200gs_deform_heads_saved_floats", ctypes.c_size_t, [ctypes.c_longlong])
-_lib.register("b200gs_deform_heads_forward", ctypes.c_int,
-              [ctypes.POINTER(_HeadsWeights), ctypes.c_longlong, ctypes.c_int, _P, _P, _P, _P, _P, _P, _P])
-_lib.register("b200gs_deform_heads_backward", ctypes.c_int,
-              [ctypes.POINTER(_HeadsWeights), ctypes.POINTER(_HeadsGrads), ctypes.c_longlong, ctypes.c_int, _P, _P, _P, _P, _P, _P,
-               _P, ctypes.c_int, _P])
-_lib.register("b200gs_hexplane_regulation", ctypes.c_int,
-              [ctypes.POINTER(_HexDesc), ctypes.c_float, ctypes.c_float, ctypes.c_float, _P, _P])
 
 
 def _cl(t):
@@ -173,7 +172,6 @@ def _check_cuda_f32(*ts):
             raise RuntimeError(f"expected float32, got {t.dtype}")
 
 
-_lib.register("b200gs_uniform_value", ctypes.c_int, [ctypes.c_longlong, _P, _P, _P, _P])
 # The reference's render() repeats the camera's ONE timestamp into a [P,1] tensor (gaussian_renderer/__init__.py:56).  With this
 # switch on (default) a tensor timestamp is checked on the device -- one tiny kernel + an 8-byte read-back, i.e. a host sync a few
 # hundred microseconds before the one the rasterizer forward performs anyway -- and a uniform one takes the same one-timestamp
@@ -224,7 +222,7 @@ class _HexPlaneFn(torch.autograd.Function):
         feat = torch.empty((P, int(planes[0].shape[1]) * levels), dtype=torch.float32, device=pts.device)
         d = _hex_desc(aabb, planes, levels, res)
         order = _cell_order(pts, aabb)
-        check(_lib.lib().b200gs_hexplane_forward(ctypes.byref(d), P, pts.data_ptr(), _optr(order),
+        check(_lib.lib().b200gs_hexplane_forward(ctypes.byref(d), P, pts.data_ptr(), _lib.ptr(order),
                                                  tt.data_ptr() if tt is not None else None, ts, feat.data_ptr(),
                                                  current_stream()), "hexplane_forward")
         ctx.save_for_backward(pts, tt if tt is not None else torch.empty(0), aabb, *planes)
@@ -246,12 +244,12 @@ class _HexPlaneFn(torch.autograd.Function):
             # One timestamp for the whole call (the reference's render() passes the camera's one time): every point adds into
             # the same two rows of each time plane, so their gradient is reduced through replicated 1-D rows first.
             scratch, nbytes = _time_row_scratch(d, pts.device)
-            check(_lib.lib().b200gs_hexplane_backward_masked(ctypes.byref(d), P, pts.data_ptr(), _optr(ctx.order), None, ts, MASK_ALL,
+            check(_lib.lib().b200gs_hexplane_backward_masked(ctypes.byref(d), P, pts.data_ptr(), _lib.ptr(ctx.order), None, ts, MASK_ALL,
                                                              None, None, d_feat.data_ptr(),
                                                              d_pts.data_ptr() if d_pts is not None else None, scratch.data_ptr(),
                                                              nbytes, current_stream()), "hexplane_backward")
             return (d_pts, None, None, None, None, *grads)
-        check(_lib.lib().b200gs_hexplane_backward(ctypes.byref(d), P, pts.data_ptr(), _optr(ctx.order),
+        check(_lib.lib().b200gs_hexplane_backward(ctypes.byref(d), P, pts.data_ptr(), _lib.ptr(ctx.order),
                                                   tt.data_ptr() if has_t else None, ts, d_feat.data_ptr(),
                                                   d_pts.data_ptr() if d_pts is not None else None, current_stream()),
               "hexplane_backward")
@@ -281,13 +279,69 @@ def _grad_target(param):
     return None
 
 
-# ---- spatial planes shared by the views of one optimiser step -------------------------------------
+# ---- the spatial product, shared by several field calls ----------------------------------------------
 # The Gaussians' xyz do not change between the views of a batch, so the product of the three SPATIAL planes
 # (xy, xz, yz) is the same for every view: b200gs.engine.ViewParallelTrainer evaluates it once per step
 # (begin_shared_step), each view then samples only the three TIME planes and multiplies, each view's backward
 # accumulates the spatial product's upstream gradient, and ONE spatial backward per step (finish_shared_step)
 # scatters it. Same mathematics as six planes per view (the product is re-associated), ~half the gathers / REDs.
+# Three holders keep a _SpatialProduct, each for its own lifetime: the explicit scope (_SHARED), the no-grad cache (_INFER), autograd's (_AUTO).
 MASK_SPATIAL, MASK_TIME, MASK_ALL = 0x0B, 0x34, 0x3F
+
+
+def _is_spatial(k):
+    """Whether plane k of the planes list (six per level: xy, xz, xt, yz, yt, zt) is one of MASK_SPATIAL's planes."""
+    return MASK_SPATIAL >> (k % 6) & 1
+
+
+def _product_key(xyz, version, aabb, planes):
+    """Identity of everything the spatial product depends on: the same tensors at the same versions.  FusedAdam.step writes
+    parameters through raw pointers and bumps their versions explicitly (adam.py), so an optimiser step always changes it."""
+    return (xyz.data_ptr(), version, int(xyz.shape[0]), aabb.data_ptr(), aabb._version) + tuple((p.data_ptr(), p._version) for p in planes)
+
+
+class _SpatialProduct:
+    """S[P, 32 levels] = product over the three spatial planes of the bilinear samples at xyz, per level, for the field calls
+    whose (xyz, aabb, planes) match `key`.  A trainer step's also holds A, its views' summed dL/dS (A_written: the first view's
+    backward has written it), and the xyz leaf and grid of its deferred backward; `auto`: each view's dL/dS goes to autograd."""
+
+    def __init__(self, key, xyz, aabb, planes, levels, res, order, auto=False):
+        self.key, self.order, self.auto = key, order, auto
+        self.A, self.A_written, self.xyz_param, self.grid = None, False, None, None
+        P = int(xyz.shape[0])
+        self.S = torch.empty((P, 32 * levels), dtype=torch.float32, device=xyz.device)
+        d = _hex_desc(aabb, planes, levels, res)
+        check(_lib.lib().b200gs_hexplane_forward_masked(ctypes.byref(d), P, xyz.data_ptr(), _lib.ptr(order), None, 0.0, MASK_SPATIAL, None,
+                                                        self.S.data_ptr(), current_stream()), "hexplane_forward(spatial)")
+        _lib.COUNTERS["spatial_product_evaluations"] += 1
+
+    def matches(self, xyz, aabb, planes):
+        return self.key == _product_key(xyz, xyz._version, aabb, planes)
+
+    @staticmethod
+    def backward(dS, xyz, order, aabb, planes, levels, res, grads):
+        """dS into `grads` (the spatial planes' gradient buffers, None for the others); returns d_xyz.  Static: _SpatialFn's
+        node must not hold the product, which holds that node's output S (a reference cycle)."""
+        d = _hex_desc(aabb, planes, levels, res, grads)
+        d_xyz = torch.empty_like(xyz)
+        check(_lib.lib().b200gs_hexplane_backward_masked(ctypes.byref(d), int(xyz.shape[0]), xyz.data_ptr(), _lib.ptr(order), None, 0.0,
+                                                         MASK_SPATIAL, None, None, dS.data_ptr(), d_xyz.data_ptr(), None, 0,
+                                                         current_stream()), "hexplane_backward(spatial)")
+        return d_xyz
+
+    def view_gradient(self, accumulate_only):
+        """Where a view's backward puts its dL/dS: (buffer, whether the kernel writes it rather than adds to it).  Autograd
+        holder: a fresh buffer per view, handed back to autograd.  Trainer step: A, written by the step's first view and added
+        to by the rest.  A kernel that can only accumulate (accumulate_only) gets the buffer zeroed instead of written."""
+        if self.auto:
+            buf, first = torch.empty_like(self.S), True
+        else:
+            buf, first, self.A_written = self.A, not self.A_written, True
+        if first and accumulate_only:
+            buf.zero_()
+        return buf, first and not accumulate_only
+
+
 _SHARED = None
 
 
@@ -297,18 +351,12 @@ def begin_shared_step(net, xyz_param, inference=False):
     global _SHARED
     grid = net.deformation_net.grid
     planes = grid._planes()
-    levels, res = len(grid.grids), tuple(grid._res)
     xyz = xyz_param.detach().contiguous()
     _check_cuda_f32(xyz, grid.aabb, *planes)
-    P = int(xyz.shape[0])
-    S = torch.empty((P, 32 * levels), dtype=torch.float32, device=xyz.device)
-    d = _hex_desc(grid.aabb, planes, levels, res)
-    order = _cell_order(xyz, grid.aabb)
-    check(_lib.lib().b200gs_hexplane_forward_masked(ctypes.byref(d), P, xyz.data_ptr(), _optr(order), None, 0.0, MASK_SPATIAL, None,
-                                                    S.data_ptr(), current_stream()), "hexplane_forward(spatial)")
-    _lib.COUNTERS["spatial_product_evaluations"] += 1
-    _SHARED = {"key": _shared_key(xyz, xyz_param._version, P, grid.aabb, planes), "S": S, "A": None if inference else torch.empty_like(S), "A_written": False,
-               "xyz_param": xyz_param, "grid": grid, "order": order, "used": False}      # A: written by the first view's backward, added to by the others
+    sh = _SpatialProduct(_product_key(xyz, xyz_param._version, grid.aabb, planes), xyz, grid.aabb, planes, len(grid.grids),
+                         tuple(grid._res), _cell_order(xyz, grid.aabb))
+    sh.A, sh.xyz_param, sh.grid = None if inference else torch.empty_like(sh.S), xyz_param, grid
+    _SHARED = sh
 
 
 @contextlib.contextmanager
@@ -330,42 +378,19 @@ def finish_shared_step():
     """The deferred spatial backward: plane gradients into the planes' .grad, xyz gradient into xyz_param.grad."""
     global _SHARED
     sh, _SHARED = _SHARED, None
-    if sh is None or not sh["used"] or not sh.get("A_written", False):
+    if sh is None or not sh.A_written:
         return          # no view's backward contributed
-    grid, xyz_param = sh["grid"], sh["xyz_param"]
+    grid, xyz_param = sh.grid, sh.xyz_param
     planes = grid._planes()
-    grads = []
-    for k, p in enumerate(planes):
-        if (k % 6) in (0, 1, 3):
-            if p.grad is None or p.grad.stride() != p.stride():
-                raise RuntimeError("finish_shared_step needs channels-last .grad buffers on the spatial planes")
-            grads.append(p.grad)
-        else:
-            grads.append(None)
+    grads = [p.grad if _is_spatial(k) else None for k, p in enumerate(planes)]
+    if any(_is_spatial(k) and (p.grad is None or p.grad.stride() != p.stride()) for k, p in enumerate(planes)):
+        raise RuntimeError("finish_shared_step needs channels-last .grad buffers on the spatial planes")
     xyz = xyz_param.detach().contiguous()
-    P = int(xyz.shape[0])
-    d = _hex_desc(grid.aabb, planes, len(grid.grids), tuple(grid._res), grads)
-    d_xyz = torch.empty_like(xyz)
-    check(_lib.lib().b200gs_hexplane_backward_masked(ctypes.byref(d), P, xyz.data_ptr(), _optr(sh["order"]), None, 0.0, MASK_SPATIAL,
-                                                     None, None, sh["A"].data_ptr(), d_xyz.data_ptr(), None, 0, current_stream()),
-          "hexplane_backward(spatial)")
+    d_xyz = _SpatialProduct.backward(sh.A, xyz, sh.order, grid.aabb, planes, len(grid.grids), tuple(grid._res), grads)
     if xyz_param.grad is None:
         xyz_param.grad = d_xyz
     else:
         xyz_param.grad += d_xyz
-
-
-def _shared_key(xyz, version, P, aabb, planes):
-    """Identity of everything the spatial product depends on: the same tensors at the same versions.  FusedAdam.step writes
-    parameters through raw pointers and bumps their versions explicitly (adam.py), so an optimiser step always changes it."""
-    return (xyz.data_ptr(), version, P, aabb.data_ptr(), aabb._version) + tuple((p.data_ptr(), p._version) for p in planes)
-
-
-def _shared_for(xyz, P, aabb, planes):
-    sh = _SHARED
-    if sh is not None and sh["key"] == _shared_key(xyz, xyz._version, P, aabb, planes):
-        return sh
-    return None
 
 
 def drop_shared():
@@ -380,7 +405,7 @@ def drop_shared():
 # shared_spatial_product does for a caller that can wrap its frame loop, done implicitly for callers that cannot -- the
 # reference's own render_4DGS.py running unchanged through the launcher.  Under torch.no_grad() the spatial product is kept
 # between calls for as long as xyz, the aabb and every plane are the same tensors at the same version; FusedAdam.step() writes
-# parameters through raw pointers (no version bump), so it drops the cache explicitly.
+# parameters through raw pointers, so it drops the cache explicitly as well.
 INFERENCE_SPATIAL_CACHE = os.environ.get("B200GS_INFERENCE_SPATIAL_CACHE") == "1"
 _INFER = None
 
@@ -388,21 +413,6 @@ _INFER = None
 def invalidate_inference_cache():
     global _INFER
     _INFER = None
-
-
-def _inference_shared(xyz, P, aabb, planes, levels, res, order):
-    global _INFER
-    if not INFERENCE_SPATIAL_CACHE or torch.is_grad_enabled():
-        return None
-    key = (xyz.data_ptr(), xyz._version, P, aabb.data_ptr(), aabb._version) + tuple((p.data_ptr(), p._version) for p in planes)
-    if _INFER is None or _INFER["key"] != key:
-        S = torch.empty((P, 32 * levels), dtype=torch.float32, device=xyz.device)
-        d = _hex_desc(aabb, planes, levels, res)
-        check(_lib.lib().b200gs_hexplane_forward_masked(ctypes.byref(d), P, xyz.data_ptr(), _optr(order), None, 0.0, MASK_SPATIAL, None,
-                                                        S.data_ptr(), current_stream()), "hexplane_forward(spatial, inference cache)")
-        _lib.COUNTERS["spatial_product_evaluations"] += 1
-        _INFER = {"key": key, "S": S, "A": None, "used": False, "order": order}
-    return _INFER
 
 
 # ---- the same split under plain autograd (the reference's own training loop through the launcher) ---------------------------
@@ -420,40 +430,29 @@ def _drop_auto(*_):
 
 
 class _SpatialFn(torch.autograd.Function):
-    """S[P, 32 levels] = product over the three spatial planes (xy, xz, yz) of the bilinear samples at xyz, per level."""
+    """(S, product) = the autograd holder's _SpatialProduct at xyz and its S, differentiable in xyz and the planes."""
 
     @staticmethod
-    def forward(ctx, xyz, aabb, levels, res, *planes):
+    def forward(ctx, key, xyz, aabb, levels, res, *planes):
         xyz = xyz.contiguous()
         _check_cuda_f32(xyz, aabb, *planes)
-        P = int(xyz.shape[0])
-        S = torch.empty((P, 32 * levels), dtype=torch.float32, device=xyz.device)
-        d = _hex_desc(aabb, planes, levels, res)
-        order = _cell_order(xyz, aabb)
-        check(_lib.lib().b200gs_hexplane_forward_masked(ctypes.byref(d), P, xyz.data_ptr(), _optr(order), None, 0.0, MASK_SPATIAL, None,
-                                                        S.data_ptr(), current_stream()), "hexplane_forward(spatial)")
-        _lib.COUNTERS["spatial_product_evaluations"] += 1
+        product = _SpatialProduct(key, xyz, aabb, planes, levels, res, _cell_order(xyz, aabb), auto=True)
         ctx.save_for_backward(xyz, aabb, *planes)
         ctx.meta = (levels, res)
-        ctx.order = order
+        ctx.order = product.order
         ctx.params = planes
-        return S
+        return product.S, product
 
     @staticmethod
-    def backward(ctx, dS):
+    def backward(ctx, dS, _):
         xyz, aabb, *planes = ctx.saved_tensors
         levels, res = ctx.meta
-        P = int(xyz.shape[0])
         dS = dS.contiguous()
-        direct = [_grad_target(q) if (k % 6) in (0, 1, 3) else None for k, q in enumerate(ctx.params)]
-        grads = [(dp if dp is not None else torch.zeros_like(p, memory_format=torch.preserve_format)) if (k % 6) in (0, 1, 3) else None
+        direct = [_grad_target(q) if _is_spatial(k) else None for k, q in enumerate(ctx.params)]
+        grads = [(dp if dp is not None else torch.zeros_like(p, memory_format=torch.preserve_format)) if _is_spatial(k) else None
                  for k, (p, dp) in enumerate(zip(planes, direct))]
-        d = _hex_desc(aabb, planes, levels, res, grads)
-        d_xyz = torch.empty_like(xyz)
-        check(_lib.lib().b200gs_hexplane_backward_masked(ctypes.byref(d), P, xyz.data_ptr(), _optr(ctx.order), None, 0.0, MASK_SPATIAL,
-                                                         None, None, dS.data_ptr(), d_xyz.data_ptr(), None, 0, current_stream()),
-              "hexplane_backward(spatial)")
-        return (d_xyz, None, None, None, *[None if dp is not None else g for g, dp in zip(grads, direct)])
+        d_xyz = _SpatialProduct.backward(dS, xyz, ctx.order, aabb, planes, levels, res, grads)
+        return (None, d_xyz, None, None, None, *[None if dp is not None else g for g, dp in zip(grads, direct)])
 
 
 def _auto_spatial(xyz, grid):
@@ -461,14 +460,28 @@ def _auto_spatial(xyz, grid):
     of those tensors changes."""
     global _AUTO
     planes = grid._planes()
-    key = _shared_key(xyz, xyz._version, int(xyz.shape[0]), grid.aabb, planes)
-    if _AUTO is not None and _AUTO["key"] == key:
-        return _AUTO["S"]
-    S = _SpatialFn.apply(xyz, grid.aabb, len(grid.grids), tuple(grid._res), *planes)
-    if S.requires_grad:
-        S.register_hook(_drop_auto)          # its gradient is being produced: the graph below it is about to be freed
-    _AUTO = {"key": key, "S": S}
-    return S
+    if _AUTO is None or not _AUTO.matches(xyz, grid.aabb, planes):
+        S, _AUTO = _SpatialFn.apply(_product_key(xyz, xyz._version, grid.aabb, planes), xyz, grid.aabb, len(grid.grids),
+                                    tuple(grid._res), *planes)
+        if S.requires_grad:
+            S.register_hook(_drop_auto)          # its gradient is being produced: the graph below it is about to be freed
+    return _AUTO.S
+
+
+def _product_for(xyz, aabb, planes, levels, res, order, S_in):
+    """The spatial product a field call multiplies its time planes by, or None (all six planes sampled): the explicit scope's
+    if it matches, else the autograd holder's if the caller passed its S (S_in, from _auto_spatial), else the implicit no-grad
+    cache's (evaluated here on a miss)."""
+    global _INFER
+    if _SHARED is not None and _SHARED.matches(xyz, aabb, planes):
+        return _SHARED
+    if S_in is not None:
+        return _AUTO
+    if not INFERENCE_SPATIAL_CACHE or torch.is_grad_enabled():
+        return None
+    if _INFER is None or not _INFER.matches(xyz, aabb, planes):
+        _INFER = _SpatialProduct(_product_key(xyz, xyz._version, aabb, planes), xyz, aabb, planes, levels, res, order)
+    return _INFER
 
 
 class _DeformFn(torch.autograd.Function):
@@ -478,8 +491,8 @@ class _DeformFn(torch.autograd.Function):
             need_backward, w1, b1, (w2,b2,w3,b3) x 5 heads, *planes
     heads: (pos, scales, rotations, opacity, shs) on / off.  opacity' / shs' are returned only for the heads that are on
     (csrc/deform_heads.cu); opacity / shs may be None when their head is off.
-    S_in: None, or the differentiable spatial product of _SpatialFn (then only the time planes are sampled here and
-    dL/dS_in is returned for autograd to sum over the views of a batch).
+    S_in: None, or the autograd holder's differentiable spatial product (_auto_spatial; then only the time planes are sampled
+    here and dL/dS_in is returned for autograd to sum over the views of a batch).
     """
     N_FIXED = 15
     N_W = 22
@@ -499,17 +512,11 @@ class _DeformFn(torch.autograd.Function):
         d = _hex_desc(aabb, planes, levels, res)
         order = _cell_order(xyz, aabb)
         ctx.order = order
-        sh = _shared_for(xyz, P, aabb, planes)
-        if sh is None and S_in is not None:
-            sh = {"S": S_in.contiguous(), "A": None, "used": False, "auto": True}
-        if sh is None:
-            sh = _inference_shared(xyz, P, aabb, planes, levels, res, order)
-        ctx.shared = sh
+        sh = ctx.product = _product_for(xyz, aabb, planes, levels, res, order, S_in)
         ctx.time_rows = False
         ctx.feat_tiled = False
         if sh is not None and tt is None and L.b200gs_hexplane_time_supported(ctypes.byref(d)):
             # shared spatial product + one timestamp for the view: time planes served from shared memory
-            sh["used"] = True
             ctx.time_rows = True
             # (no cell order here: with the rows in shared memory there is no texel locality to gain, and walking the points in
             #  storage order keeps the S / feature rows streaming)
@@ -517,16 +524,15 @@ class _DeformFn(torch.autograd.Function):
             ctx.feat_tiled = levels == 2
             if ctx.feat_tiled:
                 feat = torch.empty(((P + 127) // 128 * 128, 32 * levels), dtype=torch.float32, device=dev)
-            check(L.b200gs_hexplane_time_forward(ctypes.byref(d), P, xyz.data_ptr(), None, ts, sh["S"].data_ptr(),
+            check(L.b200gs_hexplane_time_forward(ctypes.byref(d), P, xyz.data_ptr(), None, ts, sh.S.data_ptr(),
                                                  feat.data_ptr(), int(ctx.feat_tiled), stream), "hexplane_time_forward")
             _lib.COUNTERS["time_row_forward_calls"] += 1
-        elif sh is not None:      # spatial product from begin_shared_step; only the time planes are sampled per view
-            sh["used"] = True
-            check(L.b200gs_hexplane_forward_masked(ctypes.byref(d), P, xyz.data_ptr(), _optr(order),
-                                                   tt.data_ptr() if tt is not None else None, ts, MASK_TIME, sh["S"].data_ptr(),
+        elif sh is not None:      # shared spatial product, per-point times: only the time planes are sampled per view
+            check(L.b200gs_hexplane_forward_masked(ctypes.byref(d), P, xyz.data_ptr(), _lib.ptr(order),
+                                                   tt.data_ptr() if tt is not None else None, ts, MASK_TIME, sh.S.data_ptr(),
                                                    feat.data_ptr(), stream), "hexplane_forward(time)")
         else:
-            check(L.b200gs_hexplane_forward(ctypes.byref(d), P, xyz.data_ptr(), _optr(order),
+            check(L.b200gs_hexplane_forward(ctypes.byref(d), P, xyz.data_ptr(), _lib.ptr(order),
                                             tt.data_ptr() if tt is not None else None, ts, feat.data_ptr(), stream),
                   "hexplane_forward")
         mw = _DeformFn._weights_struct(weights, heads, 32 * levels)
@@ -559,7 +565,7 @@ class _DeformFn(torch.autograd.Function):
             hw = _DeformFn._heads_struct(weights, heads, 32 * levels, ctx.feat_tiled)
             check(L.b200gs_deform_heads_forward(ctypes.byref(hw), P, _sh_coeffs(sh_in), saved.data_ptr(), _lib.ptr(op_in),
                                                 _lib.ptr(sh_in), _lib.ptr(op_o), _lib.ptr(sh_o),
-                                                hsaved.data_ptr() if hsaved.numel() else None, stream), "deform_heads_forward")
+                                                _lib.ptr(hsaved), stream), "deform_heads_forward")
             _lib.COUNTERS["deform_heads_forward"] += 1
             outs += [o for o in (op_o, sh_o) if o is not None]
         if saved is None:
@@ -626,10 +632,9 @@ class _DeformFn(torch.autograd.Function):
         d_feat = torch.empty_like(feat)
         # contiguous copies of the upstream gradients stay referenced until the launch has been queued
         d_pts, d_scales, d_rot = (t.contiguous() if t is not None else None for t in (d_pts, d_scales, d_rot))
-        cp = lambda t: t.data_ptr() if t is not None else None
         check(L.b200gs_deform_mlp_backward(ctypes.byref(mw), ctypes.byref(mg), P, feat.data_ptr(), saved.data_ptr(),
-                                           cp(d_pts) if heads[0] else None, cp(d_scales) if heads[1] else None,
-                                           cp(d_rot) if heads[2] else None, d_feat.data_ptr(), stream), "deform_mlp_backward")
+                                           _lib.ptr(d_pts) if heads[0] else None, _lib.ptr(d_scales) if heads[1] else None,
+                                           _lib.ptr(d_rot) if heads[2] else None, d_feat.data_ptr(), stream), "deform_mlp_backward")
         d_op = d_sh = None
         if heads[3] or heads[4]:
             if hsaved.numel() == 0:
@@ -648,7 +653,7 @@ class _DeformFn(torch.autograd.Function):
                     hg.w2[h], hg.b2[h], hg.w3[h], hg.b3[h] = (gws[i].data_ptr() for i in range(14 + 4 * h, 18 + 4 * h))
             hw = _DeformFn._heads_struct(weights, heads, 32 * levels, ctx.feat_tiled)
             check(L.b200gs_deform_heads_backward(ctypes.byref(hw), ctypes.byref(hg), P, _sh_coeffs(d_sh), feat.data_ptr(),
-                                                 saved.data_ptr(), hsaved.data_ptr(), cp(d_op), cp(d_sh), d_feat.data_ptr(),
+                                                 saved.data_ptr(), hsaved.data_ptr(), _lib.ptr(d_op), _lib.ptr(d_sh), d_feat.data_ptr(),
                                                  acc.data_ptr() if use_acc else None, int(use_acc and SH_GRAD_OVERWRITE), stream),
                   "deform_heads_backward")
             _lib.COUNTERS["deform_heads_backward"] += 1
@@ -656,40 +661,34 @@ class _DeformFn(torch.autograd.Function):
                 d_sh = None                     # already in the step's SH buffer
         if AFTER_MLP_BACKWARD is not None:
             AFTER_MLP_BACKWARD()
-        sh = ctx.shared
+        sh = ctx.product
         # the spatial planes receive nothing here when only the time planes were sampled (their share goes through S)
-        time_only = sh is not None
-        gplanes = [dp if dp is not None else (None if (time_only and (k % 6) in (0, 1, 3)) else torch.zeros_like(p, memory_format=torch.preserve_format))
+        gplanes = [dp if dp is not None else (None if (sh is not None and _is_spatial(k)) else torch.zeros_like(p, memory_format=torch.preserve_format))
                    for k, (p, dp) in enumerate(zip(planes, direct_p))]
         d_xyz_grid = torch.empty_like(xyz)
         d = _hex_desc(aabb, planes, levels, res, gplanes)
-        d_S = None
+        dS = None
         if ctx.time_rows:
             scratch, nbytes = _time_row_scratch(d, xyz.device)
-            if sh.get("auto"):
-                d_S = torch.empty_like(sh["S"])          # this view's dL/dS (WRITTEN by the kernel: flag bit 1); autograd sums the views
-            A = d_S if d_S is not None else sh["A"]
-            overwrite = d_S is not None or not sh.get("A_written", True)
-            check(L.b200gs_hexplane_time_backward(ctypes.byref(d), P, xyz.data_ptr(), None, ts, sh["S"].data_ptr(),
-                                                  A.data_ptr(), d_feat.data_ptr(), d_xyz_grid.data_ptr(), scratch.data_ptr(),
+            dS, overwrite = sh.view_gradient(accumulate_only=False)
+            check(L.b200gs_hexplane_time_backward(ctypes.byref(d), P, xyz.data_ptr(), None, ts, sh.S.data_ptr(),
+                                                  dS.data_ptr(), d_feat.data_ptr(), d_xyz_grid.data_ptr(), scratch.data_ptr(),
                                                   nbytes, int(ctx.feat_tiled) | (2 if overwrite else 0), stream), "hexplane_time_backward")
-            sh["A_written"] = True
         elif sh is not None or not has_t:
-            # shared step: time planes now, the spatial planes' share is accumulated for finish_shared_step.
+            # shared product: time planes now, the spatial planes' share goes into this view's dL/dS.
             # One timestamp for the whole launch (scalar time): the time planes' gradient goes through replicated 1-D rows.
             scratch, nbytes = _time_row_scratch(d, xyz.device) if not has_t else (None, 0)
-            if sh is not None and not sh.get("A_written", True):
-                sh["A"].zero_(); sh["A_written"] = True          # this kernel only accumulates
-            check(L.b200gs_hexplane_backward_masked(ctypes.byref(d), P, xyz.data_ptr(), _optr(ctx.order),
+            if sh is not None:
+                dS, _ = sh.view_gradient(accumulate_only=True)
+            check(L.b200gs_hexplane_backward_masked(ctypes.byref(d), P, xyz.data_ptr(), _lib.ptr(ctx.order),
                                                     tt.data_ptr() if has_t else None, ts, MASK_TIME if sh is not None else MASK_ALL,
-                                                    sh["S"].data_ptr() if sh is not None else None,
-                                                    sh["A"].data_ptr() if sh is not None else None, d_feat.data_ptr(),
-                                                    d_xyz_grid.data_ptr(), scratch.data_ptr() if scratch is not None else None, nbytes,
-                                                    stream), "hexplane_backward(time)")
+                                                    sh.S.data_ptr() if sh is not None else None, _lib.ptr(dS), d_feat.data_ptr(),
+                                                    d_xyz_grid.data_ptr(), _lib.ptr(scratch), nbytes, stream), "hexplane_backward(time)")
         else:
-            check(L.b200gs_hexplane_backward(ctypes.byref(d), P, xyz.data_ptr(), _optr(ctx.order),
+            check(L.b200gs_hexplane_backward(ctypes.byref(d), P, xyz.data_ptr(), _lib.ptr(ctx.order),
                                              tt.data_ptr() if has_t else None, ts, d_feat.data_ptr(), d_xyz_grid.data_ptr(),
                                              stream), "hexplane_backward")
+        d_S = dS if sh is not None and sh.auto else None        # the autograd holder's views: autograd sums dL/dS
         # pts = xyz*1 + ..., scales = scales*1 + ds, rot = rot + dr: identity paths
         d_xyz = d_xyz_grid + d_pts if d_pts is not None else d_xyz_grid
         gw_out = [None if dw is not None else g for g, dw in zip(gws, direct_w)]      # accumulated in place -> nothing for autograd

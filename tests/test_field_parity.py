@@ -193,3 +193,49 @@ def test_inference_forward_without_stash_is_bit_identical():
     # with the spatial product shared under autograd (the default) the field re-associates the six-plane product: FP32 rounding only
     p3, s3, r3, _, _ = net(a[0], a[1], a[2], opacity, shs, time, flow, fn, 1)
     assert _rel(p3.detach(), p2) < 2e-6 and _rel(s3.detach(), s2) < 2e-6 and _rel(r3.detach(), r2) < 2e-6
+
+
+def test_autograd_sharing_two_calls_one_backward():
+    """field.AUTOGRAD_SPATIAL_SHARING as the reference's training loop meets it: two field calls on the same xyz leaf, then ONE
+    backward.  The spatial product is evaluated once, each call samples only its time planes, autograd sums the two calls'
+    dL/dS into one spatial backward, and that backward drops the product.  Outputs and gradients equal the same two calls
+    without sharing (six-plane forward, MASK_ALL backward per call) up to FP32 re-association."""
+    from b200gs import _lib, field
+    P = 20011
+    xyz, scales, rot, opacity, shs, flow = _inputs(P)
+    fn = torch.tensor(7, device="cuda")
+    g = torch.Generator().manual_seed(6)
+    w = [torch.randn(P, k, generator=g).cuda() for k in (3, 3, 4, 3, 3, 4)]
+
+    def run(share):
+        net = _model([1, 2], 50)
+        a = [t.clone().requires_grad_(True) for t in (xyz, scales, rot)]
+        keep = field.AUTOGRAD_SPATIAL_SHARING
+        field.AUTOGRAD_SPATIAL_SHARING = share
+        try:
+            c0 = _lib.COUNTERS.copy()
+            outs = [o for t in (0.2, 0.7) for o in net(a[0], a[1], a[2], opacity, shs, t, flow, fn, 1)[:3]]
+            sum((o * wi).sum() for o, wi in zip(outs, w)).backward()
+            c1 = _lib.COUNTERS.copy()
+            net(a[0], a[1], a[2], opacity, shs, 0.2, flow, fn, 1)
+            c2 = _lib.COUNTERS.copy()
+        finally:
+            field.AUTOGRAD_SPATIAL_SHARING = keep
+            field.drop_shared()
+        if share:
+            assert c1["spatial_product_evaluations"] - c0["spatial_product_evaluations"] == 1
+            assert c1["time_row_forward_calls"] - c0["time_row_forward_calls"] == 2
+            assert c2["spatial_product_evaluations"] - c1["spatial_product_evaluations"] == 1       # the backward dropped it
+        else:
+            assert c2["spatial_product_evaluations"] == c0["spatial_product_evaluations"]
+        grads = dict(zip(("xyz", "scales", "rot"), (t.grad for t in a)))
+        grads.update((n, p.grad) for n, p in net.named_parameters() if p.grad is not None)
+        return [o.detach() for o in outs], grads
+
+    shared_outs, shared_grads = run(True)
+    plain_outs, plain_grads = run(False)
+    for s, p in zip(shared_outs, plain_outs):
+        assert _rel(s, p) < 2e-6
+    assert shared_grads.keys() == plain_grads.keys() and len(plain_grads) >= 3 + 2 + 12 + 12
+    for k, p in plain_grads.items():
+        assert _rel(shared_grads[k], p) < 1e-4, k

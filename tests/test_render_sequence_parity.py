@@ -70,7 +70,7 @@ def test_render_frames_matches_the_reference_stack(request):
         assert float((ddiff > 1e-3).mean()) < 1e-4, float(ddiff.max())
 
 
-def test_implicit_inference_cache_matches_and_is_dropped_by_the_optimiser():
+def test_implicit_inference_cache_matches_and_is_dropped_by_fused_adam():
     """field.INFERENCE_SPATIAL_CACHE: the same reuse without a wrapper around the frame loop (unchanged render_4DGS.py through the
     launcher); a FusedAdam step must drop the cached product, a changed plane must miss it."""
     from b200gs import engine, field, synthetic as syn
@@ -96,10 +96,10 @@ def test_implicit_inference_cache_matches_and_is_dropped_by_the_optimiser():
         assert field._INFER is None                           # FusedAdam.step dropped it
         with torch.no_grad():
             after = engine.render(cams[0], model, bg, stage="fine")["render"]
-            key = field._INFER["key"]
+            key = field._INFER.key
             next(iter(model._deformation.deformation_net.grid.grids.parameters())).add_(0.01)      # version bump
             engine.render(cams[0], model, bg, stage="fine")
-            assert field._INFER["key"] != key
+            assert field._INFER.key != key
         assert float((after - ref[0]).abs().max()) > 0        # the parameters did move
     finally:
         field.INFERENCE_SPATIAL_CACHE = False
